@@ -44,6 +44,7 @@ WORKLOADS = {
 }
 FP64_PEAK_TFLOPS = 37.0   # measured DMMA issue-rate peak on this pool's B200 (profiles/r01_fp64_peak_microbench.jsonl)
 SEED = 20260101
+DUMP_BYTES = 60 << 20     # --dump-outputs stays below 64 MB in all (npy headers included)
 
 
 def env_int(name, default):
@@ -110,6 +111,38 @@ class ClockSampler:
                     pass
         return {"sm_mhz": float(np.median(sm)) if sm else None, "sm_max_mhz": smax, "reasons": sorted(reasons),
                 "samples": len(sm), "power_w_max": max(power) if power else None}
+
+
+# fields indexed by column m of Y: (M, w) matrices and (M*w,) vectors of per-column blocks of w entries
+COLUMN_FIELDS = {
+    "dense": ("AHat",),
+    "sparse": ("AHat", "ATVecHat", "diagSigmaATVec", "CA", "beta"),
+    "dual": ("AHat", "ATVecHat", "diagSigmaATVec", "CA", "beta", "A0Hat", "A1Hat", "CA0", "CA1", "beta0", "beta1"),
+}
+
+
+def dump_outputs(out_dir, p, delta, kind):
+    """--dump-outputs: every floating-point field of the parameter struct the timed loop hands back, plus its final convergence
+    delta, as float64 DIR/<field>.npy (DIR/final_delta.npy for the delta).  The COLUMN_FIELDS of `kind` keep the same fixed,
+    seeded subset of columns, as many as DUMP_BYTES allows, so that two builds run with the same arguments can be compared
+    output for output."""
+    M = p.M
+    fields = {n: np.asarray(v, dtype=np.float64) for n, v in vars(p).items()
+              if v is not None and np.asarray(v).dtype.kind == "f"}
+    fields["final_delta"] = np.asarray(delta, dtype=np.float64)
+    cols = COLUMN_FIELDS[kind]
+    fixed = sum(a.nbytes for n, a in fields.items() if n not in cols)
+    per_col = sum(fields[n].nbytes for n in cols) // M
+    k = min(M, (DUMP_BYTES - fixed) // per_col)
+    if k < 1:
+        raise SystemExit("--dump-outputs: the outputs not indexed by column alone exceed %d bytes" % DUMP_BYTES)
+    if k < M:
+        idx = np.sort(np.random.default_rng(SEED).choice(M, k, replace=False))
+        for n in cols:
+            fields[n] = fields[n][idx] if fields[n].ndim == 2 else fields[n].reshape(M, -1)[idx].reshape(-1)
+    os.makedirs(out_dir, exist_ok=True)
+    for n, a in fields.items():
+        np.save(os.path.join(out_dir, n + ".npy"), a)
 
 
 # ------------------------------------------------------------------------------------------------ CPU arm (oracle)
@@ -331,7 +364,15 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--segments", action="store_true",
                     help="diagnosis: CUDA events between the launches of every iteration (adds stream bubbles; not for headline numbers)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed iterations, write the state they leave (rank 0's column shard when N > 1) as DIR/<field>.npy, "
+                         "float64, under 64 MB in all; column-indexed fields keep a fixed, seeded sample of the columns.  Not available "
+                         "with --workload c2, --single-process or --impl reference")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.single_process or args.workload == "c2"):
+        ap.error("--dump-outputs covers the resident-Y timed loop only (--impl ours, no --single-process, not --workload c2)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else max(args.warmup, 0)
     if args.workload == "c2":
         if args.impl == "ours":
@@ -460,6 +501,8 @@ def main():
         state_check["sum_CB"] = float(np.sum(p.CB))
     if kind == "dual":
         state_check.update({"alpha00": float(p.alpha00), "beta00": float(p.beta00), "alpha01": float(p.alpha01), "beta01": float(p.beta01)})
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, p, d, kind)
 
     # ---- roofline of the dominant kernel (the slower of the two contractions), CUDA events on the launching stream
     k1 = prof["k1_ms"] / max(prof["k1_launches"], 1)

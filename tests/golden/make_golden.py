@@ -1,8 +1,8 @@
 """Decode the reference's own JLD (HDF5) fixtures into plain .npz goldens.
 
-Inputs  (read-only, only available in the build container):
-    /root/reference/examples/data/vbmf_test/{inputs,log}.jld     dense vbmf, 100 iterations
-    /root/reference/examples/data/sparse_test/{inputs,log}.jld   vbmf_sparse full_cov, 100 iterations
+Inputs  (read-only, from a checkout of VBMatrixFactorization.jl named by the environment variable VBMF_REFERENCE_DIR):
+    $VBMF_REFERENCE_DIR/examples/data/vbmf_test/{inputs,log}.jld     dense vbmf, 100 iterations
+    $VBMF_REFERENCE_DIR/examples/data/sparse_test/{inputs,log}.jld   vbmf_sparse full_cov, 100 iterations
 They were written by examples/toy_data.jl:35-36,55-56 through save_log (src/data_manip.jl:53-66).
 
 Outputs (committed): tests/golden/vbmf_test.npz, tests/golden/sparse_test.npz
@@ -13,7 +13,7 @@ little-endian f64 / i64 datasets.  Julia arrays are column-major; HDF5 dims are 
 so a Julia (d1, d2, T) array is returned here as a C-ordered numpy array of shape (T, d2, d1); consumers
 use slice[t].T to get the Julia matrix of iteration t.
 
-Run:  python tests/golden/make_golden.py
+Run:  VBMF_REFERENCE_DIR=<checkout> python tests/golden/make_golden.py
 """
 import os
 import re
@@ -22,7 +22,6 @@ import sys
 
 import numpy as np
 
-REF = "/root/reference/examples/data"
 OUT = os.path.dirname(os.path.abspath(__file__))
 
 
@@ -113,9 +112,12 @@ def main():
     global OUT
     if "--out" in sys.argv:          # write somewhere else (tests/test_oracle_mp.py re-derives the fixtures and compares)
         OUT = sys.argv[sys.argv.index("--out") + 1]
+    if not os.environ.get("VBMF_REFERENCE_DIR"):
+        return "set VBMF_REFERENCE_DIR to a checkout of VBMatrixFactorization.jl"
+    ref = os.path.join(os.environ["VBMF_REFERENCE_DIR"], "examples", "data")
     for case in ("vbmf_test", "sparse_test"):
-        inputs = read_jld(os.path.join(REF, case, "inputs.jld"))
-        log = read_jld(os.path.join(REF, case, "log.jld"))
+        inputs = read_jld(os.path.join(ref, case, "inputs.jld"))
+        log = read_jld(os.path.join(ref, case, "log.jld"))
         Y = inputs["Y"]  # (M, L) C-order == Julia L x M column-major
         fields = {"Y": np.ascontiguousarray(Y)}
         for k, v in sorted(log.items()):

@@ -33,6 +33,30 @@ def test_reference_arm_other_ranks_are_silent():
     assert r.returncode == 0 and r.stdout.strip() == ""
 
 
+def test_dump_outputs_samples_columns_consistently(tmp_path, monkeypatch):
+    import bench
+    vb = vbmf_b200_loader.load()
+
+    class Shape:
+        shape = (30, 500)
+    p = vb.vbmf_sparse_init(Shape, 4, rng=np.random.default_rng(0), trYTY=1.0)
+    p.CA = np.arange(p.MH, dtype=np.float64)
+    monkeypatch.setattr(bench, "DUMP_BYTES", 40000)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), p, 0.25, "sparse")
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert names == sorted(os.listdir(tmp_path / "b")) and "labels.npy" not in names and "final_delta.npy" in names
+    out = {n[:-4]: np.load(tmp_path / "a" / n) for n in names}
+    assert all(a.dtype == np.float64 for a in out.values())
+    assert sum(os.path.getsize(tmp_path / "a" / n) for n in names) < 40000 + 128 * len(names)
+    for n in names:
+        assert np.array_equal(out[n[:-4]], np.load(tmp_path / "b" / n))
+    cols = out["CA"].reshape(-1, 4)[:, 0] // 4          # CA[m*H + h] = m*H + h names its column
+    assert 0 < cols.size < 500 and np.all(np.diff(cols) > 0)
+    assert np.array_equal(out["AHat"], p.AHat[cols.astype(int)]) and np.array_equal(out["ATVecHat"].reshape(-1, 4), out["AHat"])
+    assert np.array_equal(out["BHat"], p.BHat) and out["final_delta"] == 0.25
+
+
 def test_log_roundtrip(tmp_path):
     vb = vbmf_b200_loader.load()
     Y = np.arange(12.0).reshape(3, 4)

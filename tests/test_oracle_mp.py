@@ -144,15 +144,38 @@ def test_dual_lower_bound_literal():
     assert abs(got - want) <= 1e-11 * abs(want)
 
 
+GOLDEN_SHA256 = {   # content of tests/golden/*.npz as decoded from the reference's .jld logs (see the test below)
+    "vbmf_test": "3989a1a74c27586734db202ad24e1ee19eb6a453893b0a9aadf2a79d1a404f4f",
+    "sparse_test": "81db05bf56b4494d92085226d44d04c317b52b21463472b5e40f5683403dd5be",
+}
+
+
+def test_golden_fixtures_match_the_decoded_reference_logs():
+    """Every golden comparison rests on tests/golden/*.npz holding exactly what make_golden.py decoded from the reference's .jld
+    logs.  The .jld files are not part of this repository, so the decoded content is pinned by digest: any edit to a fixture
+    (a field, dtype, shape or value) fails here on every machine."""
+    import hashlib
+    import os
+    here = os.path.dirname(os.path.abspath(__file__))
+    for name, want in GOLDEN_SHA256.items():
+        g = np.load(os.path.join(here, "golden", name + ".npz"))
+        h = hashlib.sha256()
+        for k in sorted(g.files):
+            a = np.ascontiguousarray(g[k])
+            h.update(("%s|%s|%s|" % (k, a.dtype.str, a.shape)).encode())
+            h.update(a.tobytes())
+        assert h.hexdigest() == want, name
+
+
 def test_golden_fixtures_regenerate_from_the_reference(tmp_path):
-    """tests/golden/*.npz are exactly what tests/golden/make_golden.py decodes from the reference's own .jld logs (skipped where
-    /root/reference is not mounted, e.g. on the GPU box)."""
+    """tests/golden/*.npz are exactly what tests/golden/make_golden.py decodes from the reference's own .jld logs (skipped unless
+    VBMF_REFERENCE_DIR names a checkout of VBMatrixFactorization.jl; the .jld files are not part of this repository)."""
     import os
     import subprocess
     import sys
-    ref = "/root/reference/examples/data"
-    if not os.path.isdir(ref):
-        pytest.skip("reference not mounted")
+    ref = os.environ.get("VBMF_REFERENCE_DIR", "")
+    if not ref or not os.path.isdir(os.path.join(ref, "examples", "data")):
+        pytest.skip("VBMF_REFERENCE_DIR does not name a checkout of VBMatrixFactorization.jl")
     here = os.path.dirname(os.path.abspath(__file__))
     script = os.path.join(here, "golden", "make_golden.py")
     r = subprocess.run([sys.executable, script, "--out", str(tmp_path)], capture_output=True, text=True, timeout=300)
