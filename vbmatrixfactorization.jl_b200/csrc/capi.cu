@@ -105,6 +105,15 @@ struct vbmf_b200_ctx {
     int chunks_pending = 0;           // > 0: chunks whose arrival the main stream has not been ordered after yet
     bool tr_pending = false;          // trYTY lives in d_tr only (not yet read back to the host)
     bool simt = false;
+    bool gemm_dmma = false;   // VBMF_B200_GEMM=dmma: keep the FP64 tensor-core contractions at H <= 64 (A/B measurements)
+    // int8 slices of Y for the INT8 contractions (gemm_int8.cu): [8][Mloc][ldZ], exponents F[L] | E[Mloc]; built on first
+    // use after every change of Y (ctx_slices)
+    uint8_t* Z = nullptr;
+    int* Zexp = nullptr;
+    size_t Z_bytes = 0;
+    int ldZ = 0;
+    bool z_ready = false, z_failed = false;
+    CUtensorMap tmZ1, tmZ2;
     // profiling of the two contractions
     bool profile = false;
     std::vector<cudaEvent_t> ev_k1, ev_k2, ev_ar;      // K1, K2 and (world > 1) the per-iteration all-reduce
@@ -309,6 +318,7 @@ static int ctx_create_impl(int device, int rank, int world, const void* nccl_id1
     }
     const char* g = getenv("VBMF_B200_GEMM");
     c->simt = (g != nullptr && strcmp(g, "simt") == 0);
+    c->gemm_dmma = (g != nullptr && strcmp(g, "dmma") == 0);
     if (c->world > 1) {
         if (comm_in != nullptr) c->comm = comm_in;
         else {
@@ -341,7 +351,15 @@ int nccl_comm_init_all(void** comms, int ndev, const int* devs) {
 }
 }
 
+static void ctx_free_Z(vbmf_b200_ctx* c) {
+    if (c->Z) cudaFree(c->Z);
+    if (c->Zexp) cudaFree(c->Zexp);
+    c->Z = nullptr; c->Zexp = nullptr; c->Z_bytes = 0;
+    c->z_ready = false; c->z_failed = false;
+}
+
 static void ctx_free_Y(vbmf_b200_ctx* c) {
+    ctx_free_Z(c);
     if (c->copy_st) cudaStreamSynchronize(c->copy_st);
     if (c->stat_st) cudaStreamSynchronize(c->stat_st);
     c->chunks_pending = 0; c->tr_pending = false;
@@ -407,6 +425,7 @@ static int ctx_alloc_Y(vbmf_b200_ctx* c, int64_t L, int64_t Mloc, int64_t Mglob,
         c->L_cap = (int)L;
     }
     c->have_Y = false;
+    c->z_ready = false; c->z_failed = false;
     c->L = (int)L; c->Mloc = (int)Mloc; c->Mglob = (int)Mglob; c->moff = (int)off;
     c->ldY = ld;
     if (c->ldY != L) VB_CUDA_OK(cudaMemsetAsync(c->Y, 0, bytes, c->st));
@@ -450,6 +469,91 @@ static int ctx_host_trYTY(vbmf_b200_ctx* c) {
     }
     return 0;
 }
+static size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
+
+// The INT8 contractions run at H <= 64 unless the FP64 kernels are forced (VBMF_B200_GEMM=simt / dmma).
+static bool ctx_int8_wanted(const vbmf_b200_ctx* c, int64_t H) {
+    return !c->simt && !c->gemm_dmma && H >= 1 && H <= 64 && c->Y != nullptr && c->Mloc > 0;
+}
+// Slices of the resident Y, built on the main stream the first time an INT8 contraction needs them after Y changed (the
+// caller has ordered the stream after the upload).  *ok = false when they cannot be allocated: the caller then runs the
+// FP64 kernels.
+static int ctx_slices(vbmf_b200_ctx* c, bool* ok) {
+    *ok = false;
+    if (c->z_failed || c->Y == nullptr || c->Mloc <= 0) return 0;
+    if (c->z_ready) { *ok = true; return 0; }
+    const int ldZ = i8_ld(c->L);
+    const size_t bytes = (size_t)8 * c->Mloc * ldZ;
+    if (c->Z == nullptr || c->Z_bytes != bytes || c->ldZ != ldZ) {
+        ctx_free_Z(c);
+        if (cudaMalloc(&c->Z, bytes) != cudaSuccess || cudaMalloc(&c->Zexp, ((size_t)c->L + c->Mloc) * 4) != cudaSuccess) {
+            cudaGetLastError();
+            ctx_free_Z(c);
+            c->z_failed = true;
+            return 0;
+        }
+        c->Z_bytes = bytes; c->ldZ = ldZ;
+    }
+    if (i8_build_Y(c->st, c->Y, c->ldY, c->L, c->Mloc, c->Z, ldZ, c->Zexp, c->Zexp + c->L)) return -1;
+    const uint64_t s1 = (uint64_t)ldZ, s2 = (uint64_t)ldZ * c->Mloc;
+    if (make_tmap_3d_i8(&c->tmZ1, c->Z, (uint64_t)c->L, (uint64_t)c->Mloc, 8, s1, s2, 32, 128, 8, false)) return -1;
+    if (make_tmap_3d_i8(&c->tmZ2, c->Z, (uint64_t)c->L, (uint64_t)c->Mloc, 8, s1, s2, 128, 32, 8, true)) return -1;
+    c->z_ready = true;
+    *ok = true;
+    return 0;
+}
+// Split-K plans of the INT8 path: the FP64 plans with k ranges on multiples of 32 (K1: kbs1 16-row blocks per split)
+static void i8_plans(int L, int M, int H, int num_sms, int* S1, int* kbs1, int* S, int* kchunk) {
+    plan_splitk_ytb(L, M, H, num_sms, S1, kbs1);
+    *kbs1 = (*kbs1 + 1) & ~1;
+    const int nkb = (L + 15) / 16;
+    *S1 = std::max(1, (nkb + *kbs1 - 1) / *kbs1);
+    plan_splitk(L, M, H, num_sms, S, kchunk);
+    *kchunk = (*kchunk + 31) / 32 * 32;
+    *S = std::max(1, (M + *kchunk - 1) / *kchunk);
+}
+// operand slices of the INT8 path: K1 [8][Hp][ldZ] + G[Hp], K2 [8][Hp][ldM] + G[S][Hp] (one allocation)
+struct I8Operands {
+    char* mem = nullptr;
+    uint8_t *Wb = nullptr, *Wa = nullptr;
+    int *Gb = nullptr, *Ga = nullptr;
+    int ldM = 0;
+    CUtensorMap tmWb, tmWa;
+    I8Operands() = default;
+    I8Operands(const I8Operands&) = delete;
+    I8Operands& operator=(const I8Operands&) = delete;
+    ~I8Operands() { if (mem) cudaFree(mem); }
+};
+static int i8_operands_alloc(I8Operands* o, int L, int M, int H, int S, bool* ok) {
+    *ok = false;
+    const int Hp = i8_hpad(H), ldZ = i8_ld(L);
+    o->ldM = i8_ld(std::max(M, 1));
+    const size_t nb = align_up((size_t)8 * Hp * ldZ, 256), na = align_up((size_t)8 * Hp * o->ldM, 256);
+    const size_t gb = align_up((size_t)Hp * 4, 256), ga = align_up((size_t)S * Hp * 4, 256);
+    if (cudaMalloc(&o->mem, nb + na + gb + ga) != cudaSuccess) { cudaGetLastError(); o->mem = nullptr; return 0; }
+    o->Wb = (uint8_t*)o->mem; o->Wa = o->Wb + nb; o->Gb = (int*)(o->Wa + na); o->Ga = (int*)((char*)o->Gb + gb);
+    if (make_tmap_3d_i8(&o->tmWb, o->Wb, (uint64_t)L, (uint64_t)Hp, 8, (uint64_t)ldZ, (uint64_t)ldZ * Hp, 32, (uint32_t)Hp, 8, false)) return -1;
+    if (M > 0 && make_tmap_3d_i8(&o->tmWa, o->Wa, (uint64_t)M, (uint64_t)Hp, 8, (uint64_t)o->ldM, (uint64_t)o->ldM * Hp, 32, (uint32_t)Hp, 8, false)) return -1;
+    *ok = true;
+    return 0;
+}
+// K1 on the INT8 path: P (or S1 slabs of it, stride M*H) = Y' * B
+static int i8_k1(vbmf_b200_ctx* c, I8Operands* o, const double* B, int ldB, int H, double* P, int S1, int kbs1, const Scalars* sc) {
+    const int* F = c->Zexp;
+    const int* E = c->Zexp + c->L;
+    if (i8_slice_B(c->st, B, ldB, c->L, H, F, o->Wb, c->ldZ, o->Gb, sc)) return -1;
+    return launch_gemm_i8(c->st, false, &c->tmZ1, &o->tmWb, P, c->Mloc, c->L, S1, kbs1 * 16, H, E, o->Gb, 0,
+                          (size_t)c->Mloc * H, (size_t)H, 1, sc, c->num_sms);
+}
+// K2 on the INT8 path: S slabs [H][ldQ] of Y * A (A row-major [Mloc][H])
+static int i8_k2(vbmf_b200_ctx* c, I8Operands* o, const double* A, int H, double* Qpart, int ldQ, int S, int kchunk, const Scalars* sc) {
+    const int* F = c->Zexp;
+    const int* E = c->Zexp + c->L;
+    if (i8_slice_A(c->st, A, c->Mloc, H, E, kchunk, S, o->Wa, o->ldM, o->Ga, sc)) return -1;
+    return launch_gemm_i8(c->st, true, &c->tmZ2, &o->tmWa, Qpart, c->L, c->Mloc, S, kchunk, H, F, o->Ga, i8_hpad(H),
+                          (size_t)H * ldQ, 1, (size_t)ldQ, sc, c->num_sms);
+}
+
 // Upload in column chunks on the copy stream, K0 chunk by chunk on the statistics stream; returns without waiting.
 static int attach_Y_chunked(vbmf_b200_ctx* c, const double* Y, int64_t ldY, int64_t chunk_cols) {
     if (!c->copy_st) VB_CUDA_OK(cudaStreamCreateWithFlags(&c->copy_st, cudaStreamNonBlocking));
@@ -569,6 +673,7 @@ extern "C" int vbmf_b200_preprocess_Y(vbmf_b200_ctx* c, double lambda, int64_t* 
     for (int l = 0; l < L; ++l) if (hrs[l] >= 1e-5) rows.push_back(l);      // used_rows[rowsums .>= 1e-5], :79
     const int Lnew = (int)rows.size();
     if (Lnew == 0) { set_error("preprocess_Y: every row is constant, nothing left"); return -1; }
+    c->z_ready = false; c->z_failed = false;
     if (Lnew == L) {
         if (k_scale_all(st, c->Y, (size_t)c->ldY * (size_t)std::max(M, 1), lambda)) return -1;
     } else {
@@ -694,6 +799,8 @@ struct vbmf_b200_solver {
     int* d_labels = nullptr;
     CUtensorMap tmB, tmBs, tmA;
     bool k2_simt = false;
+    bool i8 = false;              // K1 / K2 on the INT8 tensor cores (gemm_int8.cu) whenever Y's slices are available
+    I8Operands i8o;
     // host-side validity of derived quantities (every enqueued kernel either runs or is skipped as a whole iteration)
     bool btb_valid = false, ata_valid = false, q_valid = false, extras_valid = false, mean_valid = false;
     bool ata_local = false;   // packed.AtA holds this shard's AHat'AHat (not yet all-reduced)
@@ -723,7 +830,6 @@ struct vbmf_b200_solver {
     Scalars h_sc;
 };
 
-static size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
 static int solver_create_impl(vbmf_b200_ctx* c, int kind, int64_t H, int64_t h_split, int64_t M0_global, int64_t n_labels,
                               const int64_t* labels, int keep_blocks, vbmf_b200_solver** out) {
@@ -754,6 +860,11 @@ static int solver_create_impl(vbmf_b200_ctx* c, int kind, int64_t H, int64_t h_s
     plan_splitk(d.L, d.Mloc, d.H, c->num_sms, &s->S, &s->kchunk);
     plan_splitk_ytb(d.L, d.Mloc, d.H, c->num_sms, &s->S1, &s->kbs1);
     if (c->simt) s->S1 = 1;
+    s->i8 = ctx_int8_wanted(c, H);
+    if (s->i8) {
+        i8_plans(d.L, d.Mloc, d.H, c->num_sms, &s->S1, &s->kbs1, &s->S, &s->kchunk);
+        if (i8_operands_alloc(&s->i8o, d.L, d.Mloc, d.H, s->S, &s->i8)) { delete s; return -1; }
+    }
     if (c->chunks_pending > 0 && kind == VBMF_B200_DENSE) {      // the first iteration may run chunk by chunk behind the upload
         for (size_t k = 0; k < c->chunk_n.size(); ++k) {
             int Sc = 1, kc = 16;
@@ -1139,9 +1250,15 @@ static int enq_k1(vbmf_b200_solver* s, bool scaledB, bool reduce_slabs = true) {
     const Dev& d = s->d;
     if (c->Y == nullptr) { set_error("this step contracts with Y: attach Y first (the context only holds its shape)"); return -1; }
     if (settle_upload(s)) return -1;
+    bool i8 = false;
+    if (s->i8 && ctx_slices(c, &i8)) return -1;
     prof_mark(c, c->ev_k1);
     int rc;
-    if (c->simt) rc = launch_gemm_ytb_simt(c->st, d.Y, d.ldY, scaledB ? d.Bs : d.B, d.ldB, d.P, d.Mloc, d.L, d.H, d.H, d.sc);
+    if (i8) {
+        const size_t MH = (size_t)d.Mloc * d.H;
+        rc = i8_k1(c, &s->i8o, scaledB ? d.Bs : d.B, d.ldB, d.H, s->S1 > 1 ? s->Ppart : d.P, s->S1, s->kbs1, d.sc);
+        if (!rc && s->S1 > 1 && reduce_slabs) rc = k_sum_slabs(c->st, s->Ppart, s->S1, MH, d.P, d.sc);
+    } else if (c->simt) rc = launch_gemm_ytb_simt(c->st, d.Y, d.ldY, scaledB ? d.Bs : d.B, d.ldB, d.P, d.Mloc, d.L, d.H, d.H, d.sc);
     else {
         const size_t MH = (size_t)d.Mloc * d.H;
         rc = launch_gemm_ytb(c->st, &c->tmY1, scaledB ? &s->tmBs : &s->tmB, s->S1 > 1 ? s->Ppart : d.P, d.Mloc, d.L, d.H, d.H,
@@ -1157,15 +1274,18 @@ static int enq_k2(vbmf_b200_solver* s) {
     const Dev& d = s->d;
     if (c->Y == nullptr) { set_error("this step contracts with Y: attach Y first (the context only holds its shape)"); return -1; }
     if (settle_upload(s)) return -1;
+    bool i8 = false;
+    if (s->i8 && ctx_slices(c, &i8)) return -1;
     prof_mark(c, c->ev_k2);
     int rc;
-    if (s->k2_simt) rc = launch_gemm_ya_simt(c->st, d.Y, d.ldY, d.A, s->Qpart, d.L, d.Mloc, d.H, d.ldB, s->kchunk, s->S, d.sc);
+    if (i8) rc = i8_k2(c, &s->i8o, d.A, d.H, s->Qpart, d.ldB, s->S, s->kchunk, d.sc);
+    else if (s->k2_simt) rc = launch_gemm_ya_simt(c->st, d.Y, d.ldY, d.A, s->Qpart, d.L, d.Mloc, d.H, d.ldB, s->kchunk, s->S, d.sc);
     else if (s->k2_sk) rc = launch_gemm_ya_sk(c->st, &c->tmY2, &s->tmA, s->Qpart, d.packed + packed_q(d), d.L, d.Mloc, d.H, d.ldB, s->sk_kq, s->sk_nk, s->sk_grid, d.sc);
     else rc = launch_gemm_ya(c->st, &c->tmY2, &s->tmA, s->Qpart, d.L, d.Mloc, d.H, d.ldB, s->kchunk, s->S, d.sc, c->num_sms);
     prof_mark(c, c->ev_k2);
     prof_seg(c, SEG_K2);
     if (rc) return rc;
-    if (s->k2_sk) rc = launch_reduce_q_sk(c->st, s->Qpart, d.packed + packed_q(d), d.L, d.Mloc, d.H, d.ldB, s->sk_nk, s->sk_grid, d.sc);
+    if (s->k2_sk && !i8) rc = launch_reduce_q_sk(c->st, s->Qpart, d.packed + packed_q(d), d.L, d.Mloc, d.H, d.ldB, s->sk_nk, s->sk_grid, d.sc);
     else rc = k_reduce_q(c->st, d, s->Qpart, s->S);
     prof_seg(c, SEG_REDUCE_Q);
     return rc;
@@ -1658,8 +1778,22 @@ extern "C" int vbmf_b200_gemm_YtB(vbmf_b200_ctx* c, const double* B, int64_t H, 
     VB_CUDA_OK(cudaMemsetAsync(dB, 0, (size_t)H * ldB * 8, c->st));
     VB_CUDA_OK(cudaMemcpy2DAsync(dB, (size_t)ldB * 8, B, (size_t)c->L * 8, (size_t)c->L * 8, (size_t)H, cudaMemcpyHostToDevice, c->st));
     int rc = 0;
-    if (c->simt) rc = launch_gemm_ytb_simt(c->st, c->Y, c->ldY, dB, ldB, dP, c->Mloc, c->L, (int)H, (int)H, nullptr);
-    else {
+    bool i8 = false;
+    I8Operands o;
+    int S1 = 1, kbs1 = 1, S2 = 1, kc2 = 32;
+    if (ctx_int8_wanted(c, H)) {
+        i8_plans(c->L, c->Mloc, (int)H, c->num_sms, &S1, &kbs1, &S2, &kc2);
+        rc = ctx_slices(c, &i8);
+        if (!rc && i8) rc = i8_operands_alloc(&o, c->L, c->Mloc, (int)H, S2, &i8);
+    }
+    if (!rc && i8) {
+        double* dPp = nullptr;
+        if (S1 > 1 && cudaMalloc(&dPp, (size_t)S1 * MH * 8) != cudaSuccess) { set_error("cudaMalloc failed"); rc = -1; }
+        if (!rc) rc = i8_k1(c, &o, dB, ldB, (int)H, S1 > 1 ? dPp : dP, S1, kbs1, nullptr);
+        if (!rc && S1 > 1) rc = k_sum_slabs(c->st, dPp, S1, MH, dP, nullptr);
+        if (dPp) { cudaStreamSynchronize(c->st); cudaFree(dPp); }
+    } else if (!rc && c->simt) rc = launch_gemm_ytb_simt(c->st, c->Y, c->ldY, dB, ldB, dP, c->Mloc, c->L, (int)H, (int)H, nullptr);
+    else if (!rc) {
         CUtensorMap tmB;
         rc = make_tmap_2d(&tmB, dB, (uint64_t)c->L, (uint64_t)H, (uint64_t)ldB * 8, 16, (uint32_t)gemm_geometry((int)H).bn);
         int S1 = 1, kbs1 = 1;
@@ -1687,9 +1821,17 @@ extern "C" int vbmf_b200_gemm_YA(vbmf_b200_ctx* c, const double* A, int64_t H, d
     const size_t MH = (size_t)std::max(c->Mloc, 1) * H;
     int S = 1, kchunk = 16;
     plan_splitk(c->L, c->Mloc, (int)H, c->num_sms, &S, &kchunk);
+    bool i8 = false;
+    I8Operands o;
+    if (ctx_int8_wanted(c, H)) {
+        int S1 = 1, kbs1 = 1;
+        i8_plans(c->L, c->Mloc, (int)H, c->num_sms, &S1, &kbs1, &S, &kchunk);
+        if (ctx_slices(c, &i8)) return -1;
+        if (i8 && i8_operands_alloc(&o, c->L, c->Mloc, (int)H, S, &i8)) return -1;
+    }
     int kq = 64, nk = 1, skgrid = 1, smax = 1;
     const char* ek2 = getenv("VBMF_B200_K2");
-    const bool use_sk = !(c->simt || (H % 2 != 0)) && c->Mloc > 0 && ek2 != nullptr && strcmp(ek2, "streamk") == 0;
+    const bool use_sk = !i8 && !(c->simt || (H % 2 != 0)) && c->Mloc > 0 && ek2 != nullptr && strcmp(ek2, "streamk") == 0;
     if (use_sk) { plan_streamk(c->L, c->Mloc, (int)H, c->num_sms, &kq, &nk, &skgrid, &smax); S = std::max(S, smax); }
     double *dA = nullptr, *dT = nullptr, *dQp = nullptr, *dQ = nullptr;
     VB_CUDA_OK(cudaMalloc(&dA, MH * 8));
@@ -1701,7 +1843,8 @@ extern "C" int vbmf_b200_gemm_YA(vbmf_b200_ctx* c, const double* A, int64_t H, d
     int rc = k_transpose(c->st, dT, dA, c->Mloc, (int)H);
     const bool simt = c->simt || (H % 2 != 0);
     if (!rc) {
-        if (simt) rc = launch_gemm_ya_simt(c->st, c->Y, c->ldY, dA, dQp, c->L, c->Mloc, (int)H, ldQ, kchunk, S, nullptr);
+        if (i8) rc = i8_k2(c, &o, dA, (int)H, dQp, ldQ, S, kchunk, nullptr);
+        else if (simt) rc = launch_gemm_ya_simt(c->st, c->Y, c->ldY, dA, dQp, c->L, c->Mloc, (int)H, ldQ, kchunk, S, nullptr);
         else {
             CUtensorMap tmA;
             if (c->Mloc > 0) rc = make_tmap_2d(&tmA, dA, (uint64_t)H, (uint64_t)c->Mloc, (uint64_t)H * 8, 16, 16);

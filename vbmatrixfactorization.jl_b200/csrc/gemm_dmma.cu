@@ -566,23 +566,25 @@ __global__ void __launch_bounds__(256) reduce_q_sk_kernel(const double* __restri
 }
 
 // ------------------------------------------------------------------------------------------- host side
-typedef CUresult (*PFN_encodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                    const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                    CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 static PFN_encodeTiled g_encode = nullptr;
 
-int make_tmap_2d(CUtensorMap* out, const void* base, uint64_t dim0, uint64_t dim1, uint64_t stride1_bytes,
-                 uint32_t box0, uint32_t box1) {
+PFN_encodeTiled tmap_encoder() {
     if (!g_encode) {
         void* fn = nullptr;
         cudaDriverEntryPointQueryResult qres;
         cudaError_t e = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres);
         if (e != cudaSuccess || fn == nullptr || qres != cudaDriverEntryPointSuccess) {
             set_error("cuTensorMapEncodeTiled entry point not available (%s)", cudaGetErrorString(e));
-            return -1;
+            return nullptr;
         }
         g_encode = (PFN_encodeTiled)fn;
     }
+    return g_encode;
+}
+
+int make_tmap_2d(CUtensorMap* out, const void* base, uint64_t dim0, uint64_t dim1, uint64_t stride1_bytes,
+                 uint32_t box0, uint32_t box1) {
+    if (!tmap_encoder()) return -1;
     if ((reinterpret_cast<uintptr_t>(base) & 15) != 0 || (stride1_bytes & 15) != 0) {
         set_error("TMA tensor map needs 16-byte aligned base and pitch (base=%p pitch=%llu)", base,
                   (unsigned long long)stride1_bytes);
@@ -681,7 +683,7 @@ int gemm_init_device() {
     VB_CUDA_OK(cudaFuncSetAttribute(gemm_ya_sk_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, Sizes<32>::SMEM));
     VB_CUDA_OK(cudaFuncSetAttribute(gemm_ya_sk_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, Sizes<64>::SMEM));
     VB_CUDA_OK(cudaFuncSetAttribute(gemm_ya_sk_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, Sizes<128>::SMEM));
-    return 0;
+    return gemm_i8_init_device();
 }
 
 int launch_gemm_ytb(cudaStream_t st, const CUtensorMap* tmY, const CUtensorMap* tmB, double* P, int M, int L, int H,
