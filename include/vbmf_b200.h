@@ -269,17 +269,25 @@ int vbmf_b200_solver_lower_bound(vbmf_b200_solver* s, double trim, int trimmed, 
 int vbmf_b200_solver_yhat(vbmf_b200_solver* s, double* YHat, int64_t ld);
 
 /* ---- batched small problems (the MIL classification pattern) ---- */
-/* vbls! (examples/mil_util.jl:179-203) for nprob independent problems in ONE kernel launch, one CTA per problem:
+/* vbls! (examples/mil_util.jl:179-203) for nprob independent problems in one call on the context's stream:
  * niter x { updateA!, updateCA!, updateSigma! } with BHat fixed, then updateYHat! -- what classify(...; class_alg="dual")
  * runs for every test bag and class model (examples/mil_util.jl:504-511; class_alg = "vbls" :470-478 for dense parameters).
  * kind = VBMF_B200_DENSE, _SPARSE, _DUAL or _TRIAL (the four branches of vbls!, :182-197); states[p] points to the matching
  * state struct of problem p, Y[p] to its L x states[p]->M matrix.  All problems share L, H (and H0); M (and M0) may differ.
  * flags: VBMF_B200_FULL_COV, VBMF_B200_DIAG_VAR (both ignored for dense).  Needs no attached Y.  Limits: H <= 64 for sparse / dual /
- * trial (H > 32 with full_cov inverts one column at a time with the whole CTA) and H <= 32 for dense, no labels, the whole
- * problem must fit one CTA's shared memory (an error names the size otherwise); dense problems need a diagonal invCA (what
- * vbmf_init creates and updateCA! maintains). */
+ * trial (H > 32 with full_cov inverts one column at a time with the whole CTA) and H <= 32 for dense, no labels; dense
+ * problems need a diagonal invCA (what vbmf_init creates and updateCA! maintains).  A problem whose whole state fits one
+ * CTA's shared memory runs in a one-CTA-per-problem kernel (one launch for all of them); a larger one runs in the wide
+ * kernel, one thread-block cluster of 1, 2, 4 or 8 CTAs per problem (one launch per cluster size), see
+ * vbmf_b200_batched_plan. */
 int vbmf_b200_batched_vbls(vbmf_b200_ctx* ctx, int kind, int64_t nprob, const double* const* Y, void* const* states,
                            int64_t niter, int flags);
+/* How vbmf_b200_batched_vbls runs each problem of a batch (host only, needs no GPU): cluster_out[p] = 0 when problem p (M[p]
+ * columns) fits the one-CTA kernel, else the cluster size 1, 2, 4 or 8 of the wide kernel: the smallest whose per-CTA column
+ * share stays within a fixed bound, at most 8.  full_cov / diag_var are 0 or 1 (ignored for dense).  Fails for H out of range
+ * (H <= 64, dense H <= 32), an unknown kind or M[p] < 1. */
+int vbmf_b200_batched_plan(int kind, int64_t L, int64_t H, int full_cov, int diag_var, int64_t nprob, const int64_t* M,
+                           int32_t* cluster_out);
 
 /* ---- one-call drop-ins: upload + loop + updateYHat! + download ---- */
 /* vbmf!(Y, params, niter; eps, est_covs, est_var)   src/vbmf.jl:175 */

@@ -328,9 +328,10 @@ end
 vbmf_trial!(Y::Array{Float64,2}, p::vbmf_trial_parameters, niter::Int; kw...) = vbmf_trial!(default_context(), Y, p, niter; kw...)
 vbmf_trial(Y::Array{Float64,2}, p_in::vbmf_trial_parameters, niter::Int; kw...) = vbmf_trial(default_context(), Y, p_in, niter; kw...)
 
-# ---- vbls! for many bags in one launch (examples/mil_util.jl:179-203, 504-511) --------------------------------------------------
+# ---- vbls! for many bags in one call (examples/mil_util.jl:179-203, 504-511) ----------------------------------------------------
 # Ys[k] is the L x M_k matrix of problem k, ps[k] its parameters (all of one type, with the same L, H, H0); one method per
-# branch of vbls! (:182-197).  kind: 0 dense, 1 sparse, 2 dual, 3 trial (include/vbmf_b200.h).
+# branch of vbls! (:182-197).  kind: 0 dense, 1 sparse, 2 dual, 3 trial (include/vbmf_b200.h).  Bags of any size: those
+# too large for one CTA's shared memory run in the wide kernel (one thread-block cluster per bag) within the same call.
 function batched_call(ctx::B200Context, kind::Int, Ys::Vector{Array{Float64,2}}, sts::Vector, niter::Int, flags::Int)
     yptr = Ptr{Float64}[pointer(Y) for Y in Ys]
     sptr = Ptr{Void}[convert(Ptr{Void}, Base.unsafe_convert(Ptr{eltype(r)}, r)) for r in sts]

@@ -104,6 +104,7 @@ SYMBOLS = {
     "vbmf_b200_solver_lower_bound": (C.c_int, [C.c_void_p, c_f64, C.c_int, p_f64]),
     "vbmf_b200_solver_yhat": (C.c_int, [C.c_void_p, p_f64, c_i64]),
     "vbmf_b200_batched_vbls": (C.c_int, [C.c_void_p, C.c_int, c_i64, C.POINTER(p_f64), C.POINTER(C.c_void_p), c_i64, C.c_int]),
+    "vbmf_b200_batched_plan": (C.c_int, [C.c_int, c_i64, c_i64, C.c_int, C.c_int, c_i64, p_i64, C.c_void_p]),
     "vbmf_b200_dense_run": (C.c_int, [C.c_void_p, C.POINTER(DenseState), c_i64, c_f64, C.c_int, C.c_int, C.c_int, p_i64, p_f64]),
     "vbmf_b200_sparse_run": (C.c_int, [C.c_void_p, C.POINTER(SparseState), c_i64, c_f64, C.c_int, C.c_int, C.c_int, C.c_int, p_i64, p_f64]),
     "vbmf_b200_dual_run": (C.c_int, [C.c_void_p, C.POINTER(DualState), c_i64, c_f64, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, p_i64, p_f64]),

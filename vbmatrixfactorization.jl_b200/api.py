@@ -936,10 +936,11 @@ class BatchedVbls:
 
 
 def vbls_batched_(Ys, params_list, niter, full_cov=False, diag_var=False, ctx=None, yhat=True, keep_blocks=False):
-    """`vbls!` (examples/mil_util.jl:179-203) for many small problems in ONE kernel launch (one CTA per problem): the MIL
-    classification pattern, classify(...; class_alg = "dual") runs it for every test bag and class model.  All params must
-    be of one type (vbmf_parameters, vbmf_sparse_parameters, vbmf_dual_parameters or vbmf_trial_parameters - the four
-    branches of vbls!) with the same L, H (and H0); M (and M0) may differ per problem."""
+    """`vbls!` (examples/mil_util.jl:179-203) for many problems in ONE C-ABI call (one CTA per problem; problems too large
+    for one CTA's shared memory get a thread-block cluster each): the MIL classification pattern, classify(...; class_alg =
+    "dual") runs it for every test bag and class model.  All params must be of one type (vbmf_parameters,
+    vbmf_sparse_parameters, vbmf_dual_parameters or vbmf_trial_parameters - the four branches of vbls!) with the same L, H
+    (and H0); M (and M0) may differ per problem."""
     batch = BatchedVbls(Ys, params_list, ctx=ctx, yhat=yhat, keep_blocks=keep_blocks)
     batch.run(niter, full_cov=full_cov, diag_var=diag_var)
     return batch.readback()

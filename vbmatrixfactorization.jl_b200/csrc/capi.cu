@@ -1921,20 +1921,6 @@ extern "C" int vbmf_b200_trial_run(vbmf_b200_ctx* c, vbmf_b200_trial_state* st, 
 }
 
 // ---- K11: batched vbls! ----------------------------------------------------------------------------------------------------
-namespace vb {
-struct BatchDesc {
-    int nprob, L, H, H0, kind, niter, full_cov, Mmax;
-    const int* moff; const double* Y; const double* B; const double* SigmaB;
-    double* A; double* CA; double* beta; double* sdiag; double* SigmaA; double* blocks; double* YHat; double* scal;
-    int diag_var; double* sigmaVec; const double* etaVec; double* zetaVec;
-};
-struct BatchDenseDesc {
-    int nprob, L, H, niter, Mmax;
-    const int* moff; const double* Y; const double* B; const double* SigmaB;
-    double* A; double* SigmaA; double* icA; double* cA; double* YHat; double* scal;
-};
-int k_batched_vbls_dense(cudaStream_t st, const BatchDenseDesc& bd);
-}
 
 // host-side packing / unpacking of many small problems: a few threads over disjoint problem ranges (plain memcpy work)
 template <class F> static void parallel_for(int64_t n, F&& fn) {
@@ -1966,6 +1952,40 @@ static int batch_reserve(vbmf_b200_ctx* c, size_t total) {
     return 0;
 }
 
+// Routes every problem of a batch (batched_cluster_size) and orders them for the launches: plist = the one-CTA problems,
+// then those of cluster size 1, 2, 4, 8; n[g] = count of group g; Mmax0 = largest M of the one-CTA problems.
+static void batch_route(int kind, int L, int H, const std::vector<int>& moff, std::vector<int>& plist, int (&n)[5], int& Mmax0) {
+    const int nprob = (int)moff.size() - 1;
+    std::vector<int> grp(nprob);
+    for (int g = 0; g < 5; ++g) n[g] = 0;
+    Mmax0 = 0;
+    for (int p = 0; p < nprob; ++p) {
+        const int M = moff[p + 1] - moff[p], cs = vb::batched_cluster_size(kind, L, H, M);
+        int g = 0;
+        while (g < 4 && cs > (g == 0 ? 0 : 1 << (g - 1))) ++g;
+        grp[p] = g;
+        ++n[g];
+        if (g == 0) Mmax0 = std::max(Mmax0, M);
+    }
+    plist.clear();
+    for (int g = 0; g < 5; ++g) for (int p = 0; p < nprob; ++p) if (grp[p] == g) plist.push_back(p);
+}
+
+extern "C" int vbmf_b200_batched_plan(int kind, int64_t L, int64_t H, int full_cov, int diag_var, int64_t nprob, const int64_t* M,
+                                      int32_t* cluster_out) {
+    if (kind < VBMF_B200_DENSE || kind > VBMF_B200_TRIAL) { set_error("batched_plan: unknown parameter kind %d", kind); return -1; }
+    const int64_t Hmax = kind == VBMF_B200_DENSE ? 32 : 64;
+    if (H < 1 || H > Hmax) { set_error("batched vbls supports 1 <= H <= %lld (got H = %lld)", (long long)Hmax, (long long)H); return -1; }
+    if (L < 1 || L > 0x7fffff00LL || nprob < 0 || (nprob > 0 && (!M || !cluster_out)) || (full_cov != 0 && full_cov != 1) ||
+        (diag_var != 0 && diag_var != 1)) {
+        set_error("batched_plan: bad argument"); return -1;
+    }
+    for (int64_t p = 0; p < nprob; ++p)
+        if (M[p] < 1 || M[p] > 0x7fffff00LL) { set_error("batched_plan: bad argument (M of problem %lld)", (long long)p); return -1; }
+    for (int64_t p = 0; p < nprob; ++p) cluster_out[p] = vb::batched_cluster_size(kind, (int)L, (int)H, (int)M[p]);
+    return 0;
+}
+
 template <class ST> struct BatchView {
     static const ST* get(void* const* states, int64_t p) { return (const ST*)states[p]; }
 };
@@ -1983,7 +2003,6 @@ static int batched_vbls_impl(vbmf_b200_ctx* c, int kind, int64_t nprob, const do
     if (L < 1 || H < 1 || H > 64) { set_error("batched vbls supports 1 <= H <= 64 (got H = %lld)", (long long)H); return -1; }
     if (H0 < 0 || H0 > H) { set_error("H must be at least H0!"); return -1; }
     std::vector<int> moff(nprob + 1, 0);
-    int Mmax = 0;
     bool want_yhat = false, want_blocks = false;
     for (int64_t p = 0; p < nprob; ++p) {
         const ST* s = (const ST*)states[p];
@@ -1993,7 +2012,6 @@ static int batched_vbls_impl(vbmf_b200_ctx* c, int kind, int64_t nprob, const do
         else { if (s->n_labels > 0 && s->H1 > 0) { set_error("batched vbls: labels are not supported"); return -1; } }
         if (dvar && (s->sigmaVecHat == nullptr || s->etaVec == nullptr)) { set_error("batched vbls: diag_var needs sigmaVecHat / etaVec of problem %lld", (long long)p); return -1; }
         moff[p + 1] = moff[p] + (int)s->M;
-        Mmax = std::max<int>(Mmax, (int)s->M);
         want_yhat = want_yhat || s->YHat != nullptr;
         want_blocks = want_blocks || s->SigmaATVec_blocks != nullptr;
     }
@@ -2003,7 +2021,12 @@ static int batched_vbls_impl(vbmf_b200_ctx* c, int kind, int64_t nprob, const do
     //      upload is one copy of [0, up_end) and the whole download one copy of [down_begin, total)
     size_t off = 0;
     auto take = [&](size_t bytes) { const size_t o = off; off += align_up(bytes, 256); return o; };
-    const size_t o_moff = take((size_t)(nprob + 1) * 4), o_Y = take(L * Mtot * 8), o_B = take(nprob * LH * 8), o_SB = take(nprob * HH * 8);
+    std::vector<int> plist;
+    int ngrp[5], Mmax0;
+    batch_route(kind, (int)L, (int)H, moff, plist, ngrp, Mmax0);
+    const bool wide = ngrp[0] < nprob;
+    const size_t o_moff = take((size_t)(nprob + 1) * 4), o_pl = take((size_t)nprob * 4), o_Y = take(L * Mtot * 8), o_B = take(nprob * LH * 8),
+                 o_SB = take(nprob * HH * 8);
     const size_t down_begin = off;
     const size_t o_CA = take(MH * 8), o_sc = take((size_t)nprob * 16 * 8);
     const size_t o_sv = dvar ? take((size_t)nprob * L * 8) : 0, o_ev = dvar ? take((size_t)nprob * L * 8) : 0;
@@ -2012,11 +2035,14 @@ static int batched_vbls_impl(vbmf_b200_ctx* c, int kind, int64_t nprob, const do
     const size_t o_zv = dvar ? take((size_t)nprob * L * 8) : 0;
     const size_t o_YH = want_yhat ? take(L * Mtot * 8) : 0, o_blk = want_blocks ? take(MH * H * 8) : 0;
     const size_t total = off;
-    if (batch_reserve(c, total)) return -1;
+    // device-only working storage of the wide kernel, neither uploaded nor downloaded
+    const size_t o_V = wide ? take(MH * 8) : 0, o_rv = wide && dvar ? take((size_t)nprob * (1 + BATCH_MAX_CLUSTER) * L * 8) : 0;
+    if (batch_reserve(c, off)) return -1;
     char* hb = c->batch_host;
     char* db = c->batch_dev;
     // ---- pack
     memcpy(hb + o_moff, moff.data(), (size_t)(nprob + 1) * 4);
+    memcpy(hb + o_pl, plist.data(), (size_t)nprob * 4);
     double *hY = (double*)(hb + o_Y), *hB = (double*)(hb + o_B), *hSB = (double*)(hb + o_SB), *hCA = (double*)(hb + o_CA), *hsc = (double*)(hb + o_sc);
     memset(hsc, 0, (size_t)nprob * 16 * 8);
     parallel_for(nprob, [&](int64_t p) {
@@ -2042,7 +2068,7 @@ static int batched_vbls_impl(vbmf_b200_ctx* c, int kind, int64_t nprob, const do
     if (cudaMemcpyAsync(db, hb, up_end, cudaMemcpyHostToDevice, st) != cudaSuccess) { cudaGetLastError(); set_error("batched vbls: upload failed"); return -1; }
     BatchDesc bd;
     bd.nprob = (int)nprob; bd.L = (int)L; bd.H = (int)H; bd.H0 = (int)H0; bd.kind = kind; bd.niter = (int)std::max<int64_t>(niter, 0);
-    bd.full_cov = (flags & F_FULL_COV) ? 1 : 0; bd.Mmax = Mmax;
+    bd.full_cov = (flags & F_FULL_COV) ? 1 : 0; bd.Mmax = Mmax0;
     bd.moff = (const int*)(db + o_moff); bd.Y = (const double*)(db + o_Y); bd.B = (const double*)(db + o_B); bd.SigmaB = (const double*)(db + o_SB);
     bd.A = (double*)(db + o_A); bd.CA = (double*)(db + o_CA); bd.beta = (double*)(db + o_beta); bd.sdiag = (double*)(db + o_s);
     bd.SigmaA = (double*)(db + o_SA); bd.blocks = want_blocks ? (double*)(db + o_blk) : nullptr; bd.YHat = want_yhat ? (double*)(db + o_YH) : nullptr;
@@ -2050,8 +2076,11 @@ static int batched_vbls_impl(vbmf_b200_ctx* c, int kind, int64_t nprob, const do
     bd.diag_var = dvar ? 1 : 0;
     bd.sigmaVec = dvar ? (double*)(db + o_sv) : nullptr; bd.etaVec = dvar ? (const double*)(db + o_ev) : nullptr;
     bd.zetaVec = dvar ? (double*)(db + o_zv) : nullptr;
-    prof_mark(c, c->ev_k1);       // profiling: the kernel alone (read back through vbmf_b200_ctx_profile_read, K1 slot)
-    if (bd.niter > 0) rc = k_batched_vbls(st, bd);
+    bd.plist = (const int*)(db + o_pl);
+    bd.V = wide ? (double*)(db + o_V) : nullptr;
+    bd.rowv = wide && dvar ? (double*)(db + o_rv) : nullptr;
+    prof_mark(c, c->ev_k1);       // profiling: the kernels alone (read back through vbmf_b200_ctx_profile_read, K1 slot)
+    if (bd.niter > 0) rc = k_batched_vbls(st, bd, ngrp, Mmax0);
     prof_mark(c, c->ev_k1);
     // ---- download + unpack
     if (!rc && bd.niter > 0 && cudaMemcpyAsync(hb + down_begin, db + down_begin, total - down_begin, cudaMemcpyDeviceToHost, st) != cudaSuccess) {
@@ -2131,7 +2160,6 @@ static int batched_vbls_dense_impl(vbmf_b200_ctx* c, int64_t nprob, const double
     const int64_t L = s0->L, H = s0->H;
     if (L < 1 || H < 1 || H > 32) { set_error("batched vbls supports 1 <= H <= 32 (got H = %lld)", (long long)H); return -1; }
     std::vector<int> moff(nprob + 1, 0);
-    int Mmax = 0;
     bool want_yhat = false;
     for (int64_t p = 0; p < nprob; ++p) {
         const ST* s = (const ST*)states[p];
@@ -2141,24 +2169,30 @@ static int batched_vbls_dense_impl(vbmf_b200_ctx* c, int64_t nprob, const double
         for (int64_t a = 0; a < H; ++a) for (int64_t b = 0; b < H; ++b)
             if (a != b && s->invCA[a + b * H] != 0.0) { set_error("batched vbls: invCA of problem %lld is not diagonal", (long long)p); return -1; }
         moff[p + 1] = moff[p] + (int)s->M;
-        Mmax = std::max<int>(Mmax, (int)s->M);
         want_yhat = want_yhat || s->YHat != nullptr;
     }
     const size_t Mtot = (size_t)moff[nprob], MH = Mtot * H, HH = (size_t)H * H, LH = (size_t)L * H;
     VB_CUDA_OK(cudaSetDevice(c->device));
     size_t off = 0;
     auto take = [&](size_t bytes) { const size_t o = off; off += align_up(bytes, 256); return o; };
-    const size_t o_moff = take((size_t)(nprob + 1) * 4), o_Y = take(L * Mtot * 8), o_B = take(nprob * LH * 8), o_SB = take(nprob * HH * 8);
+    std::vector<int> plist;
+    int ngrp[5], Mmax0;
+    batch_route(VBMF_B200_DENSE, (int)L, (int)H, moff, plist, ngrp, Mmax0);
+    const bool wide = ngrp[0] < nprob;
+    const size_t o_moff = take((size_t)(nprob + 1) * 4), o_pl = take((size_t)nprob * 4), o_Y = take(L * Mtot * 8), o_B = take(nprob * LH * 8),
+                 o_SB = take(nprob * HH * 8);
     const size_t down_begin = off;
     const size_t o_ic = take(nprob * H * 8), o_sc = take((size_t)nprob * 16 * 8);
     const size_t up_end = off;
     const size_t o_A = take(MH * 8), o_SA = take(nprob * HH * 8), o_c = take(nprob * H * 8);
     const size_t o_YH = want_yhat ? take(L * Mtot * 8) : 0;
     const size_t total = off;
-    if (batch_reserve(c, total)) return -1;
+    const size_t o_V = wide ? take(MH * 8) : 0;      // device-only working storage of the wide kernel
+    if (batch_reserve(c, off)) return -1;
     char* hb = c->batch_host;
     char* db = c->batch_dev;
     memcpy(hb + o_moff, moff.data(), (size_t)(nprob + 1) * 4);
+    memcpy(hb + o_pl, plist.data(), (size_t)nprob * 4);
     double *hY = (double*)(hb + o_Y), *hB = (double*)(hb + o_B), *hSB = (double*)(hb + o_SB), *hic = (double*)(hb + o_ic), *hsc = (double*)(hb + o_sc);
     memset(hsc, 0, (size_t)nprob * 16 * 8);
     for (int64_t p = 0; p < nprob; ++p) {
@@ -2172,13 +2206,14 @@ static int batched_vbls_dense_impl(vbmf_b200_ctx* c, int64_t nprob, const double
     cudaStream_t st = c->st;
     if (cudaMemcpyAsync(db, hb, up_end, cudaMemcpyHostToDevice, st) != cudaSuccess) { cudaGetLastError(); set_error("batched vbls: upload failed"); return -1; }
     BatchDenseDesc bd;
-    bd.nprob = (int)nprob; bd.L = (int)L; bd.H = (int)H; bd.niter = (int)std::max<int64_t>(niter, 0); bd.Mmax = Mmax;
+    bd.nprob = (int)nprob; bd.L = (int)L; bd.H = (int)H; bd.niter = (int)std::max<int64_t>(niter, 0); bd.Mmax = Mmax0;
     bd.moff = (const int*)(db + o_moff); bd.Y = (const double*)(db + o_Y); bd.B = (const double*)(db + o_B); bd.SigmaB = (const double*)(db + o_SB);
     bd.A = (double*)(db + o_A); bd.SigmaA = (double*)(db + o_SA); bd.icA = (double*)(db + o_ic); bd.cA = (double*)(db + o_c);
     bd.YHat = want_yhat ? (double*)(db + o_YH) : nullptr; bd.scal = (double*)(db + o_sc);
+    bd.plist = (const int*)(db + o_pl); bd.V = wide ? (double*)(db + o_V) : nullptr;
     int rc = 0;
     prof_mark(c, c->ev_k1);
-    if (bd.niter > 0) rc = k_batched_vbls_dense(st, bd);
+    if (bd.niter > 0) rc = k_batched_vbls_dense(st, bd, ngrp, Mmax0);
     prof_mark(c, c->ev_k1);
     if (!rc && bd.niter > 0 && cudaMemcpyAsync(hb + down_begin, db + down_begin, total - down_begin, cudaMemcpyDeviceToHost, st) != cudaSuccess) {
         cudaGetLastError(); set_error("batched vbls: download failed"); rc = -1;

@@ -139,8 +139,53 @@ int k_finish_stats(cudaStream_t st, double* v, int L, double n, int mode);
 int k_compact_rows(cudaStream_t st, const double* Y, int ldY, double* out, int ldo, const int* rows, int Lnew, int M, double lambda);
 int k_scale_all(cudaStream_t st, double* Y, size_t n, double lambda);
 
-// K11: batched one-CTA-per-problem vbls! (csrc/batched.cu)
-struct BatchDesc;
-int k_batched_vbls(cudaStream_t st, const BatchDesc& bd);
+// K11: batched vbls! (csrc/batched.cu).  A problem whose whole state fits one CTA's shared memory runs in the
+// one-CTA-per-problem kernel; a larger one runs in the wide kernel, one thread-block cluster of CS CTAs per problem.
+struct BatchDesc {
+    int nprob, L, H, H0, kind, niter, full_cov, Mmax;
+    const int* moff;        // [nprob+1] column offsets into the packed per-column arrays
+    const double* Y;        // [L][Mtot] column-major, problems concatenated
+    const double* B;        // [nprob][L*H] column-major L x H
+    const double* SigmaB;   // [nprob][H*H]
+    double* A;              // [Mtot][H]   in: unused (vbls overwrites), out: AHat rows
+    double* CA;             // [Mtot*H]    in/out
+    double* beta;           // [Mtot*H]    out
+    double* sdiag;          // [Mtot*H]    out
+    double* SigmaA;         // [nprob][H*H] out
+    double* blocks;         // [Mtot][H][H] out or nullptr
+    double* YHat;           // [L][Mtot] out or nullptr
+    double* scal;           // [nprob][16]: 0 sigmaHat 1 eta 2 zeta 3 zeta0 4 trYTY 5 alpha (sparse) | M0 (trial) 6 beta0 (sparse)
+                            //              7 8 = prior (alpha, beta) of ARD group 0, 9 10 = group 1, 14 15 = group 2 (trial)
+                            //              out: 0 sigmaHat 2 zeta 11 12 6 = alpha of groups 0 1 2, 13 fail
+    int diag_var;           // heteroscedastic noise (src/vbmf_sparse.jl:176-247 diag_var branches, :309-316)
+    double* sigmaVec;       // [nprob][L]  in/out  (diag_var)
+    const double* etaVec;   // [nprob][L]  in      (diag_var)
+    double* zetaVec;        // [nprob][L]  out     (diag_var)
+    const int* plist;       // problem of each launched CTA (one-CTA kernel) or cluster (wide kernel)
+    double* V;              // wide kernel: [Mtot][H] V = B'Y (diag_var: B'diag(sv)Y)
+    double* rowv;           // wide kernel, diag_var: [nprob][1 + 8][L] = ||Y[l,:]||^2 | per-rank partials of Y[l,:]*(A*b_l)
+};
+struct BatchDenseDesc {
+    int nprob, L, H, niter, Mmax;
+    const int* moff;
+    const double* Y;        // [L][Mtot]
+    const double* B;        // [nprob][L*H]
+    const double* SigmaB;   // [nprob][H*H]
+    double* A;              // [Mtot][H] out
+    double* SigmaA;         // [nprob][H*H] out
+    double* icA;            // [nprob][H] in: diag(invCA), out: diag(invCA)
+    double* cA;             // [nprob][H] out: diag(CA)
+    double* YHat;           // [L][Mtot] out or nullptr
+    double* scal;           // [nprob][16]
+    const int* plist;       // as BatchDesc::plist
+    double* V;              // wide kernel: [Mtot][H] V = B'Y
+};
+constexpr int BATCH_MAX_CLUSTER = 8;   // portable thread-block cluster size
+// CTAs of the wide kernel per problem: 0 = the problem fits the one-CTA kernel, else 1, 2, 4 or 8; -1 = H out of range
+int batched_cluster_size(int kind, int L, int H, int M);
+// Launches over a batch whose problems are grouped by cluster size: plist[0, n[0]) one-CTA problems (largest M: Mmax0),
+// then n[1], n[2], n[3], n[4] problems for CS = 1, 2, 4, 8.
+int k_batched_vbls(cudaStream_t st, const BatchDesc& bd, const int (&n)[5], int Mmax0);
+int k_batched_vbls_dense(cudaStream_t st, const BatchDenseDesc& bd, const int (&n)[5], int Mmax0);
 
 }  // namespace vb

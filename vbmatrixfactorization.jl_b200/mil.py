@@ -3,7 +3,8 @@
 SURVEY section 8(f) N1: `vbls!` (:179-203), `copy_vbmf_params` (:212-293), `train_dual` with its restarts (:327-385) and the
 classification loop built from them (`classify` :453-535, `test_classification` :557-588).  The reference classifies one bag
 at a time - two `vbls!` calls per bag, each a handful of tiny matrix products; here `classify_bags` puts every (bag, class
-model) pair of a whole test set into ONE launch of the one-CTA-per-problem kernel (`vbmf_b200_batched_vbls`).
+model) pair of a whole test set into ONE call of `vbmf_b200_batched_vbls`: one launch of the one-CTA-per-problem kernel, plus
+the wide kernel (one thread-block cluster per bag) for bags too large for one CTA's shared memory.
 
 Only the VB-based classifiers are mirrored ("vbls", "dual"); "ols"/"rls" are two-line host least-squares formulas with no VB
 update in them and stay with the caller.  The matrix norms of the L x M residuals follow Julia 0.5 (`norm(::Matrix)` =
