@@ -289,6 +289,17 @@ int vbmf_b200_batched_vbls(vbmf_b200_ctx* ctx, int kind, int64_t nprob, const do
 int vbmf_b200_batched_plan(int kind, int64_t L, int64_t H, int full_cov, int diag_var, int64_t nprob, const int64_t* M,
                            int32_t* cluster_out);
 
+/* lowerBound (trimmed = 0) / lowerBoundTrimmed (trimmed = 1) of nprob independent problems in one call, on the
+ * context's stream; out[p] = the ELBO of problem p.  src/vbmf_sparse.jl:435-489, src/vbmf_dual.jl:556-617,
+ * src/vbmf_trial.jl:630-697.  kind = VBMF_B200_SPARSE, _DUAL or _TRIAL (the dense kind has no lowerBound); states[p] and
+ * Y[p] as for vbmf_b200_batched_vbls, with the same limits: one L, H (and H0) for all problems, 1 <= H <= 64, M >= 1.
+ * Reads ATVecHat when it is set, else AHat, like the single solver's upload; trYTY comes from the state; labels play no part.
+ * Needs no attached Y and leaves the context's resident Y and its solvers alone.  A state whose arithmetic gives NaN (e.g.
+ * a negative beta) gives NaN for its own problem only.  Every problem is split over CTAs by its own M and H alone, so its
+ * bound is the same bit for bit whatever batch it is in. */
+int vbmf_b200_batched_lower_bound(vbmf_b200_ctx* ctx, int kind, int64_t nprob, const double* const* Y,
+                                  void* const* states, double trim, int trimmed, double* out);
+
 /* ---- one-call drop-ins: upload + loop + updateYHat! + download ---- */
 /* vbmf!(Y, params, niter; eps, est_covs, est_var)   src/vbmf.jl:175 */
 int vbmf_b200_dense_run(vbmf_b200_ctx* ctx, vbmf_b200_dense_state* st, int64_t niter, double eps, int est_covs, int est_var,

@@ -20,7 +20,7 @@ import VBMatrixFactorization: vbmf!, vbmf, vbmf_sparse!, vbmf_sparse, vbmf_dual!
                               lowerBound, lowerBoundTrimmed
 
 export b200_context, b200_close, b200_peer_exchange, b200_default_context!, vbmf!, vbmf, vbmf_sparse!, vbmf_sparse, vbmf_dual!, vbmf_dual, vbmf_trial!, vbmf_trial,
-       lowerBound, lowerBoundTrimmed, vbls_batched!, preprocess
+       lowerBound, lowerBoundTrimmed, vbls_batched!, lowerBound_batched, lowerBoundTrimmed_batched, preprocess
 
 const LIB = get(ENV, "VBMF_B200_LIB", "libvbmf_b200.so")
 
@@ -374,6 +374,37 @@ function vbls_batched!(ctx::B200Context, Ys::Vector{Array{Float64,2}}, ps::Vecto
     for (p, r) in zip(ps, sts); p.sigma2 = r[].sigma2; end
     return [p.AHat for p in ps]
 end
+
+# ---- lowerBound / lowerBoundTrimmed for many bags in one call (src/vbmf_sparse.jl:435-489, src/vbmf_dual.jl:556-617,
+# src/vbmf_trial.jl:630-697): the ELBO of every (bag, class model) pair, e.g. after vbls_batched!.  Same grouping rules as
+# vbls_batched! (one type, one L, H and H0; H <= 64); single-device contexts; needs no attached Y.  Returns a Vector{Float64}.
+function batched_lb_call(ctx::B200Context, kind::Int, Ys::Vector{Array{Float64,2}}, sts::Vector, trim::Float64, trimmed::Bool)
+    ctx.multi && error("the batched lowerBound runs on one device: use a single-device context")
+    yptr = Ptr{Float64}[pointer(Y) for Y in Ys]
+    sptr = Ptr{Void}[convert(Ptr{Void}, Base.unsafe_convert(Ptr{eltype(r)}, r)) for r in sts]
+    out = Array{Float64}(length(sts))
+    check(ccall((:vbmf_b200_batched_lower_bound, LIB), Cint,
+                (Ptr{Void}, Cint, Int64, Ptr{Ptr{Float64}}, Ptr{Ptr{Void}}, Float64, Cint, Ptr{Float64}),
+                ctx.handle, kind, length(sts), yptr, sptr, trim, trimmed, out))
+    return out
+end
+function batched_lower_bound(ctx::B200Context, Ys::Vector{Array{Float64,2}}, ps::Vector{vbmf_sparse_parameters}, trim::Float64, trimmed::Bool)
+    for p in ps; isdefined(p, :YHat) || (p.YHat = Array{Float64}(0, 0)); end
+    batched_lb_call(ctx, 1, Ys, [Ref(sparse_state(p, convert(Ptr{Float64}, C_NULL), false)) for p in ps], trim, trimmed)
+end
+function batched_lower_bound(ctx::B200Context, Ys::Vector{Array{Float64,2}}, ps::Vector{vbmf_dual_parameters}, trim::Float64, trimmed::Bool)
+    for p in ps; isdefined(p, :YHat) || (p.YHat = Array{Float64}(0, 0)); end
+    batched_lb_call(ctx, 2, Ys, [Ref(dual_state(p, false)) for p in ps], trim, trimmed)
+end
+function batched_lower_bound(ctx::B200Context, Ys::Vector{Array{Float64,2}}, ps::Vector{vbmf_trial_parameters}, trim::Float64, trimmed::Bool)
+    for p in ps; isdefined(p, :YHat) || (p.YHat = Array{Float64}(0, 0)); end
+    batched_lb_call(ctx, 3, Ys, [Ref(trial_state(p, false)) for p in ps], trim, trimmed)
+end
+batched_lower_bound(ctx::B200Context, Ys::Vector{Array{Float64,2}}, ps::Vector{vbmf_parameters}, trim::Float64, trimmed::Bool) =
+    error("the dense solver has no lowerBound (the reference defines none)")
+lowerBound_batched(ctx::B200Context, Ys::Vector{Array{Float64,2}}, ps::Vector) = batched_lower_bound(ctx, Ys, ps, 0.0, false)
+lowerBoundTrimmed_batched(ctx::B200Context, Ys::Vector{Array{Float64,2}}, ps::Vector, trim = 1e-1) =
+    batched_lower_bound(ctx, Ys, ps, Float64(trim), true)
 
 # ---- preprocess(Y, lambda) (src/util.jl:73-87) on the device; the processed matrix stays resident (pass `nothing` for Y to
 # the solvers to run on it without another upload); single-device contexts

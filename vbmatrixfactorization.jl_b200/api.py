@@ -6,7 +6,8 @@ Same names, argument meaning and error behaviour as the reference (Julia `f!` be
     vbmf_sparse_init / vbmf_sparse_ / vbmf_sparse  src/vbmf_sparse.jl:101,344,418
     vbmf_dual_init / vbmf_dual_ / vbmf_dual        src/vbmf_dual.jl:122,455,538
     updateA_, updateB_, updateCA_, updateCB_, updateSigma2_/updateSigma_, updateYHat_, updateAlpha00_ ...,
-    lowerBound, lowerBoundTrimmed, copy, vbls_ (examples/mil_util.jl:179)
+    lowerBound, lowerBoundTrimmed, copy, vbls_ (examples/mil_util.jl:179), vbls_batched_ / BatchedVbls and
+    lowerBound_batched / lowerBoundTrimmed_batched (many small problems in one call)
 
 Matrices are numpy arrays in Julia layout (Fortran order, Float64); labels are 1-based Int64.  The host keeps what the
 reference keeps on the host: initialisation (RNG), argument checking and struct marshalling.  Everything inside the
@@ -27,7 +28,7 @@ __all__ = [
     "vbmf_init", "vbmf_", "vbmf", "vbmf_sparse_init", "vbmf_sparse_", "vbmf_sparse", "vbmf_dual_init", "vbmf_dual_",
     "vbmf_dual", "updateA_", "updateB_", "updateCA_", "updateCB_", "updateSigma2_", "updateSigma_", "updateYHat_",
     "updateAlpha00_", "updateAlpha01_", "updateBeta00_", "updateBeta01_", "lowerBound", "lowerBoundTrimmed", "copy",
-    "vbls_", "vbls_batched_", "BatchedVbls", "preprocess", "VBMFWarning", "create_log", "update_log_", "save_log", "load_log", "extract_params_", "VBMFError",
+    "vbls_", "vbls_batched_", "BatchedVbls", "lowerBound_batched", "lowerBoundTrimmed_batched", "preprocess", "VBMFWarning", "create_log", "update_log_", "save_log", "load_log", "extract_params_", "VBMFError",
 ]
 
 VBMFError = L_.VBMFError
@@ -934,6 +935,26 @@ class BatchedVbls:
             _readback(p, st)
         return [p.AHat for p in self.params]
 
+    def lower_bound(self, trim=None):
+        """lowerBound (trim = None) or lowerBoundTrimmed(trim) of every problem in one C-ABI call
+        (`vbmf_b200_batched_lower_bound`) on the structs this object holds: after `run` they already point at the vbls
+        results, so nothing is marshalled again.  Returns a float64 array, one bound per problem."""
+        out = np.zeros(self.n)
+        if self.n == 0:
+            return out
+        if isinstance(self.ctx, MultiContext):
+            raise VBMFError("the batched lowerBound runs on one device: pass a single-device Context, not a MultiContext")
+        if self.kind == L_.DENSE:
+            raise VBMFError("the dense solver has no lowerBound (the reference defines none)")
+        for i, p in enumerate(self.params):
+            if _a_mismatch(p):
+                raise VBMFError("lowerBound: params.AHat and params.ATVecHat of problem %d disagree (the reference would mix the two "
+                                "copies); set both" % i)
+        L_.check(self.ctx.lib.vbmf_b200_batched_lower_bound(self.ctx.h, self.kind, self.n, self.yp, self.sp,
+                                                            0.0 if trim is None else float(trim), 0 if trim is None else 1,
+                                                            out.ctypes.data))
+        return out
+
 
 def vbls_batched_(Ys, params_list, niter, full_cov=False, diag_var=False, ctx=None, yhat=True, keep_blocks=False):
     """`vbls!` (examples/mil_util.jl:179-203) for many problems in ONE C-ABI call (one CTA per problem; problems too large
@@ -944,6 +965,19 @@ def vbls_batched_(Ys, params_list, niter, full_cov=False, diag_var=False, ctx=No
     batch = BatchedVbls(Ys, params_list, ctx=ctx, yhat=yhat, keep_blocks=keep_blocks)
     batch.run(niter, full_cov=full_cov, diag_var=diag_var)
     return batch.readback()
+
+
+def lowerBound_batched(Ys, params_list, ctx=None):
+    """`lowerBound` (src/vbmf_sparse.jl:435, src/vbmf_dual.jl:556, src/vbmf_trial.jl:630) of many problems in ONE C-ABI call:
+    the ELBO of every (bag, class model) pair of a MIL test set.  Same grouping rules as `vbls_batched_` (one parameter type
+    among sparse / dual / trial, the same L, H and H0; H <= 64), one device, no attached Y needed.  Returns a float64 array."""
+    return BatchedVbls(Ys, params_list, ctx=ctx, yhat=False).lower_bound()
+
+
+def lowerBoundTrimmed_batched(Ys, params_list, trim=1e-1, ctx=None):
+    """`lowerBoundTrimmed` (src/vbmf_sparse.jl:478, src/vbmf_dual.jl:606, src/vbmf_trial.jl:687) of many problems in one
+    call, as `lowerBound_batched`."""
+    return BatchedVbls(Ys, params_list, ctx=ctx, yhat=False).lower_bound(float(trim))
 
 
 def preprocess(Y, lam, verb=False, ctx=None):

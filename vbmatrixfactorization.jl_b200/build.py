@@ -9,7 +9,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "lib")
 LIB = os.path.join(LIBDIR, "libvbmf_b200.so")
 SOURCES = ["gemm_dmma.cu", "gemm_int8.cu", "kernels.cu", "batched.cu", "capi.cu", "multi.cu"]
-HEADERS = ["common.cuh", "gemm.cuh", "kernels.cuh", "linalg.cuh", os.path.join("..", "..", "include", "vbmf_b200.h")]
+HEADERS = ["common.cuh", "elbo.cuh", "gemm.cuh", "kernels.cuh", "linalg.cuh", os.path.join("..", "..", "include", "vbmf_b200.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC"]
 
 

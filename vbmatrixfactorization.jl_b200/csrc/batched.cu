@@ -7,6 +7,7 @@
 // Formulas: src/vbmf_sparse.jl:176-247 (updateA!, both covariance modes incl. Q2/Q3), :284-288 (updateCA!), :317-322
 // (updateSigma!, homoscedastic); src/vbmf_dual.jl:322-351 for the two-group ARD update.
 #include "kernels.cuh"
+#include "elbo.cuh"
 #include "linalg.cuh"
 #include <algorithm>
 #include <cooperative_groups.h>
@@ -892,6 +893,140 @@ int k_batched_vbls_dense(cudaStream_t st, const BatchDenseDesc& bd, const int (&
         else rc = launch_wide(batched_vbls_dense_wide_kernel<32>, b, n[g], CS, wsmem, st);
         if (rc) return rc;
     }
+    return 0;
+}
+
+
+// ---- K7 batched: lowerBound / lowerBoundTrimmed of many problems ---------------------------------------------------------
+// src/vbmf_sparse.jl:435-489, src/vbmf_dual.jl:556-617, src/vbmf_trial.jl:630-697 for every problem of the batch.  Y, AHat and
+// the per-column vectors stream from global memory, so nothing but H x H objects ever sits in shared memory.
+// Phase 1, one CTA per chunk of batched_lb_cols(H) columns: the 11 element sums of lb_partial_kernel, A'A and tr(B'*Y*A)
+// over the chunk's columns.  Phase 2, one CTA per problem: the chunk partials summed in chunk order, B'B, the traces, the LU
+// of SigmaB and the term assembly shared with the single solver (elbo.cuh).  Every sum has a fixed order, and the chunks of a
+// problem depend on its own M and H only, so its bound is the same bit for bit alone, in any batch and in every run.
+__global__ void __launch_bounds__(256) batched_lb_partial_kernel(BatchLbDesc bd) {
+    __shared__ double red[32];
+    __shared__ double wq[8];
+    const int c = blockIdx.x, p = bd.cprob[c];
+    const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
+    const int H = bd.H, L = bd.L, HH = H * H;
+    const int m0 = bd.moff[p], M = bd.moff[p + 1] - m0;
+    const int lo = (c - bd.coff[p]) * batched_lb_cols(H), hi = min(M, lo + batched_lb_cols(H));
+    const bool grouped = bd.kind == KIND_DUAL || bd.kind == KIND_TRIAL;
+    const int H0 = bd.H0, M0 = bd.m0[p];
+    const size_t eb = (size_t)m0 * H;
+    double* part = bd.part + (size_t)c * (LB_NPART + HH);
+    // the 11 sums of lb_partial_kernel
+    double a[11];
+#pragma unroll
+    for (int i = 0; i < 11; ++i) a[i] = 0.0;
+    for (int e = lo * H + t; e < hi * H; e += blockDim.x) {
+        const int m = e / H, h = e - m * H;
+        const int g = (!grouped || h < H0) ? 0 : (m < M0 ? 1 : 2);
+        lb_accumulate(a, g, bd.A[eb + e], bd.beta[eb + e], bd.CA[eb + e], bd.sdiag[eb + e], bd.trim, bd.trimmed);
+    }
+#pragma unroll
+    for (int i = 0; i < 11; ++i) {
+        const double v = block_sum(a[i], red);
+        if (t == 0) part[i] = v;
+    }
+    // A'A over the chunk: one element per thread, columns in order
+    const double* Ap = bd.A + eb;
+    for (int e = t; e < HH; e += blockDim.x) {
+        const int i = e / H, j = e - i * H;
+        double s = 0.0;
+        for (int m = lo; m < hi; ++m) s = fma(Ap[(size_t)m * H + i], Ap[(size_t)m * H + j], s);
+        part[LB_NPART + e] = s;
+    }
+    // tr(B'*Y*A) over the chunk = sum_m (B'y_m).a_m: one warp per column, the L-long dots split over the lanes
+    const double* Bp = bd.B + (size_t)p * L * H;
+    const double* Yp = bd.Y + (size_t)m0 * L;
+    double q = 0.0;
+    for (int m = lo + warp; m < hi; m += 8) {
+        const double* y = Yp + (size_t)m * L;
+        const double* am = Ap + (size_t)m * H;
+        for (int h = 0; h < H; ++h) {
+            double s = 0.0;
+            for (int l = lane; l < L; l += 32) s = fma(Bp[(size_t)h * L + l], y[l], s);
+            q = fma(warp_sum(s), am[h], q);
+        }
+    }
+    if (lane == 0) wq[warp] = q;
+    __syncthreads();
+    if (t == 0) {
+        double s = 0.0;
+        for (int w = 0; w < 8; ++w) s += wq[w];
+        part[11] = s;
+    }
+}
+
+__global__ void __launch_bounds__(256) batched_lb_final_kernel(BatchLbDesc bd) {
+    extern __shared__ double sm[];
+    __shared__ double acc[LB_NPART];
+    __shared__ double sh[2];
+    const int p = blockIdx.x, t = threadIdx.x, nt = blockDim.x;
+    const int H = bd.H, L = bd.L, HH = H * H;
+    double* AtA = sm;           // [H][H], later the LU scratch of SigmaB
+    double* BtB = sm + HH;      // [H][H]
+    const int c0 = bd.coff[p], nc = bd.coff[p + 1] - c0;
+    const size_t stride = LB_NPART + HH;
+    const double* part = bd.part + (size_t)c0 * stride;
+    for (int i = t; i < LB_NPART; i += nt) {
+        double s = 0.0;
+        for (int c = 0; c < nc; ++c) s += part[c * stride + i];
+        acc[i] = s;
+    }
+    for (int e = t; e < HH; e += nt) {
+        double s = 0.0;
+        for (int c = 0; c < nc; ++c) s += part[c * stride + LB_NPART + e];
+        AtA[e] = s;
+    }
+    const double* Bp = bd.B + (size_t)p * L * H;
+    for (int e = t; e < HH; e += nt) {
+        const int i = e / H, j = e - i * H;
+        double s = 0.0;
+        for (int l = 0; l < L; ++l) s = fma(Bp[(size_t)i * L + l], Bp[(size_t)j * L + l], s);
+        BtB[e] = s;
+    }
+    __syncthreads();
+    const double* SA = bd.SigmaA + (size_t)p * HH;
+    const double* SB = bd.SigmaB + (size_t)p * HH;
+    const double* CB = bd.CB + (size_t)p * H;
+    const double* dl = bd.delta + (size_t)p * H;
+    const double Ld = L;
+    LbInputs in;
+    if (t == 0) {   // the same loops as lb_final_kernel
+        double tGAGB = 0.0, trCBGB = 0.0, sumCB = 0.0, sumLogDelta = 0.0;
+        for (int e = 0; e < HH; ++e) tGAGB = fma(AtA[e] + SA[e], BtB[e] + Ld * SB[e], tGAGB);
+        for (int h = 0; h < H; ++h) {
+            trCBGB = fma(CB[h], BtB[h * H + h] + Ld * SB[h * H + h], trCBGB);
+            sumCB += CB[h];
+            sumLogDelta += log(dl[h]);
+        }
+        in.tGAGB = tGAGB; in.trCBGB = trCBGB; in.sumCB = sumCB; in.sumLogDelta = sumLogDelta;
+    }
+    __syncthreads();   // A'A is consumed: its buffer becomes the LU scratch
+    const double ent = normal_entropy_kron<true>(SB, H, L, AtA, sh);
+    if (t == 0) {
+        const int M = bd.moff[p + 1] - bd.moff[p];
+        in.kind = bd.kind; in.H = H; in.H0 = bd.H0; in.H1 = H - bd.H0;
+        in.L = Ld; in.M = M; in.M0 = (double)bd.m0[p];
+        in.acc = acc;
+        in.trBQ = acc[11];
+        in.entropyB = ent;
+        bd.out[p] = lb_assemble(bd.sc + p, in);
+    }
+}
+
+int k_batched_lower_bound(cudaStream_t st, const BatchLbDesc& bd) {
+    if (bd.nprob <= 0) return 0;
+    if (bd.H < 1 || bd.H > 64) { set_error("batched lowerBound supports 1 <= H <= 64 (got %d)", bd.H); return -1; }
+    batched_lb_partial_kernel<<<bd.nchunk, 256, 0, st>>>(bd);
+    VB_LAUNCH_OK();
+    const size_t smem = (size_t)2 * bd.H * bd.H * sizeof(double);
+    VB_CUDA_OK(cudaFuncSetAttribute(batched_lb_final_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    batched_lb_final_kernel<<<bd.nprob, 256, smem, st>>>(bd);
+    VB_LAUNCH_OK();
     return 0;
 }
 

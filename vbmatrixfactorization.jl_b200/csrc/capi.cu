@@ -2239,6 +2239,129 @@ static int batched_vbls_dense_impl(vbmf_b200_ctx* c, int64_t nprob, const double
     return 0;
 }
 
+// ---- K7 batched: lowerBound / lowerBoundTrimmed of many problems -------------------------------------------------------
+static void lb_scalars(const vbmf_b200_sparse_state* s, Scalars& h) { h.alpha0p = s->alpha0; h.beta0p = s->beta0; h.alpha = s->alpha; }
+static void lb_scalars(const vbmf_b200_dual_state* s, Scalars& h) {
+    h.alpha00 = s->alpha00; h.beta00 = s->beta00; h.alpha01 = s->alpha01; h.beta01 = s->beta01;
+    h.alpha_g0 = s->alpha0; h.alpha_g1 = s->alpha1;
+}
+static void lb_scalars(const vbmf_b200_trial_state* s, Scalars& h) {
+    h.alpha00 = s->alpha01; h.beta00 = s->beta01; h.alpha01 = s->alpha02; h.beta01 = s->beta02; h.alpha02 = s->alpha03; h.beta02 = s->beta03;
+    h.alpha_g0 = s->alpha1; h.alpha_g1 = s->alpha2; h.alpha_g2 = s->alpha3;
+}
+
+// Packs what the bound reads -- per column AHat, beta, CA, diag Sigma; per problem BHat, SigmaB, SigmaA, CB, delta and the
+// scalars (the fields and the AHat / ATVecHat choice of the single solver's upload) -- into the batched path's staging arena.
+template <class ST>
+static int batched_lower_bound_impl(vbmf_b200_ctx* c, int kind, int64_t nprob, const double* const* Y, void* const* states,
+                                    double trim, int trimmed, double* out) {
+    if (nprob <= 0) return 0;
+    const ST* s0 = (const ST*)states[0];
+    if (s0 == nullptr) { set_error("batched lowerBound: NULL problem 0"); return -1; }
+    const int64_t L = s0->L, H = s0->H;
+    constexpr bool IS_DUAL = std::is_same<ST, vbmf_b200_dual_state>::value, IS_TRIAL = std::is_same<ST, vbmf_b200_trial_state>::value;
+    int64_t H0 = H;
+    if constexpr (IS_DUAL || IS_TRIAL) H0 = s0->H0;
+    if (L < 1 || H < 1 || H > 64) { set_error("batched lowerBound supports 1 <= H <= 64 (got H = %lld)", (long long)H); return -1; }
+    if (H0 < 0 || H0 > H) { set_error("H must be at least H0!"); return -1; }
+    const int cw = vb::batched_lb_cols((int)H);
+    std::vector<int> moff(nprob + 1, 0), coff(nprob + 1, 0), m0(nprob, 0);
+    for (int64_t p = 0; p < nprob; ++p) {
+        const ST* s = (const ST*)states[p];
+        if (s == nullptr || Y[p] == nullptr) { set_error("batched lowerBound: NULL problem %lld", (long long)p); return -1; }
+        if (s->L != L || s->H != H || s->M < 1 || s->M > 0x7fffff00LL) {
+            set_error("batched lowerBound: problem %lld has different L/H or M < 1", (long long)p); return -1;
+        }
+        if constexpr (IS_DUAL || IS_TRIAL) { if (s->H0 != H0) { set_error("batched lowerBound: H0 differs"); return -1; } }
+        if ((s->ATVecHat == nullptr && s->AHat == nullptr) || s->beta == nullptr || s->CA == nullptr || s->diagSigmaATVec == nullptr ||
+            s->BHat == nullptr || s->SigmaB == nullptr || s->SigmaA == nullptr || s->CB == nullptr || s->delta == nullptr) {
+            set_error("batched lowerBound: a required array of problem %lld is NULL", (long long)p); return -1;
+        }
+        if ((int64_t)moff[p] + s->M > 0x7fffff00LL) { set_error("batched lowerBound: more than 2^31 columns in one batch"); return -1; }
+        moff[p + 1] = moff[p] + (int)s->M;
+        coff[p + 1] = coff[p] + (int)((s->M + cw - 1) / cw);
+        m0[p] = (int)s->M;
+        if constexpr (IS_TRIAL) m0[p] = (int)std::min<int64_t>(std::max<int64_t>(s->M0, 0), s->M);
+    }
+    const int nch = coff[nprob];
+    const size_t Mtot = (size_t)moff[nprob], MH = Mtot * H, HH = (size_t)H * H, LH = (size_t)L * H;
+    VB_CUDA_OK(cudaSetDevice(c->device));
+    // one arena: [inputs | result | device-only chunk partials]; one upload of the inputs, one download of the results
+    size_t off = 0;
+    auto take = [&](size_t bytes) { const size_t o = off; off += align_up(bytes, 256); return o; };
+    const size_t o_moff = take((size_t)(nprob + 1) * 4), o_m0 = take((size_t)nprob * 4), o_coff = take((size_t)(nprob + 1) * 4),
+                 o_cp = take((size_t)nch * 4), o_Y = take(L * Mtot * 8), o_A = take(MH * 8), o_beta = take(MH * 8), o_CA = take(MH * 8),
+                 o_s = take(MH * 8), o_B = take(nprob * LH * 8), o_SB = take(nprob * HH * 8), o_SA = take(nprob * HH * 8),
+                 o_CB = take(nprob * H * 8), o_dl = take(nprob * H * 8), o_sc = take((size_t)nprob * sizeof(Scalars));
+    const size_t up_end = off;
+    const size_t o_out = take((size_t)nprob * 8);
+    const size_t o_part = take((size_t)nch * (vb::LB_NPART + HH) * 8);
+    if (batch_reserve(c, off)) return -1;
+    char* hb = c->batch_host;
+    char* db = c->batch_dev;
+    memcpy(hb + o_moff, moff.data(), (size_t)(nprob + 1) * 4);
+    memcpy(hb + o_m0, m0.data(), (size_t)nprob * 4);
+    memcpy(hb + o_coff, coff.data(), (size_t)(nprob + 1) * 4);
+    int* hcp = (int*)(hb + o_cp);
+    for (int64_t p = 0; p < nprob; ++p) for (int k = coff[p]; k < coff[p + 1]; ++k) hcp[k] = (int)p;
+    double *hY = (double*)(hb + o_Y), *hA = (double*)(hb + o_A), *hbeta = (double*)(hb + o_beta), *hCA = (double*)(hb + o_CA),
+           *hs = (double*)(hb + o_s), *hB = (double*)(hb + o_B), *hSB = (double*)(hb + o_SB), *hSA = (double*)(hb + o_SA),
+           *hCB = (double*)(hb + o_CB), *hdl = (double*)(hb + o_dl);
+    Scalars* hsc = (Scalars*)(hb + o_sc);
+    parallel_for(nprob, [&](int64_t p) {
+        const ST* s = (const ST*)states[p];
+        const size_t M = (size_t)s->M, o = (size_t)moff[p] * H;
+        memcpy(&hY[(size_t)moff[p] * L], Y[p], M * L * 8);
+        if (s->ATVecHat) memcpy(&hA[o], s->ATVecHat, M * H * 8);      // up_A: ATVecHat when given, else AHat transposed
+        else for (size_t m = 0; m < M; ++m) for (size_t h = 0; h < (size_t)H; ++h) hA[o + m * H + h] = s->AHat[h * M + m];
+        memcpy(&hbeta[o], s->beta, M * H * 8);
+        memcpy(&hCA[o], s->CA, M * H * 8);
+        memcpy(&hs[o], s->diagSigmaATVec, M * H * 8);
+        memcpy(&hB[p * LH], s->BHat, LH * 8);
+        memcpy(&hSB[p * HH], s->SigmaB, HH * 8);
+        memcpy(&hSA[p * HH], s->SigmaA, HH * 8);
+        memcpy(&hCB[p * H], s->CB, H * 8);
+        memcpy(&hdl[p * H], s->delta, H * 8);
+        Scalars& h = hsc[p];                                          // sparse_like_upload + the kind's own upload
+        memset(&h, 0, sizeof(Scalars));
+        h.gamma0 = s->gamma0; h.delta0 = s->delta0; h.gamma = s->gamma;
+        h.sigmaHat = s->sigmaHat; h.eta0 = s->eta0; h.zeta0 = s->zeta0; h.eta = s->eta; h.zeta = s->zeta;
+        h.trYTY = s->trYTY;
+        lb_scalars(s, h);
+    });
+    cudaStream_t st = c->st;
+    if (cudaMemcpyAsync(db, hb, up_end, cudaMemcpyHostToDevice, st) != cudaSuccess) { cudaGetLastError(); set_error("batched lowerBound: upload failed"); return -1; }
+    BatchLbDesc bd;
+    bd.nprob = (int)nprob; bd.nchunk = nch; bd.L = (int)L; bd.H = (int)H; bd.H0 = (int)H0; bd.kind = kind; bd.trimmed = trimmed ? 1 : 0;
+    bd.trim = trim;
+    bd.moff = (const int*)(db + o_moff); bd.m0 = (const int*)(db + o_m0); bd.coff = (const int*)(db + o_coff); bd.cprob = (const int*)(db + o_cp);
+    bd.Y = (const double*)(db + o_Y); bd.A = (const double*)(db + o_A); bd.beta = (const double*)(db + o_beta); bd.CA = (const double*)(db + o_CA);
+    bd.sdiag = (const double*)(db + o_s); bd.B = (const double*)(db + o_B); bd.SigmaB = (const double*)(db + o_SB);
+    bd.SigmaA = (const double*)(db + o_SA); bd.CB = (const double*)(db + o_CB); bd.delta = (const double*)(db + o_dl);
+    bd.sc = (const Scalars*)(db + o_sc); bd.part = (double*)(db + o_part); bd.out = (double*)(db + o_out);
+    prof_mark(c, c->ev_k1);       // profiling: the kernels alone (vbmf_b200_ctx_profile_read, K1 slot)
+    int rc = k_batched_lower_bound(st, bd);
+    prof_mark(c, c->ev_k1);
+    if (!rc && cudaMemcpyAsync(hb + o_out, db + o_out, (size_t)nprob * 8, cudaMemcpyDeviceToHost, st) != cudaSuccess) {
+        cudaGetLastError(); set_error("batched lowerBound: download failed"); rc = -1;
+    }
+    { cudaError_t e = cudaStreamSynchronize(st); if (e != cudaSuccess && !rc) { set_error("batched lowerBound: %s", cudaGetErrorString(e)); rc = -1; } }
+    if (rc) return rc;
+    memcpy(out, hb + o_out, (size_t)nprob * 8);
+    return 0;
+}
+
+extern "C" int vbmf_b200_batched_lower_bound(vbmf_b200_ctx* c, int kind, int64_t nprob, const double* const* Y, void* const* states,
+                                             double trim, int trimmed, double* out) {
+    if (!c || (nprob > 0 && (!Y || !states || !out))) { set_error("batched lowerBound: NULL argument"); return -1; }
+    if (kind == VBMF_B200_SPARSE) return batched_lower_bound_impl<vbmf_b200_sparse_state>(c, kind, nprob, Y, states, trim, trimmed, out);
+    if (kind == VBMF_B200_DUAL) return batched_lower_bound_impl<vbmf_b200_dual_state>(c, kind, nprob, Y, states, trim, trimmed, out);
+    if (kind == VBMF_B200_TRIAL) return batched_lower_bound_impl<vbmf_b200_trial_state>(c, kind, nprob, Y, states, trim, trimmed, out);
+    if (kind == VBMF_B200_DENSE) { set_error("the dense solver has no lowerBound (the reference defines none)"); return -1; }
+    set_error("batched lowerBound: unknown parameter kind %d", kind);
+    return -1;
+}
+
 extern "C" int vbmf_b200_batched_vbls(vbmf_b200_ctx* c, int kind, int64_t nprob, const double* const* Y, void* const* states,
                                       int64_t niter, int flags) {
     if (!c || (nprob > 0 && (!Y || !states))) { set_error("batched vbls: NULL argument"); return -1; }

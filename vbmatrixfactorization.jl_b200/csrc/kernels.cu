@@ -3,6 +3,7 @@
 // the device-side convergence test; every reduction uses a fixed order (per-CTA partials + ordered final sum).
 // Reference formulas are cited per kernel (paths relative to /root/reference).
 #include "kernels.cuh"
+#include "elbo.cuh"
 #include "linalg.cuh"
 #include <algorithm>
 #include <cstdlib>
@@ -2328,12 +2329,7 @@ __global__ void __launch_bounds__(256) lb_partial_kernel(Dev d, double trim, int
     for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < n; e += (long long)gridDim.x * blockDim.x) {
         const int h = (int)(e % H);
         const int g = (!grouped || h < d.H0) ? 0 : ((d.moff + (int)(e / H) < d.M0) ? 1 : 2);
-        const double av = d.A[e], be = d.beta[e], ca = d.CAv[e], s = d.sdiag[e];
-        const double lbv = log(be);
-        if (g == 0) { a[0] += lbv; a[3] += ca; } else if (g == 1) { a[1] += lbv; a[4] += ca; } else { a[2] += lbv; a[5] += ca; }
-        if (!trimmed || fabs(av) > trim) {
-            a[6] += lbv; a[7] += ca; a[8] += ca * (av * av + s); a[9] += log(s); a[10] += 1.0;
-        }
+        lb_accumulate(a, g, d.A[e], d.beta[e], d.CAv[e], d.sdiag[e], trim, trimmed);
     }
 #pragma unroll
     for (int i = 0; i < 11; ++i) {
@@ -2350,50 +2346,12 @@ __global__ void lb_reduce_kernel(Dev d, int nparts) {
     }
 }
 
-__device__ inline double gammaELn_d(double a, double logb) { return digamma_pos(a) - logb; }
-
-// normalEntropy(kron(SigmaB, eye(L))) with Julia's left-to-right Float64 determinant product emulated (Q7):
-// LU with partial pivoting of SigmaB, u_aa each repeated L times.  Single thread, H <= 128.
-__device__ double normal_entropy_kron(const double* SigmaB, int H, int L, double* W /* H*H scratch */) {
-    const double LOG_EPS0 = -744.4400719213812;          // log(4.9406564584124654e-324)
-    const double LOG_MIN = LOG_EPS0 - 0.6931471805599453, LOG_MAX = 709.782712893384;
-    for (int e = 0; e < H * H; ++e) W[e] = SigmaB[e];
-    double sign = 1.0, run = 0.0;
-    int state = 0;   // 0 finite, 1 zero, 2 inf
-    for (int k = 0; k < H && state == 0; ++k) {
-        int piv = k; double best = fabs(W[k * H + k]);
-        for (int i = k + 1; i < H; ++i) if (fabs(W[i * H + k]) > best) { best = fabs(W[i * H + k]); piv = i; }
-        if (piv != k) {
-            for (int j = 0; j < H; ++j) { const double tmp = W[k * H + j]; W[k * H + j] = W[piv * H + j]; W[piv * H + j] = tmp; }
-            if (L & 1) sign = -sign;
-        }
-        const double u = W[k * H + k];
-        if (u == 0.0) { state = 1; break; }
-        if (u < 0.0 && (L & 1)) sign = -sign;
-        for (int i = k + 1; i < H; ++i) {
-            const double f = W[i * H + k] / u;
-            for (int j = k + 1; j < H; ++j) W[i * H + j] -= f * W[k * H + j];
-        }
-        run += (double)L * log(fabs(u));
-        if (run < LOG_MIN) state = 1; else if (run > LOG_MAX) state = 2;
-    }
-    double logd;
-    if (state == 1) logd = LOG_EPS0;
-    else if (state == 2) logd = sign > 0 ? INFINITY : LOG_EPS0;
-    else { logd = sign > 0 ? run : LOG_EPS0; if (logd < LOG_EPS0) logd = LOG_EPS0; }
-    const double m = (double)L * H;
-    return m / 2 + m / 2 * 1.8378770664093453 + 0.5 * logd;
-}
-
 __global__ void lb_final_kernel(Dev d, int trimmed) {
     extern __shared__ double W[];
     if (threadIdx.x != 0) return;
-    Scalars* sc = d.sc;
-    const double ln2pi = 1.8378770664093453;
     const int H = d.H;
-    const double L = d.L, M = d.Mglob;
+    const double L = d.L;
     const double* AtA = d.packed + packed_ata(d);
-    const double* acc = d.lbacc;
     double tGAGB = 0.0, trCBGB = 0.0, sumCB = 0.0, sumLogDelta = 0.0;
     for (int e = 0; e < H * H; ++e) tGAGB = fma(AtA[e] + d.SigmaA[e], d.BtB[e] + L * d.SigmaB[e], tGAGB);
     for (int h = 0; h < H; ++h) {
@@ -2401,66 +2359,13 @@ __global__ void lb_final_kernel(Dev d, int trimmed) {
         sumCB += d.CBv[h];
         sumLogDelta += log(d.deltav[h]);
     }
-    const double elnS = gammaELn_d(sc->eta, log(sc->zeta));
-    const double psiG = digamma_pos(sc->gamma);
-    const double elnD = H * psiG - sumLogDelta;
-    const double MHk = acc[10];                             // params.MH (kept count when trimmed)
-    double Lb = 0.0;
-    Lb += -L * M / 2 * ln2pi + L * M / 2 * elnS;
-    Lb += -sc->sigmaHat / 2 * (sc->trYTY - 2 * sc->trBQ + tGAGB);
-    if (d.kind == KIND_SPARSE) {
-        const double psiA = digamma_pos(sc->alpha);
-        const double elnB = MHk * psiA - acc[6];
-        Lb += -MHk / 2 * ln2pi + 0.5 * elnB;
-        Lb += -(0.5 * acc[8]);
-        Lb += -L * H / 2 * ln2pi;
-        Lb += L / 2 * elnD;
-        Lb += -0.5 * trCBGB;
-        Lb += sc->eta0 * log(sc->zeta0) - lgamma(sc->eta0);
-        Lb += (sc->eta0 - 1) * elnS - sc->zeta0 * sc->sigmaHat;
-        Lb += MHk * (sc->alpha0p * log(sc->beta0p) - lgamma(sc->alpha0p));
-        Lb += (sc->alpha0p - 1) * elnB;
-        Lb += -sc->beta0p * acc[7];
-        Lb += H * (sc->gamma0 * log(sc->delta0) - lgamma(sc->gamma0));
-        Lb += (sc->gamma0 - 1) * elnD;
-        Lb += -sc->gamma0 * sumCB;                          // Q13
-        Lb += MHk / 2 + MHk / 2 * ln2pi + 0.5 * acc[9];
-        Lb += normal_entropy_kron(d.SigmaB, H, d.L, W);
-        Lb += sc->eta + log(sc->zeta) + lgamma(sc->eta) + (1 - sc->eta) * digamma_pos(sc->eta);
-        Lb += MHk * (sc->alpha + lgamma(sc->alpha) + (1 - sc->alpha) * psiA) + acc[6];
-    } else {
-        // dual (src/vbmf_dual.jl:559-597): groups 0, 1; trial (src/vbmf_trial.jl:633-681): groups 0, 1, 2.  Group sums use the
-        // untrimmed beta_g / CA_g vectors even in lowerBoundTrimmed (only CA, ATVecHat, diagSigmaATVec, MH are trimmed).
-        const int ng = d.kind == KIND_TRIAL ? 3 : 2;
-        const double Ng[3] = {M * d.H0, (double)d.M0 * d.H1, (M - (double)d.M0) * d.H1};
-        const double ag[3] = {sc->alpha_g0, sc->alpha_g1, sc->alpha_g2};
-        const double a0g[3] = {sc->alpha00, sc->alpha01, sc->alpha02};
-        const double b0g[3] = {sc->beta00, sc->beta01, sc->beta02};
-        double psig[3], elng[3];
-        for (int g = 0; g < ng; ++g) { psig[g] = digamma_pos(ag[g]); elng[g] = Ng[g] * psig[g] - acc[g]; }
-        Lb += -MHk / 2 * ln2pi + 0.5 * elng[0];
-        for (int g = 1; g < ng; ++g) Lb += 0.5 * elng[g];
-        Lb += -(0.5 * acc[8]);
-        Lb += -L * H / 2 * ln2pi;
-        Lb += L / 2 * elnD;
-        Lb += -0.5 * trCBGB;
-        Lb += sc->eta0 * log(sc->zeta0) - lgamma(sc->eta0);
-        Lb += (sc->eta0 - 1) * elnS - sc->zeta0 * sc->sigmaHat;
-        for (int g = 0; g < ng; ++g) {
-            Lb += Ng[g] * (a0g[g] * log(b0g[g]) - lgamma(a0g[g]));
-            Lb += (a0g[g] - 1) * elng[g];
-            Lb += -b0g[g] * acc[3 + g];
-        }
-        Lb += H * (sc->gamma0 * log(sc->delta0) - lgamma(sc->gamma0));
-        Lb += (sc->gamma0 - 1) * elnD;
-        Lb += -sc->gamma0 * sumCB;
-        Lb += MHk / 2 + MHk / 2 * ln2pi + 0.5 * acc[9];
-        Lb += normal_entropy_kron(d.SigmaB, H, d.L, W);
-        Lb += sc->eta + log(sc->zeta) + lgamma(sc->eta) + (1 - sc->eta) * digamma_pos(sc->eta);
-        for (int g = 0; g < ng; ++g) Lb += (Ng[g] > 0 ? Ng[g] * (ag[g] + lgamma(ag[g]) + (1 - ag[g]) * psig[g]) : 0.0) + acc[g];
-    }
-    Lb += H * (sc->gamma + lgamma(sc->gamma) + (1 - sc->gamma) * psiG) + sumLogDelta;
-    sc->lb = Lb;
+    LbInputs in;
+    in.kind = d.kind; in.H = H; in.H0 = d.H0; in.H1 = d.H1;
+    in.L = L; in.M = d.Mglob; in.M0 = (double)d.M0;
+    in.acc = d.lbacc;
+    in.tGAGB = tGAGB; in.trCBGB = trCBGB; in.sumCB = sumCB; in.sumLogDelta = sumLogDelta; in.trBQ = d.sc->trBQ;
+    in.entropyB = normal_entropy_kron<false>(d.SigmaB, H, d.L, W, nullptr);
+    d.sc->lb = lb_assemble(d.sc, in);
 }
 int k_lower_bound(cudaStream_t st, const Dev& d, double trim, int trimmed, int phase) {
     if (phase == 0) {

@@ -188,4 +188,32 @@ int batched_cluster_size(int kind, int L, int H, int M);
 int k_batched_vbls(cudaStream_t st, const BatchDesc& bd, const int (&n)[5], int Mmax0);
 int k_batched_vbls_dense(cudaStream_t st, const BatchDenseDesc& bd, const int (&n)[5], int Mmax0);
 
+// K7 batched: lowerBound / lowerBoundTrimmed of many sparse / dual / trial problems (csrc/batched.cu).  Every problem is cut
+// into chunks of batched_lb_cols(H) contiguous columns, one CTA each, and one more CTA per problem combines its chunks in
+// order and assembles the bound: the work split depends only on the problem's own (M, H).
+struct BatchLbDesc {
+    int nprob, nchunk, L, H, H0, kind, trimmed;
+    double trim;
+    const int* moff;        // [nprob+1] column offsets into the packed per-column arrays
+    const int* m0;          // [nprob]   trial: row split M0 clamped to [0, M]; dual / sparse: M
+    const int* coff;        // [nprob+1] first chunk of each problem
+    const int* cprob;       // [nchunk]  problem of each chunk
+    const double* Y;        // [L][Mtot] column-major, problems concatenated
+    const double* A;        // [Mtot][H] AHat rows (= ATVecHat)
+    const double* beta;     // [Mtot*H]
+    const double* CA;       // [Mtot*H]
+    const double* sdiag;    // [Mtot*H]  diagSigmaATVec
+    const double* B;        // [nprob][L*H] column-major L x H
+    const double* SigmaB;   // [nprob][H*H]
+    const double* SigmaA;   // [nprob][H*H]
+    const double* CB;       // [nprob][H]
+    const double* delta;    // [nprob][H]
+    const Scalars* sc;      // [nprob]   the model scalars in the single solver's layout
+    double* part;           // [nchunk][LB_NPART + H*H] chunk partials: the 11 element sums, tr(B'YA), A'A
+    double* out;            // [nprob]   the bounds
+};
+constexpr int LB_NPART = 12;
+__host__ __device__ inline int batched_lb_cols(int H) { return 16384 / H > 16 ? 16384 / H : 16; }
+int k_batched_lower_bound(cudaStream_t st, const BatchLbDesc& bd);
+
 }  // namespace vb
