@@ -1,11 +1,11 @@
 """Roofs of the INT8 contractions from a bench.py JSON line: INT8 operations and slice bytes over the measured K1 / K2 times.
 
-    python tools/int8gemm/roofline.py profiles/r03_bench_c3_int8.json
+    python tools/int8gemm/roofline.py profiles/r06_bench_c3_new_1.json
 
 bench.py's roofline.frac and iteration_frac_of_peak are quoted against the FP64 peak and read above 1 on this path.  Here
 each kernel is set against the rates it can reach:
-  ops   = 36 slice products x 2*L*M*H            (levels 0..7 of 8 x 8 slices)
-  bytes = 8*L*M (eight int8 slices of Y, read once) + the operand slices (8*L*H or 8*M*H, L2-resident, not counted)
+  ops   = 28 slice products x 2*L*M*H            (levels 0..6 of 7 x 7 signed radix-256 digits)
+  bytes = 7*L*M (seven int8 digit planes of Y, read once) + the operand digits (7*L*H or 7*M*H, L2-resident, not counted)
   INT8 tensor rate: 4.5 POPS dense (B200 data sheet, 1000 W card; not measured here).  HBM: the measured 6.54 TB/s copy rate
   (bench.py hbm_peak_gbs).  The larger of ops/rate and bytes/bandwidth is the least time; share = that / kernel time.
 """
@@ -21,7 +21,7 @@ def main(path):
     L, H, M = cfg["global_shape"][0], cfg["global_shape"][2], cfg["columns_per_gpu"]
     roof = d["roofline"]
     bw = roof.get("hbm_peak_gbs", 6535.7) * 1e9
-    ops, nbytes = 36 * 2.0 * L * M * H, 8.0 * L * M
+    ops, nbytes = 28 * 2.0 * L * M * H, 7.0 * L * M
     out = {"shape": [L, M, H], "clocks": d.get("clocks")}
     for k in ("k1", "k2"):
         t = roof[k + "_ms"] * 1e-3

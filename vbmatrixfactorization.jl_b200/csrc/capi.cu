@@ -106,8 +106,8 @@ struct vbmf_b200_ctx {
     bool tr_pending = false;          // trYTY lives in d_tr only (not yet read back to the host)
     bool simt = false;
     bool gemm_dmma = false;   // VBMF_B200_GEMM=dmma: keep the FP64 tensor-core contractions at H <= 64 (A/B measurements)
-    // int8 slices of Y for the INT8 contractions (gemm_int8.cu): [8][Mloc][ldZ], exponents F[L] | E[Mloc]; built on first
-    // use after every change of Y (ctx_slices)
+    // int8 digit planes of Y for the INT8 contractions (gemm_int8.cu): [I8_NSL][Mloc][ldZ], exponents F[L] | E[Mloc]; built
+    // on first use after every change of Y (ctx_slices)
     uint8_t* Z = nullptr;
     int* Zexp = nullptr;
     size_t Z_bytes = 0;
@@ -483,7 +483,7 @@ static int ctx_slices(vbmf_b200_ctx* c, bool* ok) {
     if (c->z_failed || c->Y == nullptr || c->Mloc <= 0) return 0;
     if (c->z_ready) { *ok = true; return 0; }
     const int ldZ = i8_ld(c->L);
-    const size_t bytes = (size_t)8 * c->Mloc * ldZ;
+    const size_t bytes = (size_t)I8_NSL * c->Mloc * ldZ;
     if (c->Z == nullptr || c->Z_bytes != bytes || c->ldZ != ldZ) {
         ctx_free_Z(c);
         if (cudaMalloc(&c->Z, bytes) != cudaSuccess || cudaMalloc(&c->Zexp, ((size_t)c->L + c->Mloc) * 4) != cudaSuccess) {
@@ -496,8 +496,8 @@ static int ctx_slices(vbmf_b200_ctx* c, bool* ok) {
     }
     if (i8_build_Y(c->st, c->Y, c->ldY, c->L, c->Mloc, c->Z, ldZ, c->Zexp, c->Zexp + c->L)) return -1;
     const uint64_t s1 = (uint64_t)ldZ, s2 = (uint64_t)ldZ * c->Mloc;
-    if (make_tmap_3d_i8(&c->tmZ1, c->Z, (uint64_t)c->L, (uint64_t)c->Mloc, 8, s1, s2, 32, 128, 8, false)) return -1;
-    if (make_tmap_3d_i8(&c->tmZ2, c->Z, (uint64_t)c->L, (uint64_t)c->Mloc, 8, s1, s2, 128, 32, 8, true)) return -1;
+    if (make_tmap_3d_i8(&c->tmZ1, c->Z, (uint64_t)c->L, (uint64_t)c->Mloc, I8_NSL, s1, s2, 32, 128, I8_NSL, false)) return -1;
+    if (make_tmap_3d_i8(&c->tmZ2, c->Z, (uint64_t)c->L, (uint64_t)c->Mloc, I8_NSL, s1, s2, 128, 32, I8_NSL, true)) return -1;
     c->z_ready = true;
     *ok = true;
     return 0;
@@ -512,7 +512,7 @@ static void i8_plans(int L, int M, int H, int num_sms, int* S1, int* kbs1, int* 
     *kchunk = (*kchunk + 31) / 32 * 32;
     *S = std::max(1, (M + *kchunk - 1) / *kchunk);
 }
-// operand slices of the INT8 path: K1 [8][Hp][ldZ] + G[Hp], K2 [8][Hp][ldM] + G[S][Hp] (one allocation)
+// operand digits of the INT8 path: K1 [I8_NSL][Hp][ldZ] + G[Hp], K2 [I8_NSL][Hp][ldM] + G[S][Hp] (one allocation)
 struct I8Operands {
     char* mem = nullptr;
     uint8_t *Wb = nullptr, *Wa = nullptr;
@@ -528,12 +528,12 @@ static int i8_operands_alloc(I8Operands* o, int L, int M, int H, int S, bool* ok
     *ok = false;
     const int Hp = i8_hpad(H), ldZ = i8_ld(L);
     o->ldM = i8_ld(std::max(M, 1));
-    const size_t nb = align_up((size_t)8 * Hp * ldZ, 256), na = align_up((size_t)8 * Hp * o->ldM, 256);
+    const size_t nb = align_up((size_t)I8_NSL * Hp * ldZ, 256), na = align_up((size_t)I8_NSL * Hp * o->ldM, 256);
     const size_t gb = align_up((size_t)Hp * 4, 256), ga = align_up((size_t)S * Hp * 4, 256);
     if (cudaMalloc(&o->mem, nb + na + gb + ga) != cudaSuccess) { cudaGetLastError(); o->mem = nullptr; return 0; }
     o->Wb = (uint8_t*)o->mem; o->Wa = o->Wb + nb; o->Gb = (int*)(o->Wa + na); o->Ga = (int*)((char*)o->Gb + gb);
-    if (make_tmap_3d_i8(&o->tmWb, o->Wb, (uint64_t)L, (uint64_t)Hp, 8, (uint64_t)ldZ, (uint64_t)ldZ * Hp, 32, (uint32_t)Hp, 8, false)) return -1;
-    if (M > 0 && make_tmap_3d_i8(&o->tmWa, o->Wa, (uint64_t)M, (uint64_t)Hp, 8, (uint64_t)o->ldM, (uint64_t)o->ldM * Hp, 32, (uint32_t)Hp, 8, false)) return -1;
+    if (make_tmap_3d_i8(&o->tmWb, o->Wb, (uint64_t)L, (uint64_t)Hp, I8_NSL, (uint64_t)ldZ, (uint64_t)ldZ * Hp, 32, (uint32_t)Hp, I8_NSL, false)) return -1;
+    if (M > 0 && make_tmap_3d_i8(&o->tmWa, o->Wa, (uint64_t)M, (uint64_t)Hp, I8_NSL, (uint64_t)o->ldM, (uint64_t)o->ldM * Hp, 32, (uint32_t)Hp, I8_NSL, false)) return -1;
     *ok = true;
     return 0;
 }

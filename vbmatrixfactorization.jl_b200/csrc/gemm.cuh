@@ -49,23 +49,25 @@ int launch_reduce_q_sk(cudaStream_t st, const double* Qpart, double* Q, int L, i
 void plan_splitk(int L, int M, int H, int num_sms, int* S, int* kchunk);
 
 // ---- INT8 tensor-core contractions with exact slice splitting (gemm_int8.cu), H <= 64 ----
-// Slices are int8 [8][rows][ld] planes, ld a multiple of 16; exponents are ints (2^e scales).
+// Operands are I8_NSL signed radix-256 digit planes, int8 [I8_NSL][rows][ld], ld a multiple of 16; exponents are ints (2^e
+// scales).
+constexpr int I8_NSL = 7;
 inline int i8_hpad(int H) { return (H + 15) / 16 * 16; }
 inline int i8_ld(int n) { return (n + 15) / 16 * 16; }
 int gemm_i8_init_device();
 // rank-3 uint8 tensor map {d0, d1, d2} with byte pitches s1, s2; 32-byte swizzle, or 128-byte with swizzle128
 int make_tmap_3d_i8(CUtensorMap* out, const void* base, uint64_t d0, uint64_t d1, uint64_t d2, uint64_t s1, uint64_t s2,
                     uint32_t b0, uint32_t b1, uint32_t b2, bool swizzle128);
-// Y (L x M, column-major) -> row exponents F[L], column exponents E[M], slices Z [8][M][ldZ] (ldZ = i8_ld(L))
+// Y (L x M, column-major) -> row exponents F[L], column exponents E[M], digits Z [7][M][ldZ] (ldZ = i8_ld(L))
 int i8_build_Y(cudaStream_t st, const double* Y, int ldY, int L, int M, uint8_t* Z, int ldZ, int* F, int* E);
-// K1 operand: diag(2^F) * B (B column-major [H][ldB]) -> exponents G[Hp], slices W [8][Hp][ldZ]
+// K1 operand: diag(2^F) * B (B column-major [H][ldB]) -> exponents G[Hp], digits W [7][Hp][ldZ]
 int i8_slice_B(cudaStream_t st, const double* B, int ldB, int L, int H, const int* F, uint8_t* W, int ldZ, int* G, const Scalars* sc);
-// K2 operand: diag(2^E) * A (A row-major [M][H]) -> exponents G[S][Hp] per split-K chunk of kchunk rows, slices W [8][Hp][ldM]
+// K2 operand: diag(2^E) * A (A row-major [M][H]) -> exponents G[S][Hp] per split-K chunk of kchunk rows, digits W [7][Hp][ldM]
 int i8_slice_A(cudaStream_t st, const double* A, int M, int H, const int* E, int kchunk, int S, uint8_t* W, int ldM, int* G, const Scalars* sc);
 // out[s*slab + row*rs + h*hs] = 2^(rowexp[row] + colexp[s*cstride + h]) * sum_{k in split s} A(row, k) * B(k, h).
-// mn = false (K1): tmA = Y slices {L, M, 8}, box {32, 128, 8}, 32-byte swizzle; rows are columns of Y, k = l.
-// mn = true  (K2): tmA = Y slices {L, M, 8}, box {128, 32, 8}, 128-byte swizzle; rows are rows of Y, k = m.
-// tmB: operand slices {kdim, Hp, 8}, box {32, Hp, 8}, 32-byte swizzle.  klen: split length, a multiple of 32.
+// mn = false (K1): tmA = Y digits {L, M, 7}, box {32, 128, 7}, 32-byte swizzle; rows are columns of Y, k = l.
+// mn = true  (K2): tmA = Y digits {L, M, 7}, box {128, 32, 7}, 128-byte swizzle; rows are rows of Y, k = m.
+// tmB: operand digits {kdim, Hp, 7}, box {32, Hp, 7}, 32-byte swizzle.  klen: split length, a multiple of 32.
 int launch_gemm_i8(cudaStream_t st, bool mn, const CUtensorMap* tmA, const CUtensorMap* tmB, double* out, int nrows, int kdim,
                    int S, int klen, int H, const int* rowexp, const int* colexp, int cstride, size_t slab, size_t rs, size_t hs,
                    const Scalars* sc, int num_sms);

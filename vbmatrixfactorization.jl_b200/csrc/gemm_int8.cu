@@ -1,26 +1,31 @@
 // K1 / K2 on the INT8 tensor cores (tcgen05.mma.kind::i8) with exact slice splitting, for H <= 64.
 //
-// Both operands are written as eight int8 slices with power-of-two scales (the Ozaki scheme):
-//   Y = diag(2^F) * Z * diag(2^E),  Z = sum_{i<8} 128^-(i+1) S_i + r,  |S_i| <= 127, |r| < 2^-56
-// F_l is the exponent of the row maximum of Y, E_m the exponent of the column maximum of the row-scaled Y, so |Z| < 1.  The
-// small operand of a contraction (BHat for K1, AHat for K2) is scaled by the same exponents (diag(2^F) * B, diag(2^E) * A),
-// given one exponent per column (K2: per column and split-K chunk) and cut the same way.  The slice products S_i * T_j with
-// i + j = k form level k; levels 0..7 (36 products) are accumulated exactly in INT32 tensor memory and combined in FP64:
-//   sum_k 2^-7(k+2) * level_k,  levels 7 down to 0,  times 2^(row exponent + column exponent).
-// Y's slices are built once per attached Y (i8_build_Y); the small operand is sliced every iteration (i8_slice_B / _A).
+// Both operands are written as seven signed radix-256 digits with power-of-two scales (the Ozaki scheme):
+//   Y = diag(2^F) * Z * diag(2^E),  Z = sum_{i<7} 2^-(7+8i) S_i + r,  -128 <= S_i <= 127, |r| <= 2^-56
+// F_l is the exponent of the row maximum of Y.  E_m is the smallest exponent with |row-scaled Y| <= (127/128) 2^E_m over the
+// column, so |Z| <= 127/128 and rint(Z * 2^55) lies inside the range of seven balanced digits, whose positive end is only
+// 127 (2^56 - 1) / 255.  The small operand of a contraction (BHat for K1, AHat for K2) is scaled by the same exponents
+// (diag(2^F) * B, diag(2^E) * A), given one exponent per column (K2: per column and split-K chunk) under the same 127/128
+// rule and cut the same way.  Every digit is a plain int8, so signed kind::i8 multiplies them as they are.  The digit
+// products S_i * T_j with i + j = k form level k; levels 0..6 (28 products) are accumulated exactly in INT32 tensor memory and
+// combined in FP64:
+//   sum_k 2^-(8k+14) * level_k,  levels 6 down to 0,  times 2^(row exponent + column exponent).
+// Y's digits are built once per attached Y (i8_build_Y); the small operand is cut every iteration (i8_slice_B / _A).
 //
-// Tensor memory: level k of the 128 x Hp tile lives in columns [Hp*k, Hp*(k+1)) (Hp = H rounded up to 16, <= 64, at most 512
-// columns).  For Y slice i, ONE run of MMAs takes the operand slices j = 0..7-i, laid side by side along N in shared memory,
-// and writes columns [Hp*i, Hp*8): every level the slice contributes to in one instruction stream (N split in pieces <= 256).
-// Level 7 sums 8 products of |S| <= 127 per k, so INT32 holds 16643 k; the accumulators are flushed every 16384 k.
+// Tensor memory: level k of the 128 x Hp tile lives in columns [Hp*k, Hp*(k+1)) (Hp = H rounded up to 16, <= 64, at most 448
+// of the 512 columns allocated).  For Y digit i, ONE run of MMAs takes the operand digits j = 0..6-i, laid side by side along
+// N in shared memory, and writes columns [Hp*i, Hp*7): every level the digit contributes to in one instruction stream (N
+// split in pieces <= 256: 10 MMAs per stage at Hp = 64).  Level 6 sums 7 products of |S| <= 128 per k (114688), so INT32
+// holds 18724 k; the accumulators are flushed every 16384 k.
 //
-// Pipeline (one CTA per SM): warp 4 issues TMA loads of 32 k of all 8 Y slices and all 8 operand slices per stage into a
-// 4-stage ring guarded by full / empty mbarriers, one lane of warp 5 issues the MMAs and commits each stage back, warps 0-3
-// read tensor memory (warp q owns lanes 32q..32q+31 = tile rows) and write the FP64 result.  Persistent CTAs walk a static
-// list of (tile, split) work items; split-K slabs are summed in fixed order by the caller, so results are bit-reproducible.
-//   K1  P = Y' * B:  A operand = Y slices, K-major (rows m, k = l), box {32, 128, 8}, 32-byte swizzle.
-//   K2  Q = Y  * A:  A operand = the same slices read MN-major (rows l, k = m), box {128, 32, 8}, 128-byte swizzle.
-//   The B operand is the small operand's slices, K-major [8][Hp][ld], box {32, Hp, 8}, 32-byte swizzle.
+// Pipeline (one CTA per SM): warp 4 issues TMA loads of 32 k of all 7 Y digit planes and all 7 operand planes per stage into
+// a STAGES-deep ring guarded by full / empty mbarriers, one lane of warp 5 issues the MMAs and commits each stage back, warps
+// 0-3 read tensor memory (warp q owns lanes 32q..32q+31 = tile rows) and write the FP64 result.  Persistent CTAs walk a
+// static list of (tile, split) work items; split-K slabs are summed in fixed order by the caller, so results are
+// bit-reproducible.
+//   K1  P = Y' * B:  A operand = Y digits, K-major (rows m, k = l), box {32, 128, 7}, 32-byte swizzle.
+//   K2  Q = Y  * A:  A operand = the same digits read MN-major (rows l, k = m), box {128, 32, 7}, 128-byte swizzle.
+//   The B operand is the small operand's digits, K-major [7][Hp][ld], box {32, Hp, 7}, 32-byte swizzle.
 #include "gemm.cuh"
 #include <algorithm>
 
@@ -29,13 +34,16 @@ namespace i8k {
 
 constexpr int TM = 128;                 // tile rows (MMA M)
 constexpr int KB = 32;                  // k per stage = K of one int8 MMA
-constexpr int NSL = 8;                  // slices per operand
-constexpr int STAGES = 4;
-constexpr int A_BYTES = NSL * TM * KB;  // 32 KB: 8 slices x 128 rows x 32 k
-constexpr int B_BYTES = NSL * 64 * KB;  // 16 KB at Hp = 64
-constexpr int SB = A_BYTES + B_BYTES;
+constexpr int NSL = I8_NSL;             // digit planes per operand
+constexpr int STAGES = 4;               // measured a little faster than 5 stages (which also fit) at config 3
+constexpr int A_BYTES = NSL * TM * KB;  // 28 KB: 7 digits x 128 rows x 32 k
+constexpr int B_BYTES = NSL * 64 * KB;  // 14 KB at Hp = 64
+constexpr int SB = A_BYTES + B_BYTES;   // 42 KB: stage and plane offsets stay 1024-aligned for the 128-byte swizzle
+static_assert(SB % 1024 == 0 && A_BYTES % 1024 == 0, "stage layout must stay 1024-byte aligned");
 constexpr int SMEM = STAGES * SB + 1024 + 256;
-constexpr int SEG_KB = 16384 / KB;      // k-blocks per flush: level 7 stays below 2^31
+static_assert(SMEM <= 227 * 1024, "stage ring exceeds the shared memory of one CTA");
+constexpr int SEG_KB = 16384 / KB;      // k-blocks per flush: level 6 stays below 2^31
+static_assert((long long)SEG_KB * KB * NSL * 128 * 128 < (1ll << 31), "level 6 may overflow INT32 between flushes");
 constexpr int EXP_NONE = -(1 << 30);    // exponent of 0 (and of non-finite values): below every real exponent
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -94,21 +102,32 @@ __device__ __forceinline__ int exp_of(double x) {
     frexp(x, &e);
     return e;
 }
+// smallest e with |x| <= (127/128) 2^e: frexp's exponent, plus one when the mantissa exceeds 127/128 (monotonic in |x|)
+__device__ __forceinline__ int exp_digits(double x) {
+    if (x == 0.0 || !isfinite(x)) return EXP_NONE;
+    int e;
+    const double m = frexp(x, &e);
+    return fabs(m) > 127.0 / 128.0 ? e + 1 : e;
+}
 __device__ __forceinline__ int exp_fix(int e) { return e <= EXP_NONE ? 0 : e; }
 
-// eight truncated 7-bit slices of w (|w| < 1), four consecutive values packed per 32-bit word: byte q of word i = slice i of w[q]
-__device__ __forceinline__ void slice4(const double (&w)[4], uint32_t (&out)[NSL]) {
+// rint(x * 2^(55 - e)): the digits' fixed-point form of w = x * 2^-e (|w| <= 127/128, so |result| <= 127 * 2^48)
+__device__ __forceinline__ long long fixed55(double x, int e) { return __double2ll_rn(ldexp(x, 55 - e)); }
+
+// seven balanced radix-256 digits of X = rint(w * 2^55): w = sum_i d_i 2^-(7+8i), d_i in [-128, 127], taken from the bottom.
+// The digit is the low byte read as signed; X - d is then a multiple of 256.  Four consecutive values per 32-bit word: byte q
+// of word i = digit i of x[q].
+__device__ __forceinline__ void digits4(const long long (&x)[4], uint32_t (&out)[NSL]) {
 #pragma unroll
     for (int i = 0; i < NSL; ++i) out[i] = 0u;
 #pragma unroll
     for (int q = 0; q < 4; ++q) {
-        double t = w[q];
+        long long t = x[q];
 #pragma unroll
-        for (int i = 0; i < NSL; ++i) {
-            t *= 128.0;
-            const double s = trunc(t);
-            t -= s;
-            out[i] |= ((uint32_t)(int)s & 0xffu) << (8 * q);
+        for (int i = NSL - 1; i >= 0; --i) {
+            const int d = (int8_t)(t & 255);
+            out[i] |= ((uint32_t)t & 0xffu) << (8 * q);
+            t = (t - d) >> 8;
         }
     }
 }
@@ -139,7 +158,7 @@ __global__ void __launch_bounds__(256) y_row_exp_kernel(const double* __restrict
     atomicMax(F + l, e);
 }
 
-// one CTA per column m: E_m, then the column's eight slices (4 rows per thread and 32-bit word)
+// one CTA per column m: E_m, then the column's seven digit planes (4 rows per thread and 32-bit word)
 __global__ void __launch_bounds__(256) y_slices_kernel(const double* __restrict__ Y, int ldY, int L, int M, const int* __restrict__ F,
                                                        int* __restrict__ E, uint8_t* __restrict__ Z, int ldZ) {
     __shared__ int red[32];
@@ -147,28 +166,28 @@ __global__ void __launch_bounds__(256) y_slices_kernel(const double* __restrict_
     const double* y = Y + (size_t)m * ldY;
     int e = EXP_NONE;
     for (int l = threadIdx.x; l < L; l += blockDim.x) {
-        const int ey = exp_of(y[l]);
+        const int ey = exp_digits(y[l]);
         if (ey > EXP_NONE) e = max(e, ey - exp_fix(F[l]));
     }
     const int Em = exp_fix(block_max_int(e, red));
     if (threadIdx.x == 0) E[m] = Em;
     const size_t plane = (size_t)M * ldZ;
     for (int l4 = threadIdx.x; l4 < ldZ / 4; l4 += blockDim.x) {
-        double w[4];
+        long long x[4];
 #pragma unroll
         for (int q = 0; q < 4; ++q) {
             const int l = 4 * l4 + q;
-            w[q] = l < L ? ldexp(y[l], -(exp_fix(F[l]) + Em)) : 0.0;
+            x[q] = l < L ? fixed55(y[l], exp_fix(F[l]) + Em) : 0;
         }
         uint32_t s[NSL];
-        slice4(w, s);
+        digits4(x, s);
 #pragma unroll
         for (int i = 0; i < NSL; ++i) reinterpret_cast<uint32_t*>(Z + i * plane + (size_t)m * ldZ)[l4] = s[i];
     }
 }
 
-// ------------------------------------------------------------------------------------------- K1 operand: slices of diag(2^F) B
-// one CTA per column h < Hp (rows h >= H are zero): G_h, then the column's slices, layout [8][Hp][ldZ]
+// ------------------------------------------------------------------------------------------- K1 operand: digits of diag(2^F) B
+// one CTA per column h < Hp (rows h >= H are zero): G_h, then the column's digits, layout [7][Hp][ldZ]
 __global__ void __launch_bounds__(512) b_slices_kernel(const double* __restrict__ B, int ldB, int L, int H, int Hp, const int* __restrict__ F,
                                                        uint8_t* __restrict__ W, int ldZ, int* __restrict__ G, const Scalars* __restrict__ sc) {
     if (sc != nullptr && !sc->active) return;
@@ -178,27 +197,27 @@ __global__ void __launch_bounds__(512) b_slices_kernel(const double* __restrict_
     int e = EXP_NONE;
     if (h < H)
         for (int l = threadIdx.x; l < L; l += blockDim.x) {
-            const int eb = exp_of(b[l]);
+            const int eb = exp_digits(b[l]);
             if (eb > EXP_NONE) e = max(e, eb + exp_fix(F[l]));
         }
     const int Gh = exp_fix(block_max_int(e, red));
     if (threadIdx.x == 0) G[h] = Gh;
     const size_t plane = (size_t)Hp * ldZ;
     for (int l4 = threadIdx.x; l4 < ldZ / 4; l4 += blockDim.x) {
-        double w[4];
+        long long x[4];
 #pragma unroll
         for (int q = 0; q < 4; ++q) {
             const int l = 4 * l4 + q;
-            w[q] = (h < H && l < L) ? ldexp(b[l], exp_fix(F[l]) - Gh) : 0.0;
+            x[q] = (h < H && l < L) ? fixed55(b[l], Gh - exp_fix(F[l])) : 0;
         }
         uint32_t s[NSL];
-        slice4(w, s);
+        digits4(x, s);
 #pragma unroll
         for (int i = 0; i < NSL; ++i) reinterpret_cast<uint32_t*>(W + i * plane + (size_t)h * ldZ)[l4] = s[i];
     }
 }
 
-// ------------------------------------------------------------------------------------------- K2 operand: slices of diag(2^E) A
+// ------------------------------------------------------------------------------------------- K2 operand: digits of diag(2^E) A
 // A is [M][H] (row m contiguous in h).  Exponents per (split-K chunk, column): G[c][h] = max over m in chunk c (atomicMax on
 // integers: order-independent).  256 rows per CTA, thread = (h = t % 64, rows t / 64 + 4 r).
 __global__ void __launch_bounds__(256) a_exp_kernel(const double* __restrict__ A, int M, int H, int Hp, const int* __restrict__ E, int kchunk,
@@ -214,13 +233,13 @@ __global__ void __launch_bounds__(256) a_exp_kernel(const double* __restrict__ A
             if (cur >= 0 && e > EXP_NONE) atomicMax(G + cur * Hp + h, e);
             cur = c; e = EXP_NONE;
         }
-        const int ea = exp_of(A[(size_t)m * H + h]);
+        const int ea = exp_digits(A[(size_t)m * H + h]);
         if (ea > EXP_NONE) e = max(e, ea + E[m]);
     }
     if (cur >= 0 && e > EXP_NONE) atomicMax(G + cur * Hp + h, e);
 }
 
-// 64 rows per CTA through shared memory; output K-major [8][Hp][ldM]
+// 64 rows per CTA through shared memory; output K-major [7][Hp][ldM]
 __global__ void __launch_bounds__(256) a_slices_kernel(const double* __restrict__ A, int M, int H, int Hp, const int* __restrict__ E, int kchunk,
                                                        const int* __restrict__ G, uint8_t* __restrict__ W, int ldM, const Scalars* __restrict__ sc) {
     if (sc != nullptr && !sc->active) return;
@@ -233,15 +252,15 @@ __global__ void __launch_bounds__(256) a_slices_kernel(const double* __restrict_
     for (int t = threadIdx.x; t < Hp * 16; t += blockDim.x) {
         const int h = t >> 4, g = t & 15;
         if (m0 + 4 * g >= ldM) continue;
-        double w[4];
+        long long x[4];
 #pragma unroll
         for (int q = 0; q < 4; ++q) {
             const int r = 4 * g + q, m = m0 + r;
-            w[q] = 0.0;
-            if (h < H && r < nm) w[q] = ldexp(tile[r * H + h], E[m] - exp_fix(G[(m / kchunk) * Hp + h]));
+            x[q] = 0;
+            if (h < H && r < nm) x[q] = fixed55(tile[r * H + h], exp_fix(G[(m / kchunk) * Hp + h]) - E[m]);
         }
         uint32_t s[NSL];
-        slice4(w, s);
+        digits4(x, s);
 #pragma unroll
         for (int i = 0; i < NSL; ++i) reinterpret_cast<uint32_t*>(W + i * plane + (size_t)h * ldM + m0)[g] = s[i];
     }
@@ -357,10 +376,10 @@ gemm_i8_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
 #pragma unroll
                     for (int c = 0; c < 8; ++c) {
                         const int h = h0 + c;
-                        // levels 7 down to 0: acc = sum_k level_k * 2^-7k (every step exact up to one rounding)
+                        // levels 6 down to 0: acc = sum_k level_k * 2^-8k (every step exact up to one rounding)
                         double acc = (double)(int)v[NSL - 1][c];
 #pragma unroll
-                        for (int k = NSL - 2; k >= 0; --k) acc = fma(acc, 0x1p-7, (double)(int)v[k][c]);
+                        for (int k = NSL - 2; k >= 0; --k) acc = fma(acc, 0x1p-8, (double)(int)v[k][c]);
                         if (live && h < H) {
                             const double x = ldexp(acc, re + ce[h] - 14);
                             double* p = o + (size_t)h * hs;
