@@ -484,9 +484,10 @@ static int ctx_slices(vbmf_b200_ctx* c, bool* ok) {
     if (c->z_ready) { *ok = true; return 0; }
     const int ldZ = i8_ld(c->L);
     const size_t bytes = (size_t)I8_NSL * c->Mloc * ldZ;
+    // Zexp = F[L], E[Mloc], Fbad[L], Ebad[Mloc]; sized by ldZ >= L because a re-attach with the same Z_bytes may change L
     if (c->Z == nullptr || c->Z_bytes != bytes || c->ldZ != ldZ) {
         ctx_free_Z(c);
-        if (cudaMalloc(&c->Z, bytes) != cudaSuccess || cudaMalloc(&c->Zexp, ((size_t)c->L + c->Mloc) * 4) != cudaSuccess) {
+        if (cudaMalloc(&c->Z, bytes) != cudaSuccess || cudaMalloc(&c->Zexp, 2 * ((size_t)ldZ + c->Mloc) * 4) != cudaSuccess) {
             cudaGetLastError();
             ctx_free_Z(c);
             c->z_failed = true;
@@ -494,7 +495,8 @@ static int ctx_slices(vbmf_b200_ctx* c, bool* ok) {
         }
         c->Z_bytes = bytes; c->ldZ = ldZ;
     }
-    if (i8_build_Y(c->st, c->Y, c->ldY, c->L, c->Mloc, c->Z, ldZ, c->Zexp, c->Zexp + c->L)) return -1;
+    int* F = c->Zexp;
+    if (i8_build_Y(c->st, c->Y, c->ldY, c->L, c->Mloc, c->Z, ldZ, F, F + c->L, F + c->L + c->Mloc, F + 2 * c->L + c->Mloc)) return -1;
     const uint64_t s1 = (uint64_t)ldZ, s2 = (uint64_t)ldZ * c->Mloc;
     if (make_tmap_3d_i8(&c->tmZ1, c->Z, (uint64_t)c->L, (uint64_t)c->Mloc, I8_NSL, s1, s2, 32, 128, I8_NSL, false)) return -1;
     if (make_tmap_3d_i8(&c->tmZ2, c->Z, (uint64_t)c->L, (uint64_t)c->Mloc, I8_NSL, s1, s2, 128, 32, I8_NSL, true)) return -1;
@@ -541,16 +543,18 @@ static int i8_operands_alloc(I8Operands* o, int L, int M, int H, int S, bool* ok
 static int i8_k1(vbmf_b200_ctx* c, I8Operands* o, const double* B, int ldB, int H, double* P, int S1, int kbs1, const Scalars* sc) {
     const int* F = c->Zexp;
     const int* E = c->Zexp + c->L;
+    const int* Ebad = c->Zexp + 2 * c->L + c->Mloc;
     if (i8_slice_B(c->st, B, ldB, c->L, H, F, o->Wb, c->ldZ, o->Gb, sc)) return -1;
-    return launch_gemm_i8(c->st, false, &c->tmZ1, &o->tmWb, P, c->Mloc, c->L, S1, kbs1 * 16, H, E, o->Gb, 0,
+    return launch_gemm_i8(c->st, false, &c->tmZ1, &o->tmWb, P, c->Mloc, c->L, S1, kbs1 * 16, H, E, Ebad, o->Gb, 0,
                           (size_t)c->Mloc * H, (size_t)H, 1, sc, c->num_sms);
 }
 // K2 on the INT8 path: S slabs [H][ldQ] of Y * A (A row-major [Mloc][H])
 static int i8_k2(vbmf_b200_ctx* c, I8Operands* o, const double* A, int H, double* Qpart, int ldQ, int S, int kchunk, const Scalars* sc) {
     const int* F = c->Zexp;
     const int* E = c->Zexp + c->L;
+    const int* Fbad = c->Zexp + c->L + c->Mloc;
     if (i8_slice_A(c->st, A, c->Mloc, H, E, kchunk, S, o->Wa, o->ldM, o->Ga, sc)) return -1;
-    return launch_gemm_i8(c->st, true, &c->tmZ2, &o->tmWa, Qpart, c->L, c->Mloc, S, kchunk, H, F, o->Ga, i8_hpad(H),
+    return launch_gemm_i8(c->st, true, &c->tmZ2, &o->tmWa, Qpart, c->L, c->Mloc, S, kchunk, H, F, Fbad, o->Ga, i8_hpad(H),
                           (size_t)H * ldQ, 1, (size_t)ldQ, sc, c->num_sms);
 }
 

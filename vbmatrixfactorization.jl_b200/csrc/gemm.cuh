@@ -58,19 +58,21 @@ int gemm_i8_init_device();
 // rank-3 uint8 tensor map {d0, d1, d2} with byte pitches s1, s2; 32-byte swizzle, or 128-byte with swizzle128
 int make_tmap_3d_i8(CUtensorMap* out, const void* base, uint64_t d0, uint64_t d1, uint64_t d2, uint64_t s1, uint64_t s2,
                     uint32_t b0, uint32_t b1, uint32_t b2, bool swizzle128);
-// Y (L x M, column-major) -> row exponents F[L], column exponents E[M], digits Z [7][M][ldZ] (ldZ = i8_ld(L))
-int i8_build_Y(cudaStream_t st, const double* Y, int ldY, int L, int M, uint8_t* Z, int ldZ, int* F, int* E);
+// Y (L x M, column-major) -> row exponents F[L], column exponents E[M] (both over the finite values), digits Z [7][M][ldZ]
+// (ldZ = i8_ld(L)), and the flags Fbad[L] / Ebad[M]: row / column holds a NaN or Inf
+int i8_build_Y(cudaStream_t st, const double* Y, int ldY, int L, int M, uint8_t* Z, int ldZ, int* F, int* E, int* Fbad, int* Ebad);
 // K1 operand: diag(2^F) * B (B column-major [H][ldB]) -> exponents G[Hp], digits W [7][Hp][ldZ]
 int i8_slice_B(cudaStream_t st, const double* B, int ldB, int L, int H, const int* F, uint8_t* W, int ldZ, int* G, const Scalars* sc);
 // K2 operand: diag(2^E) * A (A row-major [M][H]) -> exponents G[S][Hp] per split-K chunk of kchunk rows, digits W [7][Hp][ldM]
 int i8_slice_A(cudaStream_t st, const double* A, int M, int H, const int* E, int kchunk, int S, uint8_t* W, int ldM, int* G, const Scalars* sc);
-// out[s*slab + row*rs + h*hs] = 2^(rowexp[row] + colexp[s*cstride + h]) * sum_{k in split s} A(row, k) * B(k, h).
+// out[s*slab + row*rs + h*hs] = 2^(rowexp[row] + colexp[s*cstride + h]) * sum_{k in split s} A(row, k) * B(k, h), NaN where
+// rowbad[row] != 0 or the operand column held a NaN or Inf (non-finite inputs give NaN, never a finite value).
 // mn = false (K1): tmA = Y digits {L, M, 7}, box {32, 128, 7}, 32-byte swizzle; rows are columns of Y, k = l.
 // mn = true  (K2): tmA = Y digits {L, M, 7}, box {128, 32, 7}, 128-byte swizzle; rows are rows of Y, k = m.
 // tmB: operand digits {kdim, Hp, 7}, box {32, Hp, 7}, 32-byte swizzle.  klen: split length, a multiple of 32.
 int launch_gemm_i8(cudaStream_t st, bool mn, const CUtensorMap* tmA, const CUtensorMap* tmB, double* out, int nrows, int kdim,
-                   int S, int klen, int H, const int* rowexp, const int* colexp, int cstride, size_t slab, size_t rs, size_t hs,
-                   const Scalars* sc, int num_sms);
+                   int S, int klen, int H, const int* rowexp, const int* rowbad, const int* colexp, int cstride, size_t slab,
+                   size_t rs, size_t hs, const Scalars* sc, int num_sms);
 
 // Plain SIMT FP64 versions (debug / cross-check only; selected with VBMF_B200_GEMM=simt).
 int launch_gemm_ytb_simt(cudaStream_t st, const double* Y, int ldY, const double* B, int ldB, double* P,

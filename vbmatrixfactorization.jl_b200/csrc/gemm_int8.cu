@@ -45,6 +45,7 @@ static_assert(SMEM <= 227 * 1024, "stage ring exceeds the shared memory of one C
 constexpr int SEG_KB = 16384 / KB;      // k-blocks per flush: level 6 stays below 2^31
 static_assert((long long)SEG_KB * KB * NSL * 128 * 128 < (1ll << 31), "level 6 may overflow INT32 between flushes");
 constexpr int EXP_NONE = -(1 << 30);    // exponent of 0 (and of non-finite values): below every real exponent
+constexpr int EXP_NAN = 1 << 30;        // operand column exponent of a column with a non-finite value: above every real one
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
@@ -111,8 +112,9 @@ __device__ __forceinline__ int exp_digits(double x) {
 }
 __device__ __forceinline__ int exp_fix(int e) { return e <= EXP_NONE ? 0 : e; }
 
-// rint(x * 2^(55 - e)): the digits' fixed-point form of w = x * 2^-e (|w| <= 127/128, so |result| <= 127 * 2^48)
-__device__ __forceinline__ long long fixed55(double x, int e) { return __double2ll_rn(ldexp(x, 55 - e)); }
+// rint(x * 2^(55 - e)): the digits' fixed-point form of w = x * 2^-e (|w| <= 127/128, so |result| <= 127 * 2^48).
+// Non-finite values get zero digits; the outputs they reach are set to NaN from the flags instead.
+__device__ __forceinline__ long long fixed55(double x, int e) { return isfinite(x) ? __double2ll_rn(ldexp(x, 55 - e)) : 0ll; }
 
 // seven balanced radix-256 digits of X = rint(w * 2^55): w = sum_i d_i 2^-(7+8i), d_i in [-128, 127], taken from the bottom.
 // The digit is the low byte read as signed; X - d is then a multiple of 256.  Four consecutive values per 32-bit word: byte q
@@ -150,27 +152,38 @@ __device__ __forceinline__ int block_max_int(int v, int* red) {
 }
 
 // ------------------------------------------------------------------------------------------- slices of Y (once per attach)
-__global__ void __launch_bounds__(256) y_row_exp_kernel(const double* __restrict__ Y, int ldY, int L, int M, int* __restrict__ F) {
+// F_l = frexp exponent of the row maximum over the finite values; Fbad[l] = 1 when row l holds a NaN or Inf (zeroed before)
+__global__ void __launch_bounds__(256) y_row_exp_kernel(const double* __restrict__ Y, int ldY, int L, int M, int* __restrict__ F,
+                                                        int* __restrict__ Fbad) {
     const int l = blockIdx.x * blockDim.x + threadIdx.x;
     if (l >= L) return;
     int e = EXP_NONE;
-    for (int m = blockIdx.y; m < M; m += gridDim.y) e = max(e, exp_of(Y[(size_t)m * ldY + l]));
+    bool bad = false;
+    for (int m = blockIdx.y; m < M; m += gridDim.y) {
+        const double y = Y[(size_t)m * ldY + l];
+        e = max(e, exp_of(y));
+        bad |= !isfinite(y);
+    }
     atomicMax(F + l, e);
+    if (bad) Fbad[l] = 1;
 }
 
-// one CTA per column m: E_m, then the column's seven digit planes (4 rows per thread and 32-bit word)
+// one CTA per column m: E_m over the finite values and Ebad[m] (column m holds a NaN or Inf), then the column's seven digit
+// planes (4 rows per thread and 32-bit word)
 __global__ void __launch_bounds__(256) y_slices_kernel(const double* __restrict__ Y, int ldY, int L, int M, const int* __restrict__ F,
-                                                       int* __restrict__ E, uint8_t* __restrict__ Z, int ldZ) {
+                                                       int* __restrict__ E, int* __restrict__ Ebad, uint8_t* __restrict__ Z, int ldZ) {
     __shared__ int red[32];
     const int m = blockIdx.x;
     const double* y = Y + (size_t)m * ldY;
-    int e = EXP_NONE;
+    int e = EXP_NONE, bad = 0;
     for (int l = threadIdx.x; l < L; l += blockDim.x) {
         const int ey = exp_digits(y[l]);
         if (ey > EXP_NONE) e = max(e, ey - exp_fix(F[l]));
+        bad |= !isfinite(y[l]);
     }
+    bad = __syncthreads_or(bad);
     const int Em = exp_fix(block_max_int(e, red));
-    if (threadIdx.x == 0) E[m] = Em;
+    if (threadIdx.x == 0) { E[m] = Em; Ebad[m] = bad; }
     const size_t plane = (size_t)M * ldZ;
     for (int l4 = threadIdx.x; l4 < ldZ / 4; l4 += blockDim.x) {
         long long x[4];
@@ -187,20 +200,23 @@ __global__ void __launch_bounds__(256) y_slices_kernel(const double* __restrict_
 }
 
 // ------------------------------------------------------------------------------------------- K1 operand: digits of diag(2^F) B
-// one CTA per column h < Hp (rows h >= H are zero): G_h, then the column's digits, layout [7][Hp][ldZ]
+// one CTA per column h < Hp (rows h >= H are zero): G_h (EXP_NAN when the column holds a NaN or Inf), then the column's
+// digits, layout [7][Hp][ldZ]
 __global__ void __launch_bounds__(512) b_slices_kernel(const double* __restrict__ B, int ldB, int L, int H, int Hp, const int* __restrict__ F,
                                                        uint8_t* __restrict__ W, int ldZ, int* __restrict__ G, const Scalars* __restrict__ sc) {
     if (sc != nullptr && !sc->active) return;
     __shared__ int red[32];
     const int h = blockIdx.x;
     const double* b = B + (size_t)h * ldB;
-    int e = EXP_NONE;
+    int e = EXP_NONE, bad = 0;
     if (h < H)
         for (int l = threadIdx.x; l < L; l += blockDim.x) {
             const int eb = exp_digits(b[l]);
             if (eb > EXP_NONE) e = max(e, eb + exp_fix(F[l]));
+            bad |= !isfinite(b[l]);
         }
-    const int Gh = exp_fix(block_max_int(e, red));
+    bad = __syncthreads_or(bad);
+    const int Gh = bad ? EXP_NAN : exp_fix(block_max_int(e, red));
     if (threadIdx.x == 0) G[h] = Gh;
     const size_t plane = (size_t)Hp * ldZ;
     for (int l4 = threadIdx.x; l4 < ldZ / 4; l4 += blockDim.x) {
@@ -219,7 +235,8 @@ __global__ void __launch_bounds__(512) b_slices_kernel(const double* __restrict_
 
 // ------------------------------------------------------------------------------------------- K2 operand: digits of diag(2^E) A
 // A is [M][H] (row m contiguous in h).  Exponents per (split-K chunk, column): G[c][h] = max over m in chunk c (atomicMax on
-// integers: order-independent).  256 rows per CTA, thread = (h = t % 64, rows t / 64 + 4 r).
+// integers: order-independent), EXP_NAN when the chunk of the column holds a NaN or Inf.  256 rows per CTA, thread =
+// (h = t % 64, rows t / 64 + 4 r).
 __global__ void __launch_bounds__(256) a_exp_kernel(const double* __restrict__ A, int M, int H, int Hp, const int* __restrict__ E, int kchunk,
                                                     int* __restrict__ G, const Scalars* __restrict__ sc) {
     if (sc != nullptr && !sc->active) return;
@@ -233,8 +250,10 @@ __global__ void __launch_bounds__(256) a_exp_kernel(const double* __restrict__ A
             if (cur >= 0 && e > EXP_NONE) atomicMax(G + cur * Hp + h, e);
             cur = c; e = EXP_NONE;
         }
-        const int ea = exp_digits(A[(size_t)m * H + h]);
-        if (ea > EXP_NONE) e = max(e, ea + E[m]);
+        const double a = A[(size_t)m * H + h];
+        const int ea = exp_digits(a);
+        if (!isfinite(a)) e = EXP_NAN;
+        else if (ea > EXP_NONE) e = max(e, ea + E[m]);
     }
     if (cur >= 0 && e > EXP_NONE) atomicMax(G + cur * Hp + h, e);
 }
@@ -269,12 +288,13 @@ __global__ void __launch_bounds__(256) a_slices_kernel(const double* __restrict_
 // ------------------------------------------------------------------------------------------- the contraction
 // Work item w: tile = w % ntile (128 output rows), split s = w / ntile (k range [s*klen, min(kdim, (s+1)*klen)), klen a
 // multiple of 32).  Output element (row, h) of slab s: out[s*slab + row*rs + h*hs] = 2^(rowexp[row] + colexp[s*cstride + h])
-// * sum over the k range; rows >= nrows and h >= H are not written.
+// * sum over the k range, or NaN when rowbad[row] is set or the column exponent is EXP_NAN (a non-finite input reaches the
+// element); rows >= nrows and h >= H are not written.
 template <bool MN>
 __global__ void __launch_bounds__(192, 1)
 gemm_i8_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, double* __restrict__ out,
                int nrows, int kdim, int S, int klen, int H, int Hp, const int* __restrict__ rowexp,
-               const int* __restrict__ colexp, int cstride, size_t slab, size_t rs, size_t hs, const Scalars* __restrict__ sc) {
+               const int* __restrict__ rowbad, const int* __restrict__ colexp, int cstride, size_t slab, size_t rs, size_t hs, const Scalars* __restrict__ sc) {
     if (sc != nullptr && !sc->active) return;
     extern __shared__ uint8_t smem_raw[];
     const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
@@ -363,6 +383,7 @@ gemm_i8_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             const int row = tile * TM + warp * 32 + lane;
             const bool live = row < nrows;
             const int re = live ? rowexp[row] : 0;
+            const bool bad = live && rowbad[row] != 0;
             double* o = out + (size_t)sp * slab + (size_t)(live ? row : 0) * rs;
             const int* ce = colexp + (size_t)sp * cstride;
             for (int kb0 = 0; kb0 < nkb; kb0 += SEG_KB, ++sg) {
@@ -381,7 +402,8 @@ gemm_i8_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
 #pragma unroll
                         for (int k = NSL - 2; k >= 0; --k) acc = fma(acc, 0x1p-8, (double)(int)v[k][c]);
                         if (live && h < H) {
-                            const double x = ldexp(acc, re + ce[h] - 14);
+                            const double x = (bad || ce[h] == EXP_NAN) ? __longlong_as_double(0x7ff8000000000000ll)
+                                                                       : ldexp(acc, re + ce[h] - 14);
                             double* p = o + (size_t)h * hs;
                             *p = kb0 == 0 ? x : *p + x;
                         }
@@ -435,13 +457,14 @@ int gemm_i8_init_device() {
     return 0;
 }
 
-int i8_build_Y(cudaStream_t st, const double* Y, int ldY, int L, int M, uint8_t* Z, int ldZ, int* F, int* E) {
+int i8_build_Y(cudaStream_t st, const double* Y, int ldY, int L, int M, uint8_t* Z, int ldZ, int* F, int* E, int* Fbad, int* Ebad) {
     if (L <= 0 || M <= 0) return 0;
     VB_CUDA_OK(cudaMemsetAsync(F, 0x80, (size_t)L * 4, st));
+    VB_CUDA_OK(cudaMemsetAsync(Fbad, 0, (size_t)L * 4, st));
     dim3 g1((L + 255) / 256, std::min(M, 512));
-    y_row_exp_kernel<<<g1, 256, 0, st>>>(Y, ldY, L, M, F);
+    y_row_exp_kernel<<<g1, 256, 0, st>>>(Y, ldY, L, M, F, Fbad);
     VB_LAUNCH_OK();
-    y_slices_kernel<<<M, 256, 0, st>>>(Y, ldY, L, M, F, E, Z, ldZ);
+    y_slices_kernel<<<M, 256, 0, st>>>(Y, ldY, L, M, F, E, Ebad, Z, ldZ);
     VB_LAUNCH_OK();
     return 0;
 }
@@ -465,15 +488,15 @@ int i8_slice_A(cudaStream_t st, const double* A, int M, int H, const int* E, int
 }
 
 int launch_gemm_i8(cudaStream_t st, bool mn, const CUtensorMap* tmA, const CUtensorMap* tmB, double* out, int nrows, int kdim,
-                   int S, int klen, int H, const int* rowexp, const int* colexp, int cstride, size_t slab, size_t rs, size_t hs,
-                   const Scalars* sc, int num_sms) {
+                   int S, int klen, int H, const int* rowexp, const int* rowbad, const int* colexp, int cstride, size_t slab,
+                   size_t rs, size_t hs, const Scalars* sc, int num_sms) {
     if (H > 64) { set_error("H = %d > 64 is not supported by the INT8 contraction", H); return -1; }
     if (klen % KB != 0) { set_error("INT8 split-K chunk %d is not a multiple of %d", klen, KB); return -1; }
     if (nrows <= 0 || kdim <= 0 || H <= 0) return 0;
     const int nwork = ((nrows + TM - 1) / TM) * S;
     const int grid = std::max(1, std::min(nwork, num_sms));
-    if (mn) gemm_i8_kernel<true><<<grid, 192, SMEM, st>>>(*tmA, *tmB, out, nrows, kdim, S, klen, H, i8_hpad(H), rowexp, colexp, cstride, slab, rs, hs, sc);
-    else gemm_i8_kernel<false><<<grid, 192, SMEM, st>>>(*tmA, *tmB, out, nrows, kdim, S, klen, H, i8_hpad(H), rowexp, colexp, cstride, slab, rs, hs, sc);
+    if (mn) gemm_i8_kernel<true><<<grid, 192, SMEM, st>>>(*tmA, *tmB, out, nrows, kdim, S, klen, H, i8_hpad(H), rowexp, rowbad, colexp, cstride, slab, rs, hs, sc);
+    else gemm_i8_kernel<false><<<grid, 192, SMEM, st>>>(*tmA, *tmB, out, nrows, kdim, S, klen, H, i8_hpad(H), rowexp, rowbad, colexp, cstride, slab, rs, hs, sc);
     VB_LAUNCH_OK();
     return 0;
 }

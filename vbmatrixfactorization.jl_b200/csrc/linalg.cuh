@@ -318,6 +318,11 @@ __device__ __forceinline__ bool block_spd_inverse_reg(double (&a)[Q], const int 
 // Householder tridiagonalisation followed by parallel multisection on the Sturm sequence: orthogonal similarity +
 // bisection, so lambda_max carries an absolute error of a few ulp of ||A|| (what LAPACK's SVD gives the reference for
 // norm(::Matrix)).  work = 4*n doubles.  Whole CTA (blockDim.x >= 64, multiple of 32); result valid in every thread.
+// A is first scaled by 2^-e so that its largest entry lies in [1/2, 1), and lambda is scaled back by 2^e: the Sturm
+// recurrence is division-free and would overflow or underflow for entries beyond about 1e+-77.  The scale itself is exact and
+// every input scale then runs on the same matrix, but the every-4-steps rescale picks max(|p_{i-1}|, |p_i|), whose winner
+// depends on the scale, so against the unscaled recurrence lambda may move in its last bits.  An all-zero matrix gives
+// exactly 0.
 __device__ inline double sym_lambda_max(double* A, int ld, int n, double* work) {
     const int t = threadIdx.x, nt = blockDim.x, lane = t & 31, warp = t >> 5;
     double* dv = work;            // diagonal of T
@@ -327,12 +332,27 @@ __device__ inline double sym_lambda_max(double* A, int ld, int n, double* work) 
     __shared__ double s_sc[4];    // beta, alpha, K, flag
     __shared__ double s_lo, s_hi;
     __shared__ int s_first;
+    __shared__ unsigned long long s_amax;   // bit pattern of max |A_ij| (non-negative doubles order as their bit patterns)
     if (n <= 0) return 0.0;
+    if (t == 0) s_amax = 0ull;
     // NaN / Inf anywhere -> NaN (the reference's norm would propagate it)
     int bad = 0;
-    for (int e = t; e < n * n; e += nt) { const double x = A[(e / n) * ld + (e % n)]; if (!(fabs(x) <= 1.79e308)) bad = 1; }
+    double amax = 0.0;
+    for (int e = t; e < n * n; e += nt) {
+        const double x = A[(e / n) * ld + (e % n)];
+        if (!(fabs(x) <= 1.79e308)) bad = 1;
+        else amax = fmax(amax, fabs(x));
+    }
     if (__syncthreads_or(bad)) return nan("");
     if (n == 1) return A[0];
+    atomicMax(&s_amax, (unsigned long long)__double_as_longlong(amax));
+    __syncthreads();
+    const double big = __longlong_as_double((long long)s_amax);
+    if (big == 0.0) return 0.0;
+    int escale;
+    frexp(big, &escale);
+    for (int e = t; e < n * n; e += nt) { double* x = A + (e / n) * ld + (e % n); *x = ldexp(*x, -escale); }
+    __syncthreads();
     for (int k = 0; k < n - 2; ++k) {
         const int m = n - k - 1;                  // trailing block is rows/cols k+1 .. n-1
         double* Asub = A + (k + 1) * ld + (k + 1);
@@ -438,7 +458,7 @@ __device__ inline double sym_lambda_max(double* A, int ld, int n, double* work) 
         }
         __syncthreads();
     }
-    return 0.5 * (s_lo + s_hi);
+    return ldexp(0.5 * (s_lo + s_hi), escale);
 }
 
 }  // namespace vb
