@@ -1,7 +1,8 @@
 // Stand-alone timing + correctness probe for K4 (per-column H x H SPD inverses of the full-covariance A update,
 // src/vbmf_sparse.jl:178-202): links the library's kernels.o, drives k_sparse_A_full on synthetic ARD-like precisions and
 // compares with a host long-double Gauss-Jordan.  Development tool, not part of the product path.
-//   k4bench <dmma|reg> [H=32] [M=100000] [reps=20]
+//   k4bench [H=32] [M=100000] [reps=20]
+//   k4bench hxh <H> [reps=50]
 #include "../../vbmatrixfactorization.jl_b200/csrc/kernels.cuh"
 #include <cstdarg>
 #include <cstdlib>
@@ -73,16 +74,14 @@ static int bench_hxh(int H, int reps) {
     CK(cudaMemcpy(hSA.data(), dSA, HH * 8, cudaMemcpyDeviceToHost));
     double err = 0, mx = 0;
     for (size_t e = 0; e < HH; ++e) { err = std::max(err, fabs(hSA[e] - s2 * Si[e])); mx = std::max(mx, fabs(s2 * Si[e])); }
-    printf("{\"kernel\": \"hxh (k_dense_sigmaA)\", \"mode\": \"%s\", \"H\": %d, \"us_per_launch\": %.2f, \"rel_err\": %.3g}\n",
-           getenv("VBMF_B200_HXH") ? getenv("VBMF_B200_HXH") : "dmma", H, ms / reps * 1e3, err / mx);
+    printf("{\"kernel\": \"hxh (k_dense_sigmaA)\", \"H\": %d, \"us_per_launch\": %.2f, \"rel_err\": %.3g}\n", H, ms / reps * 1e3, err / mx);
     return 0;
 }
 
 int main(int argc, char** argv) {
     if (argc > 2 && strcmp(argv[1], "hxh") == 0) return bench_hxh(atoi(argv[2]), argc > 3 ? atoi(argv[3]) : 50);
-    const char* mode = argc > 1 ? argv[1] : "dmma";
-    const int H = argc > 2 ? atoi(argv[2]) : 32, M = argc > 3 ? atoi(argv[3]) : 100000, reps = argc > 4 ? atoi(argv[4]) : 20;
-    if (strcmp(mode, "reg") == 0) setenv("VBMF_B200_K4", "reg", 1);
+    const int H = argc > 1 ? atoi(argv[1]) : 32, M = argc > 2 ? atoi(argv[2]) : 100000, reps = argc > 3 ? atoi(argv[3]) : 20;
+    if (H < 1 || H > 128 || M < 1 || reps < 1) { fprintf(stderr, "usage: k4bench [H=32] [M=100000] [reps=20] | k4bench hxh <H> [reps=50]\n"); return 2; }
     CK(cudaSetDevice(0));
     if (kernels_init_device()) return 1;
     const int L = 64, ldB = 64;
@@ -141,9 +140,9 @@ int main(int argc, char** argv) {
     if (stride == 1) { double mx = 0; errS = 0; for (size_t e = 0; e < HH; ++e) { mx = std::max(mx, fabs((double)SA[e])); errS = std::max(errS, fabs(hSA[e] - (double)SA[e])); } errS /= mx; }
     int fail = 0; CK(cudaMemcpy(&hs, dsc, sizeof(hs), cudaMemcpyDeviceToHost)); fail = hs.chol_fail;
     const double per = ms / reps;
-    printf("{\"kernel\": \"k_sparse_A_full\", \"mode\": \"%s\", \"minb\": \"%s\", \"H\": %d, \"M\": %d, \"ms_per_launch\": %.4f, \"inverses_per_s\": %.4g, "
+    printf("{\"kernel\": \"k_sparse_A_full\", \"H\": %d, \"M\": %d, \"ms_per_launch\": %.4f, \"inverses_per_s\": %.4g, "
            "\"gflops_2H3\": %.1f, \"rel_err_A\": %.3g, \"rel_err_diag\": %.3g, \"rel_err_sumSigma\": %.3g, \"chol_fail\": %d}\n",
-           mode, getenv("VBMF_B200_K4_MINB") ? getenv("VBMF_B200_K4_MINB") : "3", H, M, per, M / (per * 1e-3), 2.0 * H * H * H * M / (per * 1e-3) * 1e-9,
+           H, M, per, M / (per * 1e-3), 2.0 * H * H * H * M / (per * 1e-3) * 1e-9,
            errA / maxA, errD, errS, fail);
     return 0;
 }

@@ -796,8 +796,6 @@ struct vbmf_b200_solver {
     size_t arena_bytes = 0;
     double* Qpart = nullptr;
     int S = 1, kchunk = 16;
-    bool k2_sk = false;           // K2 uses the stream-K decomposition (gemm_dmma.cu)
-    int sk_kq = 64, sk_nk = 1, sk_grid = 1, sk_smax = 1;
     double* Ppart = nullptr;      // split-K slabs of K1 (nullptr when S1 == 1)
     int S1 = 1, kbs1 = 1;
     int* d_labels = nullptr;
@@ -877,15 +875,6 @@ static int solver_create_impl(vbmf_b200_ctx* c, int kind, int64_t H, int64_t h_s
         }
     }
     s->k2_simt = c->simt || (H % 2 != 0);       // the A tensor map needs a 16-byte row pitch
-    {   // stream-K for K2: opt-in (VBMF_B200_K2=streamk).  It removes the 16 slabs of L x H (reduction 28 -> 18 us at
-        // 20000 x 25000 x 64) but the kernel itself measured 4-5 % slower than the classic split (15.0 vs 14.4 ms at config 3,
-        // 1.89 vs 1.82 ms on a 25000-column shard: the tile-change test, the flush path and 26 more registers), so the
-        // classic decomposition stays the default.
-        const char* e = getenv("VBMF_B200_K2");
-        const bool want = e != nullptr && strcmp(e, "streamk") == 0;
-        s->k2_sk = !s->k2_simt && want && d.Mloc > 0;
-        if (s->k2_sk) plan_streamk(d.L, d.Mloc, d.H, c->num_sms, &s->sk_kq, &s->sk_nk, &s->sk_grid, &s->sk_smax);
-    }
 
     const size_t MH = (size_t)std::max(d.Mloc, 1) * H, LH = (size_t)H * d.ldB, HH = (size_t)H * H, Lr = (size_t)d.L;
     const size_t part_elems = std::max<size_t>({(size_t)MAX_PARTS * HH, (size_t)2400 * std::min<size_t>(H, 32) * std::min<size_t>(H, 32),
@@ -909,7 +898,7 @@ static int solver_create_impl(vbmf_b200_ctx* c, int kind, int64_t H, int64_t h_s
         {&d.A, MH}, {&d.P, MH}, {&d.Bold, LH}, {&d.D, LH}, {&d.Bs, LH},
         {&d.SigmaA, HH}, {&d.SigmaB, HH}, {&d.BtB, HH}, {&d.BtBw, HH}, {&d.DtD, HH}, {&d.Gm, HH},
         {&d.sigmaVec, Lr}, {&d.etaVec, Lr}, {&d.zetaVec, Lr}, {&d.part, part_elems}, {&d.lbacc, 32},
-        {&s->Qpart, (size_t)std::max(std::max(s->S, s->S_chunk), s->k2_sk ? s->sk_smax : 1) * LH},
+        {&s->Qpart, (size_t)std::max(s->S, s->S_chunk) * LH},
     };
     if (s->S1 > 1) items.push_back({&s->Ppart, (size_t)s->S1 * MH});
     if (s->px) {
@@ -1284,13 +1273,11 @@ static int enq_k2(vbmf_b200_solver* s) {
     int rc;
     if (i8) rc = i8_k2(c, &s->i8o, d.A, d.H, s->Qpart, d.ldB, s->S, s->kchunk, d.sc);
     else if (s->k2_simt) rc = launch_gemm_ya_simt(c->st, d.Y, d.ldY, d.A, s->Qpart, d.L, d.Mloc, d.H, d.ldB, s->kchunk, s->S, d.sc);
-    else if (s->k2_sk) rc = launch_gemm_ya_sk(c->st, &c->tmY2, &s->tmA, s->Qpart, d.packed + packed_q(d), d.L, d.Mloc, d.H, d.ldB, s->sk_kq, s->sk_nk, s->sk_grid, d.sc);
     else rc = launch_gemm_ya(c->st, &c->tmY2, &s->tmA, s->Qpart, d.L, d.Mloc, d.H, d.ldB, s->kchunk, s->S, d.sc, c->num_sms);
     prof_mark(c, c->ev_k2);
     prof_seg(c, SEG_K2);
     if (rc) return rc;
-    if (s->k2_sk && !i8) rc = launch_reduce_q_sk(c->st, s->Qpart, d.packed + packed_q(d), d.L, d.Mloc, d.H, d.ldB, s->sk_nk, s->sk_grid, d.sc);
-    else rc = k_reduce_q(c->st, d, s->Qpart, s->S);
+    rc = k_reduce_q(c->st, d, s->Qpart, s->S);
     prof_seg(c, SEG_REDUCE_Q);
     return rc;
 }
@@ -1344,7 +1331,7 @@ static int enq_updateA(vbmf_b200_solver* s, int flags, bool fused) {
         const bool dv = (flags & F_DIAG_VAR) != 0;
         // (H > 64: the fused kernel's 68 Gram accumulator registers leave one CTA per SM and it loses to the separate
         //  passes, 0.74 vs 0.55 ms at 125000 x 128)
-        if (fused && !(flags & F_FULL_COV) && d.H <= 64 && getenv("VBMF_B200_NO_DIAG_FUSION") == nullptr) {
+        if (fused && !(flags & F_FULL_COV) && d.H <= 64) {
             // whole-loop diagonal path: slab sum, A, diag, mask, updateCA! and A'A in one pass over vec(A')
             if (enq_k1(s, dv, false) || wait_post(s)) return -1;
             const bool slabs = !s->c->simt && s->S1 > 1;
@@ -1353,20 +1340,6 @@ static int enq_updateA(vbmf_b200_solver* s, int flags, bool fused) {
             if (k_sparse_A_diag_fused(st, d, slabs ? s->Ppart : d.P, slabs ? s->S1 : 1, (size_t)d.Mloc * d.H, flags, defer ? &s->diag_parts : nullptr)) return -1;
             s->ata_valid = false; s->q_valid = false;
             s->ata_local = true; s->ca_done = true;
-            return 0;
-        }
-        if (fused && (flags & F_FULL_COV) && k_sparse_A_full_can_fuse(d) && getenv("VBMF_B200_K4_FUSION") != nullptr) {
-            // optional (VBMF_B200_K4_FUSION=1): the per-column inverse kernel sums the K1 slabs itself and, for the sparse kind,
-            // applies the label mask and updateCA! to the column it has just produced.  Measured neutral on the step time (the
-            // extra dependent global loads / stores sit on each warp's latency chain: 0.475 vs 0.415 ms + two small kernels),
-            // so the separate passes stay the default.
-            if (enq_k1(s, dv, false) || wait_post(s)) return -1;
-            const bool slabs = !s->c->simt && s->S1 > 1;
-            const int fuse_ca = d.kind == KIND_SPARSE ? 1 : 0;
-            if (k_sparse_A_full_ex(st, d, flags, slabs ? s->Ppart : d.P, slabs ? s->S1 : 1, (size_t)d.Mloc * d.H, fuse_ca)) return -1;
-            if (!fuse_ca && k_mask(st, d)) return -1;
-            s->ata_valid = false; s->q_valid = false; s->ata_local = false;
-            s->ca_done = fuse_ca != 0;
             return 0;
         }
         if (enq_k1(s, dv) || wait_post(s)) return -1;
@@ -1640,7 +1613,7 @@ extern "C" int vbmf_b200_solver_run(vbmf_b200_solver* s, int64_t niter, double e
     if (k_set_control(st, d, (int)niter, eps, norm_mode, 0)) return -1;
     s->btb_valid = false;
     s->sigmaA_ahead = false;
-    s->loop_ahead = getenv("VBMF_B200_NO_SIGMAA_AHEAD") == nullptr;
+    s->loop_ahead = true;
     if (enq_gram_B(s, flags) || k_norms_init(st, d)) return -1;      // old = BHat, src/vbmf.jl:188
     int64_t enq = 0;
     int slot = 0;
@@ -1833,10 +1806,6 @@ extern "C" int vbmf_b200_gemm_YA(vbmf_b200_ctx* c, const double* A, int64_t H, d
         if (ctx_slices(c, &i8)) return -1;
         if (i8 && i8_operands_alloc(&o, c->L, c->Mloc, (int)H, S, &i8)) return -1;
     }
-    int kq = 64, nk = 1, skgrid = 1, smax = 1;
-    const char* ek2 = getenv("VBMF_B200_K2");
-    const bool use_sk = !i8 && !(c->simt || (H % 2 != 0)) && c->Mloc > 0 && ek2 != nullptr && strcmp(ek2, "streamk") == 0;
-    if (use_sk) { plan_streamk(c->L, c->Mloc, (int)H, c->num_sms, &kq, &nk, &skgrid, &smax); S = std::max(S, smax); }
     double *dA = nullptr, *dT = nullptr, *dQp = nullptr, *dQ = nullptr;
     VB_CUDA_OK(cudaMalloc(&dA, MH * 8));
     VB_CUDA_OK(cudaMalloc(&dT, MH * 8));
@@ -1852,13 +1821,10 @@ extern "C" int vbmf_b200_gemm_YA(vbmf_b200_ctx* c, const double* A, int64_t H, d
         else {
             CUtensorMap tmA;
             if (c->Mloc > 0) rc = make_tmap_2d(&tmA, dA, (uint64_t)H, (uint64_t)c->Mloc, (uint64_t)H * 8, 16, 16);
-            if (!rc && use_sk) {
-                rc = launch_gemm_ya_sk(c->st, &c->tmY2, &tmA, dQp, dQ, c->L, c->Mloc, (int)H, ldQ, kq, nk, skgrid, nullptr);
-                if (!rc) rc = launch_reduce_q_sk(c->st, dQp, dQ, c->L, c->Mloc, (int)H, ldQ, nk, skgrid, nullptr);
-            } else if (!rc) rc = launch_gemm_ya(c->st, &c->tmY2, &tmA, dQp, c->L, c->Mloc, (int)H, ldQ, kchunk, S, nullptr, c->num_sms);
+            if (!rc) rc = launch_gemm_ya(c->st, &c->tmY2, &tmA, dQp, c->L, c->Mloc, (int)H, ldQ, kchunk, S, nullptr, c->num_sms);
         }
     }
-    if (!rc && !use_sk) {
+    if (!rc) {
         Dev d; memset(&d, 0, sizeof(d));
         d.H = (int)H; d.ldB = ldQ; d.L = c->L; d.packed = dQ;
         Scalars* none = nullptr; d.sc = none;

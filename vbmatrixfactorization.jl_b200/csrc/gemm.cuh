@@ -38,13 +38,6 @@ void plan_splitk_ytb(int L, int M, int H, int num_sms, int* S, int* kb_per_split
 int launch_gemm_ya(cudaStream_t st, const CUtensorMap* tmY, const CUtensorMap* tmA, double* Qpart,
                    int L, int M, int H, int ldQ, int kchunk, int S, const Scalars* sc, int num_sms);
 
-// K2 with the stream-K decomposition (gemm_dmma.cu): Qpart holds smax partial slabs [H][ldQ]; launch_reduce_q_sk sums the partials
-// of every row tile in fixed CTA order into Q.  plan_streamk: unit length kq, units per tile nk, grid, worst-case partials per tile.
-int plan_streamk(int L, int M, int H, int num_sms, int* kq, int* nk, int* grid, int* smax);
-int launch_gemm_ya_sk(cudaStream_t st, const CUtensorMap* tmY, const CUtensorMap* tmA, double* Qpart, double* Q, int L, int M, int H,
-                      int ldQ, int kq, int nk, int grid, const Scalars* sc);
-int launch_reduce_q_sk(cudaStream_t st, const double* Qpart, double* Q, int L, int M, int H, int ldQ, int nk, int grid, const Scalars* sc);
-
 // split-K plan for K2: number of slabs and chunk length (multiple of 16)
 void plan_splitk(int L, int M, int H, int num_sms, int* S, int* kchunk);
 

@@ -305,266 +305,6 @@ gemm_ya_kernel(const __grid_constant__ CUtensorMap tmY, const __grid_constant__ 
     }
 }
 
-// ------------------------------------------------------------------------------------------- K2 without a producer warp
-// At BN = 128 the 16 consumer warps + 1 producer warp make a 17-warp CTA, which the register file serves like 20 warps:
-// 96 registers per thread, address arithmetic recomputed and spilled in the main loop (ncu round 1: 4.1 instructions per
-// DMMA, dmma pipe 94.2 % against K1's 97.2 %).  Here lane 0 of consumer warp 0 issues the TMA loads itself, LAG k-blocks
-// behind its own consumption (so the stage it refills has normally been released by every warp already): 16 warps, 128
-// registers.  Same tiles, same fragment permutation, same results as gemm_ya_kernel.
-template <int BN, int LAG>
-__global__ void __launch_bounds__(Cfg<BN>::WM * Cfg<BN>::WN * 32, Cfg<BN>::CPS)
-gemm_ya_fold_kernel(const __grid_constant__ CUtensorMap tmY, const __grid_constant__ CUtensorMap tmA,
-                    double* __restrict__ Qpart, int L, int M, int H, int ldQ, int kchunk, int S,
-                    const Scalars* __restrict__ sc) {
-    if (sc != nullptr && !sc->active) return;
-    constexpr int WM = Cfg<BN>::WM, WN = Cfg<BN>::WN, STAGES = Cfg<BN>::STAGES;
-    constexpr int NCW = WM * WN;
-    constexpr int MT = BM / WM / 8, NT = BN / WN / 8;
-    static_assert(MT % 4 == 0 && NT % 4 == 0, "K2 needs 32-wide warp tiles");
-    static_assert(LAG >= 1 && LAG < STAGES, "refill lag");
-    constexpr int YB = BM * BK * 8, SB = Sizes<BN>::STAGE;
-
-    extern __shared__ uint8_t smem_raw[];
-    const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-    const uint32_t full0 = base + STAGES * SB, empty0 = full0 + STAGES * 8;
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    if (threadIdx.x == 0) {
-        for (int s = 0; s < STAGES; ++s) { mbar_init(full0 + 8 * s, 1); mbar_init(empty0 + 8 * s, NCW); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    }
-    __syncthreads();
-
-    const int ntl = (L + BM - 1) / BM;
-    const int nwork = ntl * S;
-    const bool prod = threadIdx.x == 0;
-
-    // producer cursor (thread 0 only): next k-block to issue
-    int pw = blockIdx.x, pk = 0, pk_end = 0, pl0 = 0;
-    uint32_t pit = 0;
-    bool pmore = pw < nwork;
-    if (pmore) { const int kc = pw / ntl; pl0 = (pw % ntl) * BM; pk = kc * kchunk; pk_end = min(M, pk + kchunk); }
-    auto issue = [&]() {
-        const uint32_t s = pit % STAGES, ph = (pit / STAGES) & 1;
-        mbar_wait(empty0 + 8 * s, ph ^ 1);
-        mbar_expect_tx(full0 + 8 * s, SB);
-        const uint32_t dst = base + s * SB;
-#pragma unroll
-        for (int b = 0; b < BM / 16; ++b) tma_load_2d(dst + b * BOX, &tmY, full0 + 8 * s, pl0 + 16 * b, pk);
-#pragma unroll
-        for (int b = 0; b < BN / 16; ++b) tma_load_2d(dst + YB + b * BOX, &tmA, full0 + 8 * s, 16 * b, pk);
-        ++pit;
-        pk += BK;
-        if (pk >= pk_end) {
-            pw += gridDim.x;
-            pmore = pw < nwork;
-            if (pmore) { const int kc = pw / ntl; pl0 = (pw % ntl) * BM; pk = kc * kchunk; pk_end = min(M, pk + kchunk); }
-        }
-    };
-    if (prod) {
-#pragma unroll 1
-        for (int i = 0; i < STAGES && pmore; ++i) issue();
-    }
-
-    const int r = lane >> 2, j = lane & 3;
-    const int wl0 = (warp / WN) * (MT * 8), wn0 = (warp % WN) * (NT * 8);
-    const int chi = (r >> 1) & 1;
-    const uint32_t rowoff = j * 128 + ((r & 1) << 3) + (r >> 2) * BOX;
-
-    uint32_t it = 0;
-    for (int w = blockIdx.x; w < nwork; w += gridDim.x) {
-        const int kc = w / ntl, l0 = (w % ntl) * BM;
-        const int k_begin = kc * kchunk, k_end = min(M, k_begin + kchunk);
-        double acc[MT][NT][2];
-#pragma unroll
-        for (int a = 0; a < MT; ++a)
-#pragma unroll
-            for (int b = 0; b < NT; ++b) { acc[a][b][0] = 0.0; acc[a][b][1] = 0.0; }
-
-        for (int k = k_begin; k < k_end; k += BK, ++it) {
-            // refill the stage consumed LAG iterations ago (k-block it - LAG + STAGES)
-            if (prod && it >= (uint32_t)LAG && pmore) issue();
-            const uint32_t s = it % STAGES, ph = (it / STAGES) & 1;
-            mbar_wait(full0 + 8 * s, ph);
-            const uint32_t ys = base + s * SB + (wl0 / 16) * BOX + rowoff;
-            const uint32_t as = base + s * SB + YB + (wn0 / 16) * BOX + rowoff;
-#pragma unroll
-            for (int sp = 0; sp < 4; ++sp) {
-                double af[MT], bf[NT];
-                const uint32_t hi = (uint32_t)((chi ^ (sp & 1)) << 6) + sp * 512;
-#pragma unroll
-                for (int a = 0; a < MT; ++a) af[a] = lds64(ys + (a >> 2) * (2 * BOX) + hi + (((a & 3) ^ j) << 4));
-#pragma unroll
-                for (int b = 0; b < NT; ++b) bf[b] = lds64(as + (b >> 2) * (2 * BOX) + hi + (((b & 3) ^ j) << 4));
-#pragma unroll
-                for (int a = 0; a < MT; ++a)
-#pragma unroll
-                    for (int b = 0; b < NT; ++b) dmma(acc[a][b], af[a], bf[b]);
-            }
-            consumer_release(empty0 + 8 * s, lane);
-        }
-        double* slab = Qpart + (size_t)kc * H * ldQ;
-#pragma unroll
-        for (int a = 0; a < MT; ++a) {
-            const int l = l0 + wl0 + 32 * (a >> 2) + perm32(r, a & 3);
-            if (l < L) {
-#pragma unroll
-                for (int b = 0; b < NT; ++b) {
-#pragma unroll
-                    for (int i = 0; i < 2; ++i) {
-                        const int h = wn0 + 32 * (b >> 2) + perm32(2 * j + i, b & 3);
-                        if (h < H) slab[(size_t)h * ldQ + l] = acc[a][b][i];
-                    }
-                }
-            }
-        }
-    }
-}
-
-// ------------------------------------------------------------------------------------------- K2, stream-K decomposition
-// The classic split-K above gives every (128-row tile, K chunk) pair its own slab: at L = 20000 (157 tiles on 148 SMs) the
-// planner needs S = 16 chunks for an even last wave, i.e. 16 slabs of L x H written by K2 and read back by the reduction
-// (164 MB per iteration at H = 64, a visible part of the replicated tail on 8 GPUs).  Stream-K instead cuts the linear
-// sequence of U = ntl * nk work units (tile-major, unit = one tile x kq columns of Y) into one contiguous range per CTA:
-// consecutive units of the same tile accumulate in registers, a CTA writes one partial tile per tile it touches (at most
-// three), and a tile is completed by summing at most Smax (= 2 when a CTA's range spans more than a tile) partials in fixed
-// CTA order.  Load balance is within ONE unit (kq columns) instead of one wave; the decomposition depends only on
-// (L, M, grid), so results stay bit-reproducible.
-struct StreamKPlan { int ntl, nk, kq, grid, smax; };
-// CTA that owns unit u when CTA b owns [b*U/G, (b+1)*U/G):  b(u) = floor(((u + 1)*G - 1) / U)
-__host__ __device__ inline int sk_owner(long long u, long long U, int G) { return (int)(((u + 1) * G - 1) / U); }
-
-template <int BN>
-__global__ void __launch_bounds__((Cfg<BN>::WM * Cfg<BN>::WN + 1) * 32, Cfg<BN>::CPS)
-gemm_ya_sk_kernel(const __grid_constant__ CUtensorMap tmY, const __grid_constant__ CUtensorMap tmA,
-                  double* __restrict__ Qpart, int L, int M, int H, int ldQ, int kq, int nk, int ntl,
-                  const Scalars* __restrict__ sc) {
-    if (sc != nullptr && !sc->active) return;
-    constexpr int WM = Cfg<BN>::WM, WN = Cfg<BN>::WN, STAGES = Cfg<BN>::STAGES;
-    constexpr int NCW = WM * WN;
-    constexpr int MT = BM / WM / 8, NT = BN / WN / 8;
-    static_assert(MT % 4 == 0 && NT % 4 == 0, "K2 needs 32-wide warp tiles");
-    constexpr int YB = BM * BK * 8, SB = Sizes<BN>::STAGE;
-
-    extern __shared__ uint8_t smem_raw[];
-    const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-    const uint32_t full0 = base + STAGES * SB, empty0 = full0 + STAGES * 8;
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    if (threadIdx.x == 0) {
-        for (int s = 0; s < STAGES; ++s) { mbar_init(full0 + 8 * s, 1); mbar_init(empty0 + 8 * s, NCW); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    }
-    __syncthreads();
-
-    const long long U = (long long)ntl * nk;
-    const int u0 = (int)((blockIdx.x * U) / gridDim.x), u1 = (int)(((blockIdx.x + 1) * U) / gridDim.x);
-
-    if (warp == NCW) {  // ---------------- producer
-        if (lane == 0) {
-            uint32_t it = 0;
-            for (int u = u0; u < u1; ++u) {
-                const int lt = u / nk, kcn = u - lt * nk, l0 = lt * BM;
-                const int k_begin = kcn * kq, k_end = min(M, k_begin + kq);
-                for (int k = k_begin; k < k_end; k += BK, ++it) {
-                    const uint32_t s = it % STAGES, ph = (it / STAGES) & 1;
-                    mbar_wait(empty0 + 8 * s, ph ^ 1);
-                    mbar_expect_tx(full0 + 8 * s, SB);
-                    const uint32_t dst = base + s * SB;
-#pragma unroll
-                    for (int b = 0; b < BM / 16; ++b) tma_load_2d(dst + b * BOX, &tmY, full0 + 8 * s, l0 + 16 * b, k);
-#pragma unroll
-                    for (int b = 0; b < BN / 16; ++b) tma_load_2d(dst + YB + b * BOX, &tmA, full0 + 8 * s, 16 * b, k);
-                }
-            }
-        }
-        return;
-    }
-    // ---------------- consumers
-    const int r = lane >> 2, j = lane & 3;
-    const int wl0 = (warp / WN) * (MT * 8), wn0 = (warp % WN) * (NT * 8);
-    const int chi = (r >> 1) & 1;
-    const uint32_t rowoff = j * 128 + ((r & 1) << 3) + (r >> 2) * BOX;
-
-    double acc[MT][NT][2];
-    int cur = -1;
-    // one partial tile: slot = position of this CTA among the CTAs that touch the tile (fixed summation order later)
-    auto flush = [&](int lt) {
-        const int slot = (int)blockIdx.x - sk_owner((long long)lt * nk, U, gridDim.x);
-        double* slab = Qpart + (size_t)slot * H * ldQ;
-        const int l0 = lt * BM;
-#pragma unroll
-        for (int a = 0; a < MT; ++a) {
-            const int l = l0 + wl0 + 32 * (a >> 2) + perm32(r, a & 3);
-            if (l < L) {
-#pragma unroll
-                for (int b = 0; b < NT; ++b) {
-#pragma unroll
-                    for (int i = 0; i < 2; ++i) {
-                        const int h = wn0 + 32 * (b >> 2) + perm32(2 * j + i, b & 3);
-                        if (h < H) slab[(size_t)h * ldQ + l] = acc[a][b][i];
-                    }
-                }
-            }
-        }
-    };
-    uint32_t it = 0;
-    for (int u = u0; u < u1; ++u) {
-        const int lt = u / nk, kcn = u - lt * nk;
-        if (lt != cur) {
-            if (cur >= 0) flush(cur);
-#pragma unroll
-            for (int a = 0; a < MT; ++a)
-#pragma unroll
-                for (int b = 0; b < NT; ++b) { acc[a][b][0] = 0.0; acc[a][b][1] = 0.0; }
-            cur = lt;
-        }
-        const int k_begin = kcn * kq, k_end = min(M, k_begin + kq);
-        for (int k = k_begin; k < k_end; k += BK, ++it) {
-            const uint32_t s = it % STAGES, ph = (it / STAGES) & 1;
-            mbar_wait(full0 + 8 * s, ph);
-            const uint32_t ys = base + s * SB + (wl0 / 16) * BOX + rowoff;
-            const uint32_t as = base + s * SB + YB + (wn0 / 16) * BOX + rowoff;
-#pragma unroll
-            for (int sp = 0; sp < 4; ++sp) {
-                double af[MT], bf[NT];
-                const uint32_t hi = (uint32_t)((chi ^ (sp & 1)) << 6) + sp * 512;
-#pragma unroll
-                for (int a = 0; a < MT; ++a) af[a] = lds64(ys + (a >> 2) * (2 * BOX) + hi + (((a & 3) ^ j) << 4));
-#pragma unroll
-                for (int b = 0; b < NT; ++b) bf[b] = lds64(as + (b >> 2) * (2 * BOX) + hi + (((b & 3) ^ j) << 4));
-#pragma unroll
-                for (int a = 0; a < MT; ++a)
-#pragma unroll
-                    for (int b = 0; b < NT; ++b) dmma(acc[a][b], af[a], bf[b]);
-            }
-            consumer_release(empty0 + 8 * s, lane);
-        }
-    }
-    if (cur >= 0) flush(cur);
-}
-
-// Q[h][l] = sum over the partial tiles of row tile l / 128 in CTA order (fixed): the number of partials of a tile follows
-// from the same ownership formula the kernel used
-__global__ void __launch_bounds__(256) reduce_q_sk_kernel(const double* __restrict__ Qpart, double* __restrict__ Q, int L, int H, int ldQ,
-                                                          int nk, int ntl, int grid, const Scalars* sc) {
-    if (sc != nullptr && !sc->active) return;
-    const long long U = (long long)ntl * nk;
-    const size_t n = (size_t)H * ldQ, slab = n;
-    for (size_t e = (size_t)blockIdx.x * blockDim.x + threadIdx.x; e < n; e += (size_t)gridDim.x * blockDim.x) {
-        const int l = (int)(e % ldQ);
-        double s = 0.0;
-        if (l < L) {
-            const int lt = l / BM;
-            const int b0 = sk_owner((long long)lt * nk, U, grid), b1 = sk_owner((long long)(lt + 1) * nk - 1, U, grid);
-            for (int q = 0; q <= b1 - b0; ++q) s += Qpart[(size_t)q * slab + e];
-        }
-        Q[e] = s;
-    }
-}
-
 // ------------------------------------------------------------------------------------------- host side
 static PFN_encodeTiled g_encode = nullptr;
 
@@ -677,12 +417,6 @@ int gemm_init_device() {
     VB_CUDA_OK(cudaFuncSetAttribute(gemm_ya_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, Sizes<32>::SMEM));
     VB_CUDA_OK(cudaFuncSetAttribute(gemm_ya_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, Sizes<64>::SMEM));
     VB_CUDA_OK(cudaFuncSetAttribute(gemm_ya_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, Sizes<128>::SMEM));
-    VB_CUDA_OK(cudaFuncSetAttribute((gemm_ya_fold_kernel<128, 1>), cudaFuncAttributeMaxDynamicSharedMemorySize, Sizes<128>::SMEM));
-    VB_CUDA_OK(cudaFuncSetAttribute((gemm_ya_fold_kernel<128, 2>), cudaFuncAttributeMaxDynamicSharedMemorySize, Sizes<128>::SMEM));
-    VB_CUDA_OK(cudaFuncSetAttribute((gemm_ya_fold_kernel<128, 3>), cudaFuncAttributeMaxDynamicSharedMemorySize, Sizes<128>::SMEM));
-    VB_CUDA_OK(cudaFuncSetAttribute(gemm_ya_sk_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, Sizes<32>::SMEM));
-    VB_CUDA_OK(cudaFuncSetAttribute(gemm_ya_sk_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, Sizes<64>::SMEM));
-    VB_CUDA_OK(cudaFuncSetAttribute(gemm_ya_sk_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, Sizes<128>::SMEM));
     return gemm_i8_init_device();
 }
 
@@ -713,69 +447,7 @@ int launch_gemm_ya(cudaStream_t st, const CUtensorMap* tmY, const CUtensorMap* t
     if (kchunk % BK != 0) { set_error("split-K chunk %d is not a multiple of %d", kchunk, BK); return -1; }
     if (H <= 32) return launch_ya_t<32>(st, tmY, tmA, Qpart, L, M, H, ldQ, kchunk, S, sc, num_sms);
     if (H <= 64) return launch_ya_t<64>(st, tmY, tmA, Qpart, L, M, H, ldQ, kchunk, S, sc, num_sms);
-    static const int fold = getenv("VBMF_B200_K2_FOLD") ? atoi(getenv("VBMF_B200_K2_FOLD")) : 0;
-    if (fold > 0) {
-        const int ntl = (L + BM - 1) / BM;
-        const int grid = std::max(1, std::min(ntl * S, num_sms * Cfg<128>::CPS));
-        const int threads = Cfg<128>::WM * Cfg<128>::WN * 32;
-        if (fold == 1) gemm_ya_fold_kernel<128, 1><<<grid, threads, Sizes<128>::SMEM, st>>>(*tmY, *tmA, Qpart, L, M, H, ldQ, kchunk, S, sc);
-        else if (fold == 3) gemm_ya_fold_kernel<128, 3><<<grid, threads, Sizes<128>::SMEM, st>>>(*tmY, *tmA, Qpart, L, M, H, ldQ, kchunk, S, sc);
-        else gemm_ya_fold_kernel<128, 2><<<grid, threads, Sizes<128>::SMEM, st>>>(*tmY, *tmA, Qpart, L, M, H, ldQ, kchunk, S, sc);
-        VB_LAUNCH_OK();
-        return 0;
-    }
     return launch_ya_t<128>(st, tmY, tmA, Qpart, L, M, H, ldQ, kchunk, S, sc, num_sms);
-}
-
-// stream-K plan: unit length kq (columns of Y per unit), units per tile nk, grid, worst-case partials per tile
-int plan_streamk(int L, int M, int H, int num_sms, int* kq_out, int* nk_out, int* grid_out, int* smax_out) {
-    const GemmGeometry g = gemm_geometry(H);
-    const long ntl = (L + BM - 1) / BM;
-    // unit length = granularity of the CTA boundaries: ~1/32 of the K extent (balance within ~1 % of a CTA's range), at least
-    // 4 and at most 128 k-blocks -- short units cost a tile-change test and an integer division every few k-blocks
-    // (kq = 64 measured 7 % slower than the classic split on K2)
-    int kq = (int)std::min<long>(2048, std::max<long>(64, (((long)M / 32 + 63) / 64) * 64));
-    while (((long)M + kq - 1) / kq * ntl > 0x7fffff00L) kq *= 2;
-    const long nk = std::max<long>(1, ((long)M + kq - 1) / kq);
-    const long U = ntl * nk;
-    const long G = std::max<long>(1, std::min<long>(U, (long)num_sms * g.ctas_per_sm));
-    const long per = std::max<long>(1, U / G);              // smallest range of a CTA
-    *kq_out = kq; *nk_out = (int)nk; *grid_out = (int)G;
-    *smax_out = (int)((nk + per - 1) / per + 1);
-    return 0;
-}
-
-template <int BN>
-static int launch_ya_sk_t(cudaStream_t st, const CUtensorMap* tmY, const CUtensorMap* tmA, double* Qpart, int L, int M, int H,
-                          int ldQ, int kq, int nk, int grid, const Scalars* sc) {
-    const int ntl = (L + BM - 1) / BM;
-    const int threads = (Cfg<BN>::WM * Cfg<BN>::WN + 1) * 32;
-    gemm_ya_sk_kernel<BN><<<grid, threads, Sizes<BN>::SMEM, st>>>(*tmY, *tmA, Qpart, L, M, H, ldQ, kq, nk, ntl, sc);
-    VB_LAUNCH_OK();
-    return 0;
-}
-int launch_gemm_ya_sk(cudaStream_t st, const CUtensorMap* tmY, const CUtensorMap* tmA, double* Qpart, double* Q, int L, int M, int H,
-                      int ldQ, int kq, int nk, int grid, const Scalars* sc) {
-    if (H > 128) { set_error("H = %d > 128 is not supported by the K2 kernel yet", H); return -1; }
-    if (L <= 0 || H <= 0) return 0;
-    int rc = 0;
-    if (M > 0) {
-        if (H <= 32) rc = launch_ya_sk_t<32>(st, tmY, tmA, Qpart, L, M, H, ldQ, kq, nk, grid, sc);
-        else if (H <= 64) rc = launch_ya_sk_t<64>(st, tmY, tmA, Qpart, L, M, H, ldQ, kq, nk, grid, sc);
-        else rc = launch_ya_sk_t<128>(st, tmY, tmA, Qpart, L, M, H, ldQ, kq, nk, grid, sc);
-        if (rc) return rc;
-    }
-    return 0;
-}
-int launch_reduce_q_sk(cudaStream_t st, const double* Qpart, double* Q, int L, int M, int H, int ldQ, int nk, int grid, const Scalars* sc) {
-    const int ntl = (L + BM - 1) / BM;
-    const size_t n = (size_t)H * ldQ;
-    if (n == 0) return 0;
-    if (M <= 0) { VB_CUDA_OK(cudaMemsetAsync(Q, 0, n * 8, st)); return 0; }
-    const int blocks = (int)std::max<size_t>(1, std::min<size_t>((n + 255) / 256, 1184));
-    reduce_q_sk_kernel<<<blocks, 256, 0, st>>>(Qpart, Q, L, H, ldQ, nk, ntl, grid, sc);
-    VB_LAUNCH_OK();
-    return 0;
 }
 
 // ------------------------------------------------------------------------------------------- SIMT cross-check kernels

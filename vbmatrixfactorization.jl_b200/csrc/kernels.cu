@@ -403,87 +403,8 @@ int k_gram_w2(cudaStream_t st, const Dev& d, const double* X, int n, const doubl
 // mode 1: SigmaB = sigma2*inv(A'A + M*SigmaA + sigma2*invCB)            src/vbmf.jl:110-111
 // mode 2: SigmaA <- all-reduced sum of per-column blocks; SigmaB = inv(diag(CB) + c*(A'A + SigmaA)),
 //         c = sigmaHat or mean(sigmaVecHat)                             src/vbmf_sparse.jl:256-265, src/vbmf_dual.jl:294-303
-template <int HP2>   // H rounded up to a power of two (32, 64, 128); thread t owns column t % HP2, rows t / HP2 + q * (1024 / HP2)
-__global__ void __launch_bounds__(1024, 1) hxh_kernel(Dev d, int mode, int diag_var) {
-    ACTIVE_OR_RETURN(d);
-    __shared__ double cbuf[2 * 128], sbuf[128], idb[2];
-    constexpr int Q = HP2 * HP2 / 1024, RP = 1024 / HP2;
-    const int H = d.H;
-    Scalars* sc = d.sc;
-    const double* AtA = d.packed + packed_ata(d);
-    const double* SA = d.packed + packed_sa(d);
-    const int j = threadIdx.x % HP2, i0 = threadIdx.x / HP2;
-    double a[Q];
-#pragma unroll
-    for (int q = 0; q < Q; ++q) {
-        const int i = i0 + q * RP;
-        double v = (i == j) ? 1.0 : 0.0;               // padding: identity
-        if (i < H && j < H) {
-            const int e = i * H + j;
-            if (mode == 0) v = d.BtB[e] + (double)d.L * d.SigmaB[e] + sc->sigma2 * d.invCA[e];
-            else if (mode == 1) v = AtA[e] + (double)d.Mglob * d.SigmaA[e] + sc->sigma2 * d.invCB[e];
-            else {
-                const double sa = SA[e];
-                d.SigmaA[e] = sa;
-                const double c = diag_var ? sc->meanSigmaVec : sc->sigmaHat;
-                v = ((i == j) ? d.CBv[i] : 0.0) + c * (AtA[e] + sa);
-            }
-        }
-        a[q] = v;
-    }
-    // equilibrated symmetric Gauss-Jordan, matrix in registers, column k through a double-buffered shared vector
-    bool ok = true;
-    const bool live = j < H;
-#pragma unroll
-    for (int q = 0; q < Q; ++q) if (live && i0 + q * RP == j) sbuf[j] = 1.0 / sqrt(a[q]);
-    __syncthreads();
-    const double sj = live ? sbuf[j] : 1.0;
-#pragma unroll
-    for (int q = 0; q < Q; ++q) { const int i = i0 + q * RP; if (live && i < H) a[q] *= sbuf[i] * sj; }
-    // One barrier per sweep: the owners of column k+1 publish it (and the owner of the next pivot its reciprocal, so the
-    // other 1023 threads do not each pay for a double-precision division) right after their own update of sweep k.
-    // Per element one FMA: a + col[i]*beta with beta = -col[j]/d, and beta = 1/d - 1 in the pivot column (a == col[i] there).
-    if (j == 0) {
-#pragma unroll
-        for (int q = 0; q < Q; ++q) { const int i = i0 + q * RP; if (i < H) cbuf[i] = a[q]; }
-        if (i0 == 0) idb[0] = 1.0 / a[0];
-    }
-    __syncthreads();
-    for (int k = 0; k < H; ++k) {
-        const double* col = cbuf + (k & 1) * 128;
-        double* coln = cbuf + ((k + 1) & 1) * 128;
-        const double dk = col[k];
-        if (!(dk > 0.0) || !(dk < 1e300)) ok = false;
-        const double id = idb[k & 1];
-        const double t = (live ? col[j] : 0.0) * id;
-        const bool pc = j == k;
-        const double beta = pc ? id - 1.0 : -t, rowv = pc ? -id : t;
-#pragma unroll
-        for (int q = 0; q < Q; ++q) {
-            const int i = i0 + q * RP;
-            if (live && i < H) {
-                const double v = (i == k) ? rowv : fma(col[i], beta, a[q]);
-                a[q] = v;
-                if (j == k + 1) {
-                    coln[i] = v;
-                    if (i == k + 1) idb[(k + 1) & 1] = 1.0 / v;
-                }
-            }
-        }
-        __syncthreads();
-    }
-    if (!ok && threadIdx.x == 0) sc->chol_fail = 1;
-    double* out = (mode == 0) ? d.SigmaA : d.SigmaB;
-    const double scale = (mode == 2) ? 1.0 : sc->sigma2;
-#pragma unroll
-    for (int q = 0; q < Q; ++q) {
-        const int i = i0 + q * RP;
-        if (live && i < H) out[i * H + j] = ok ? scale * (-a[q] * sbuf[i] * sj) : nan("");
-    }
-}
-// Tensor-core versions of the same three inverses (blocked rank-4 Gauss-Jordan, see linalg.cuh::warp_block_gj_sym): the
-// register sweep above pays one CTA barrier per pivot (58 us at H = 64, 400 us at H = 128, all of it on the critical path of
-// every iteration and replicated on every GPU); here a step handles four pivots with one barrier and one DMMA per tile.
+// Blocked rank-4 Gauss-Jordan on the tensor cores (linalg.cuh::warp_block_gj_sym): a step handles four pivots with one
+// barrier and one DMMA per tile.  These inverses sit on the critical path of every iteration, replicated on every GPU.
 __device__ __forceinline__ double hxh_elem(const Dev& d, int mode, int diag_var, int i, int j) {
     const Scalars* sc = d.sc;
     const int e = i * d.H + j;
@@ -492,7 +413,7 @@ __device__ __forceinline__ double hxh_elem(const Dev& d, int mode, int diag_var,
     const double c = diag_var ? sc->meanSigmaVec : sc->sigmaHat;
     return ((i == j) ? d.CBv[i] : 0.0) + c * ((d.packed + packed_ata(d))[e] + (d.packed + packed_sa(d))[e]);
 }
-// H <= 32: one warp, upper-triangular tiles
+// H <= 8: one warp, upper-triangular tiles
 template <int NT>
 __global__ void __launch_bounds__(32, 1) hxh_warp_kernel(Dev d, int mode, int diag_var) {
     ACTIVE_OR_RETURN(d);
@@ -533,11 +454,11 @@ __global__ void __launch_bounds__(32, 1) hxh_warp_kernel(Dev d, int mode, int di
                 }
             }
 }
-// 32 < H <= 128: 16 warps, the full NTD x NTD tile grid spread over the warps (warp w: tile row w / WPR, TPW tile columns).
+// 8 < H <= 128: 16 warps, the full NTD x NTD tile grid spread over the warps (warp w: tile row w / WPR, TPW tile columns).
 // Per block step: the owners of the pivot column block publish the panel (double buffered); the first N/32 warps run the
 // four sweeps with lane = row (linalg.cuh::gj_panel_sweeps, the 4 x 4 pivot block evolved in every lane) and leave the
 // multipliers G and the pre-sweep columns Q in shared memory; every warp then reads its A / B fragments and issues TPW DMMAs.
-// Two barriers per FOUR pivots (the register sweep: one per pivot, with 1024 threads).
+// Two barriers per four pivots.
 template <int NTD, int TPW>
 __global__ void __launch_bounds__(512, 1) hxh_dmma_kernel(Dev d, int mode, int diag_var) {
     ACTIVE_OR_RETURN(d);
@@ -614,25 +535,11 @@ __global__ void __launch_bounds__(512, 1) hxh_dmma_kernel(Dev d, int mode, int d
         }
 }
 static int hxh_launch(cudaStream_t st, const Dev& d, int mode, int dv) {
-    static const bool use_reg = getenv("VBMF_B200_HXH") != nullptr && strcmp(getenv("VBMF_B200_HXH"), "reg") == 0;
-    if (!use_reg) {
-        const int H = d.H;
-        static const bool one_warp = getenv("VBMF_B200_HXH") != nullptr && strcmp(getenv("VBMF_B200_HXH"), "warp") == 0;
-        if (H <= 8) hxh_warp_kernel<1><<<1, 32, 0, st>>>(d, mode, dv);
-        else if (H <= 32 && !one_warp) hxh_dmma_kernel<4, 1><<<1, 512, 0, st>>>(d, mode, dv);   // 16 warps, one tile each: 26 -> ~10 us at H = 32
-        else if (H <= 16) hxh_warp_kernel<2><<<1, 32, 0, st>>>(d, mode, dv);
-        else if (H <= 24) hxh_warp_kernel<3><<<1, 32, 0, st>>>(d, mode, dv);
-        else if (H <= 32) hxh_warp_kernel<4><<<1, 32, 0, st>>>(d, mode, dv);
-        else if (H <= 64) hxh_dmma_kernel<8, 4><<<1, 512, 0, st>>>(d, mode, dv);
-        else hxh_dmma_kernel<16, 16><<<1, 512, 0, st>>>(d, mode, dv);
-        VB_LAUNCH_OK();
-        return 0;
-    }
-    const int hh = d.H * d.H;
-    // 1024 threads beat 512 / 256 (46 vs 62 vs ~100 us at H = 64): the sweep is latency bound, more warps hide it
-    if (hh <= 1024) hxh_kernel<32><<<1, 1024, 0, st>>>(d, mode, dv);
-    else if (hh <= 4096) hxh_kernel<64><<<1, 1024, 0, st>>>(d, mode, dv);
-    else hxh_kernel<128><<<1, 1024, 0, st>>>(d, mode, dv);
+    const int H = d.H;
+    if (H <= 8) hxh_warp_kernel<1><<<1, 32, 0, st>>>(d, mode, dv);
+    else if (H <= 32) hxh_dmma_kernel<4, 1><<<1, 512, 0, st>>>(d, mode, dv);   // 16 warps, one tile each: 26 -> ~10 us at H = 32
+    else if (H <= 64) hxh_dmma_kernel<8, 4><<<1, 512, 0, st>>>(d, mode, dv);
+    else hxh_dmma_kernel<16, 16><<<1, 512, 0, st>>>(d, mode, dv);
     VB_LAUNCH_OK();
     return 0;
 }
@@ -1152,82 +1059,13 @@ __global__ void __launch_bounds__(256) sparse_A_full_kernel(Dev d, int diag_var,
         if (e < H * H) out[e] = acc[q];
     }
 }
-// H <= 32: one warp per matrix, the matrix lives in registers (lane l owns column l), see warp_spd_inverse_reg.
-// G and the warps' running sums of Sigma_m live in shared memory so the kernel fits 128 registers and two CTAs (16 warps)
-// share an SM: the sweeps are latency bound and need the extra warps.
-template <int HP>
-__global__ void __launch_bounds__(256, 2) sparse_A_full_warp_kernel(Dev d, int diag_var, int nwarps_total) {
-    ACTIVE_OR_RETURN(d);
-    extern __shared__ __align__(16) double wsm[];
-    double* s_G = wsm;                       // [HP][32]  G[q][lane], zero padded
-    double* s_col = s_G + HP * 32;           // [8][64]
-    double* s_p = s_col + 8 * 64;            // [8][32]
-    double* s_accw = s_p + 8 * 32;           // [8][HP][32]
-    const int H = d.H;
-    const Scalars* sc = d.sc;
-    const int lane = threadIdx.x & 31, wic = threadIdx.x >> 5;
-    const int gw = blockIdx.x * (blockDim.x >> 5) + wic;
-    double* col = s_col + wic * 64;
-    double* pv = s_p + wic * 32;
-    double* acc = s_accw + wic * HP * 32;
-    const double sh = sc->sigmaHat;
-    const bool live = lane < H;
-    for (int e = threadIdx.x; e < HP * 32; e += blockDim.x) {
-        const int q = e >> 5, l = e & 31;
-        s_G[e] = (q < H && l < H) ? d.Gm[q * H + l] : 0.0;
-    }
-#pragma unroll
-    for (int q = 0; q < HP; ++q) acc[q * 32 + lane] = 0.0;
-    __syncthreads();
-    const double gll = s_G[min(lane, HP - 1) * 32 + lane];
-    bool all_ok = true;
-    for (int m = gw; m < d.Mloc; m += nwarps_total) {
-        const double ca = live ? d.CAv[(size_t)m * H + lane] : 1.0;     // padded lanes: identity
-        const double p = live ? d.P[(size_t)m * H + lane] : 0.0;
-        double a[HP];
-#pragma unroll
-        for (int q = 0; q < HP; ++q) a[q] = s_G[q * 32 + lane] + ((q == lane) ? ca : 0.0);
-        pv[lane] = p;
-        const bool ok = warp_spd_inverse_reg<HP>(a, gll + ca, lane, col);      // ends with __syncwarp (pv visible)
-        all_ok = all_ok && ok;
-        double s = 0.0, dg = 0.0;
-#pragma unroll
-        for (int q = 0; q < HP; ++q) {
-            const double pq = pv[q];
-            s = diag_var ? fma(a[q], pq, s) : fma(sh * a[q], pq, s);     // row `lane` of Sigma_m (symmetric) times p
-            if (q == lane) dg = a[q];
-        }
-        if (live) {
-            d.A[(size_t)m * H + lane] = ok ? s : nan("");
-            d.sdiag[(size_t)m * H + lane] = ok ? dg : nan("");
-            if (d.blocks != nullptr) {
-#pragma unroll
-                for (int q = 0; q < HP; ++q) if (q < H) d.blocks[(size_t)m * H * H + q * H + lane] = a[q];
-            }
-        }
-#pragma unroll
-        for (int q = 0; q < HP; ++q) acc[q * 32 + lane] += a[q];
-        __syncwarp();
-    }
-    if (!all_ok && lane == 0) d.sc->chol_fail = 1;
-    __syncthreads();
-    // per-CTA sum of the warps' accumulators in fixed warp order (one partial per CTA instead of one per warp)
-    double* out = d.part + (size_t)blockIdx.x * H * H;
-    for (int e = threadIdx.x; e < H * H; e += blockDim.x) {
-        const int q = e / H, l = e - q * H;
-        double t = 0.0;
-        for (int w = 0; w < (int)(blockDim.x >> 5); ++w) t += s_accw[(w * HP + q) * 32 + l];
-        out[e] = t;
-    }
-}
-// H <= 32, tensor-core version: one warp per matrix, upper-triangular 8 x 8 tiles in DMMA accumulator registers, blocked
+// H <= 32: one warp per matrix, upper-triangular 8 x 8 tiles in DMMA accumulator registers, blocked
 // rank-4 Gauss-Jordan (linalg.cuh::warp_block_gj_sym).  The right-hand side p_m rides through the sweeps.  The running sum
 // of Sigma_m (tiles on and above the diagonal only) lives in registers (ACCS = false) or in per-warp shared memory
 // (ACCS = true: 40 registers less, one more CTA per SM).  Shared memory: G as accumulator-layout tiles (read once per matrix
 // with conflict-free 128-bit loads), 2.5 KB of scratch per warp.
 template <int NT, int MINB, bool ACCS>
-__global__ void __launch_bounds__(128, MINB) sparse_A_full_dmma_kernel(Dev d, int diag_var, int nwarps_total, const double* __restrict__ slabs,
-                                                                        int S, size_t slab_stride, int fuse_ca) {
+__global__ void __launch_bounds__(128, MINB) sparse_A_full_dmma_kernel(Dev d, int diag_var, int nwarps_total) {
     ACTIVE_OR_RETURN(d);
     constexpr int NTRI = NT * (NT + 1) / 2, WPC = 4, SCR = GJ_SCRATCH + 64;
     extern __shared__ __align__(16) double wsm[];
@@ -1264,17 +1102,13 @@ __global__ void __launch_bounds__(128, MINB) sparse_A_full_dmma_kernel(Dev d, in
     __syncthreads();
     bool all_ok = true;
     for (int m = gw; m < d.Mloc; m += nwarps_total) {
-        // inputs of column m: CA_m (padded rows / columns: identity) and (Y'B)[m, :] = fixed-order sum of the K1 split-K slabs.
+        // inputs of column m: CA_m (padded rows / columns: identity) and (Y'B)[m, :].
         // (Fetching them one column ahead with cp.async measured 12 % SLOWER, 0.454 vs 0.407 ms: plain loads stay.)
         double ca = 1.0, p = 0.0;
         if (live) {
             const size_t idx = (size_t)m * H + lane;
             ca = d.CAv[idx];
-            const double p0 = slabs[idx], p1 = S > 1 ? slabs[slab_stride + idx] : 0.0, p2 = S > 2 ? slabs[2 * slab_stride + idx] : 0.0;
-            p = p0;
-            if (S > 1) p += p1;
-            if (S > 2) p += p2;
-            for (int s2 = 3; s2 < S; ++s2) p += slabs[(size_t)s2 * slab_stride + idx];
+            p = d.P[idx];
         }
         const double sl = rsqrt(gll + ca);
         sv[lane] = sl;
@@ -1301,8 +1135,7 @@ __global__ void __launch_bounds__(128, MINB) sparse_A_full_dmma_kernel(Dev d, in
         double v = p * sl;
         const bool ok = warp_block_gj_sym<NT>(c, v, lane, scr);
         all_ok = all_ok && ok;
-        double aval = ok ? (diag_var ? sl * v : (sh * sl) * v) : nan("");
-        if (fuse_ca && d.rowmask != nullptr && lane >= H - d.H1 && d.rowmask[m]) aval = 0.0;       // label mask (src/vbmf_sparse.jl:245)
+        const double aval = ok ? (diag_var ? sl * v : (sh * sl) * v) : nan("");
         if (live) d.A[(size_t)m * H + lane] = aval;
         // Sigma_m = D*c*D: un-equilibrate (the scale vector is re-read: holding it across the sweeps costs 24 registers) fused
         // with the running sum; the diagonal (and the blocks on request) are emitted separately
@@ -1328,7 +1161,6 @@ __global__ void __launch_bounds__(128, MINB) sparse_A_full_dmma_kernel(Dev d, in
                 if (ti == tj && j == (r >> 1)) {
                     const double sd = ok ? ((r & 1) ? c[t][1] * w1 : c[t][0] * w0) : nan("");
                     if (row < H) d.sdiag[(size_t)m * H + row] = sd;
-                    if (fuse_ca) cav[row] = sd;
                 }
                 if (d.blocks != nullptr && row < H) {
                     double* blk = d.blocks + (size_t)m * H * H;
@@ -1337,14 +1169,6 @@ __global__ void __launch_bounds__(128, MINB) sparse_A_full_dmma_kernel(Dev d, in
                     if (col + 1 < H) { blk[row * H + col + 1] = s1; if (ti != tj) blk[(col + 1) * H + row] = s1; }
                 }
             }
-        __syncwarp();
-        if (fuse_ca && live) {
-            // updateCA! of the sparse kind for this column (src/vbmf_sparse.jl:284-288): it only needs a, diag(Sigma_m) and
-            // replicated scalars, so doing it here saves one pass over vec(A')
-            const double beta = sc->beta0p + 0.5 * (aval * aval + cav[lane]);
-            d.beta[(size_t)m * H + lane] = beta;
-            d.CAv[(size_t)m * H + lane] = sc->alpha / beta;
-        }
         __syncwarp();
     }
     if (!all_ok && lane == 0) d.sc->chol_fail = 1;
@@ -1368,46 +1192,23 @@ __global__ void __launch_bounds__(128, MINB) sparse_A_full_dmma_kernel(Dev d, in
 }
 template <int NT> static size_t k4_dmma_smem() { return (size_t)(NT * (NT + 1) / 2 * 64 + 4 * (GJ_SCRATCH + 64) + 4 * (NT * (NT + 1) / 2) * 64) * sizeof(double); }
 
-static bool k4_use_reg() {
-    static const bool v = getenv("VBMF_B200_K4") != nullptr && strcmp(getenv("VBMF_B200_K4"), "reg") == 0;
-    return v;
-}
-bool k_sparse_A_full_can_fuse(const Dev& d) { return d.H <= 32 && !k4_use_reg(); }
-int k_sparse_A_full(cudaStream_t st, const Dev& d, int flags) { return k_sparse_A_full_ex(st, d, flags, d.P, 1, 0, 0); }
-// slabs / S / slab_stride: the K1 output (S split-K slabs or the single P buffer); fuse_ca: also do updateCA! of the sparse kind
-// (tensor-core path, H <= 32, only; the caller checks *did_ca)
-int k_sparse_A_full_ex(cudaStream_t st, const Dev& d, int flags, const double* slabs, int S, size_t slab_stride, int fuse_ca) {
+int k_sparse_A_full(cudaStream_t st, const Dev& d, int flags) {
     const int H = d.H;
     const int dv = (flags & F_DIAG_VAR) ? 1 : 0;
     build_G_kernel<<<1, 256, 0, st>>>(d, dv);
     VB_LAUNCH_OK();
     int ngroups;
-    const bool use_reg = k4_use_reg();
-    if ((S > 1 || fuse_ca) && !k_sparse_A_full_can_fuse(d)) { set_error("k_sparse_A_full_ex: slab / updateCA fusion needs the tensor-core path"); return -1; }
-    if (H <= 32 && !use_reg) {
-        static const int minb = getenv("VBMF_B200_K4_MINB") ? atoi(getenv("VBMF_B200_K4_MINB")) : 4;     // tuning probe: 2, 3 (sums in registers), 4 / 5 (sums in shared memory; 4 CTAs per SM measured fastest: 0.407 vs 0.435 ms for 1e5 32 x 32)
+    if (H <= 32) {
+        // CTAs per SM = the instantiation's MINB.  H > 24 keeps the running sums in shared memory for 4 CTAs per SM (measured
+        // fastest: 0.407 vs 0.435 ms for 1e5 32 x 32 with 3 CTAs and the sums in registers)
         const int wpc = 4;
-        const int per_sm = (H <= 16) ? 4 : (H <= 24 ? 3 : (minb == 5 ? 3 : minb));
+        const int per_sm = (H > 16 && H <= 24) ? 3 : 4;
         const int grid = std::max(1, std::min(cdiv(std::max(d.Mloc, 1), wpc), 148 * per_sm));
         ngroups = grid;                                   // one partial per CTA
-        if (H <= 8) sparse_A_full_dmma_kernel<1, 4, false><<<grid, 128, k4_dmma_smem<1>(), st>>>(d, dv, grid * wpc, slabs, S, slab_stride, fuse_ca);
-        else if (H <= 16) sparse_A_full_dmma_kernel<2, 4, false><<<grid, 128, k4_dmma_smem<2>(), st>>>(d, dv, grid * wpc, slabs, S, slab_stride, fuse_ca);
-        else if (H <= 24) sparse_A_full_dmma_kernel<3, 3, false><<<grid, 128, k4_dmma_smem<3>(), st>>>(d, dv, grid * wpc, slabs, S, slab_stride, fuse_ca);
-        else if (minb == 2) sparse_A_full_dmma_kernel<4, 2, false><<<grid, 128, k4_dmma_smem<4>(), st>>>(d, dv, grid * wpc, slabs, S, slab_stride, fuse_ca);
-        else if (minb == 4) sparse_A_full_dmma_kernel<4, 4, true><<<grid, 128, k4_dmma_smem<4>(), st>>>(d, dv, grid * wpc, slabs, S, slab_stride, fuse_ca);
-        else if (minb == 5) sparse_A_full_dmma_kernel<4, 3, true><<<std::max(1, std::min(cdiv(std::max(d.Mloc, 1), wpc), 148 * 3)), 128, k4_dmma_smem<4>(), st>>>(d, dv, std::max(1, std::min(cdiv(std::max(d.Mloc, 1), wpc), 148 * 3)) * wpc, slabs, S, slab_stride, fuse_ca);
-        else sparse_A_full_dmma_kernel<4, 3, false><<<grid, 128, k4_dmma_smem<4>(), st>>>(d, dv, grid * wpc, slabs, S, slab_stride, fuse_ca);
-    } else if (H <= 32) {
-        const int wpc = 8;
-        const int grid = std::max(1, std::min(cdiv(std::max(d.Mloc, 1), wpc), 296));
-        ngroups = grid;                                   // one partial per CTA
-#define WK(HPV)                                                                                                          \
-    {                                                                                                                    \
-        const size_t smem = (size_t)(HPV * 32 + 8 * 64 + 8 * 32 + 8 * HPV * 32) * sizeof(double);                        \
-        sparse_A_full_warp_kernel<HPV><<<grid, 256, smem, st>>>(d, dv, grid * wpc);                                      \
-    }
-        if (H <= 8) WK(8) else if (H <= 16) WK(16) else if (H <= 24) WK(24) else WK(32)
-#undef WK
+        if (H <= 8) sparse_A_full_dmma_kernel<1, 4, false><<<grid, 128, k4_dmma_smem<1>(), st>>>(d, dv, grid * wpc);
+        else if (H <= 16) sparse_A_full_dmma_kernel<2, 4, false><<<grid, 128, k4_dmma_smem<2>(), st>>>(d, dv, grid * wpc);
+        else if (H <= 24) sparse_A_full_dmma_kernel<3, 3, false><<<grid, 128, k4_dmma_smem<3>(), st>>>(d, dv, grid * wpc);
+        else sparse_A_full_dmma_kernel<4, 4, true><<<grid, 128, k4_dmma_smem<4>(), st>>>(d, dv, grid * wpc);
     } else {
         const size_t smem = (size_t)(H * (H + 1) + 3 * H) * sizeof(double);
         const int grid = std::max(1, std::min(std::max(d.Mloc, 1), 148));
@@ -1525,89 +1326,6 @@ __global__ void trbq_kernel(Dev d, int nparts);
 // sparse: BHat = ((sigmaHat*Y)*AHat)*SigmaB                     src/vbmf_sparse.jl:266   (diag_var: diagm(sv)*Y*AHat*SigmaB, :261)
 // Fused with everything that needs the new rows while they sit in shared memory: Bold, D = BHat - Bold and the Grams
 // BHat'BHat, D'D of the convergence test (src/util.jl:27-29) and of updateCB!/updateSigma*!, and tr(BHat'*(Y*AHat)).
-// TD x TD threads, every thread owns an R x R patch of both Grams; TR rows per tile.
-template <int R, int TD, int TR>
-__global__ void __launch_bounds__(TD * TD) B_epilogue_kernel(Dev d, int diag_var) {
-    ACTIVE_OR_RETURN(d);
-    extern __shared__ double sm[];
-    __shared__ double red[32];
-    constexpr int NT = TD * TD;
-    const int H = d.H, ld = H + 1;
-    double* S = sm;                  // [H][ld]   SigmaB
-    double* T = S + H * ld;          // [TR][ld]  scaled Q tile
-    double* Bn = T + TR * ld;        // [TR][ld]  new BHat rows
-    double* Dn = Bn + TR * ld;       // [TR][ld]  BHat - Bold
-    const Scalars* sc = d.sc;
-    const double* Q = d.packed + packed_q(d);
-    for (int e = threadIdx.x; e < H * H; e += NT) S[(e / H) * ld + (e % H)] = d.SigmaB[e];
-    const bool dense = d.kind == KIND_DENSE;
-    const double s2 = sc->sigma2, sh = sc->sigmaHat;
-    const int ta = threadIdx.x % TD, tb = threadIdx.x / TD;
-    double gB[R][R], gD[R][R];
-#pragma unroll
-    for (int p = 0; p < R; ++p)
-#pragma unroll
-        for (int q = 0; q < R; ++q) { gB[p][q] = 0.0; gD[p][q] = 0.0; }
-    double tr = 0.0;
-    const int ntiles = (d.L + TR - 1) / TR;
-    for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
-        const int l0 = tile * TR, nr = min(TR, d.L - l0);
-        __syncthreads();
-        for (int e = threadIdx.x; e < TR * H; e += NT) {
-            const int h = e / TR, i = e - h * TR;
-            double q = 0.0;
-            if (i < nr) {
-                q = Q[(size_t)h * d.ldB + l0 + i];
-                if (!dense) q *= diag_var ? d.sigmaVec[l0 + i] : sh;
-            }
-            T[i * ld + h] = q;
-        }
-        __syncthreads();
-        for (int e = threadIdx.x; e < TR * H; e += NT) {
-            const int h = e / TR, i = e - h * TR;
-            double bn = 0.0, dn = 0.0;
-            if (i < nr) {
-                double s = 0.0;
-                for (int k = 0; k < H; ++k) s = fma(T[i * ld + k], S[k * ld + h], s);
-                if (dense) s /= s2;
-                const size_t idx = (size_t)h * d.ldB + l0 + i;
-                const double old = d.B[idx];
-                d.Bold[idx] = old;
-                dn = s - old;
-                d.D[idx] = dn;
-                d.B[idx] = s;
-                tr = fma(s, Q[idx], tr);
-                bn = s;
-            }
-            Bn[i * ld + h] = bn;
-            Dn[i * ld + h] = dn;
-        }
-        __syncthreads();
-        for (int i = 0; i < TR; ++i) {
-            double xa[R], xb[R], ya[R], yb[R];
-#pragma unroll
-            for (int q = 0; q < R; ++q) {
-                const int a = ta + TD * q, b = tb + TD * q;
-                xa[q] = (a < H) ? Bn[i * ld + a] : 0.0; xb[q] = (b < H) ? Bn[i * ld + b] : 0.0;
-                ya[q] = (a < H) ? Dn[i * ld + a] : 0.0; yb[q] = (b < H) ? Dn[i * ld + b] : 0.0;
-            }
-#pragma unroll
-            for (int p = 0; p < R; ++p)
-#pragma unroll
-                for (int q = 0; q < R; ++q) { gB[p][q] = fma(xa[p], xb[q], gB[p][q]); gD[p][q] = fma(ya[p], yb[q], gD[p][q]); }
-        }
-    }
-    double* out = d.part + (size_t)blockIdx.x * (2 * H * H + 1);
-#pragma unroll
-    for (int p = 0; p < R; ++p)
-#pragma unroll
-        for (int q = 0; q < R; ++q) {
-            const int a = ta + TD * p, b = tb + TD * q;
-            if (a < H && b < H) { out[a * H + b] = gB[p][q]; out[H * H + a * H + b] = gD[p][q]; }
-        }
-    tr = block_sum(tr, red);
-    if (threadIdx.x == 0) out[2 * H * H] = tr;
-}
 // ---- peer exchange: tile transfers of the row-sharded epilogue.  W is a template parameter and the rounds are real loops so
 // that the executed code stays small: a CTA runs this once or twice, and a fully unrolled, predicated 8-rank version spent
 // 24-32 us per tile fetching its own instructions (measured: the load phase took that long even with W = 1, all local).
@@ -1675,7 +1393,7 @@ __device__ __forceinline__ void px_store_tile(const PxDev& px, const double* __r
         case 7: { constexpr int PW = 7; CALL; } break;                                           \
         default: { constexpr int PW = 8; CALL; } break;                                          \
     }
-// DMMA version of the same epilogue for H <= 64 (HP8 = H rounded up to 8, shared pitch = 4 mod 16 as in the A epilogue):
+// DMMA kernel of this epilogue (formulas at the top of the section), for H <= 64 (HP8 = H rounded up to 8, shared pitch = 4 mod 16 as in the A epilogue):
 //   Bn = (c .* Qtile) * SigmaB [/ sigma2]        32 x HP8 x HP8 product, 4 x HP8/8 mma tiles over 8 warps
 //   G_B += Bn' Bn,  G_D += Dn' Dn                 accumulators in registers across the CTA's tiles
 // PX (peer exchange, world > 1): the CTA grid covers only this rank's share of the 32-row tiles; a tile of Q is the sum of
@@ -1906,8 +1624,7 @@ __global__ void __launch_bounds__(256) B_reduce_kernel(Dev d, int nparts, PxDev 
 }
 int k_B_epilogue(cudaStream_t st, const Dev& d, int flags) {
     const int H = d.H, dv = (flags & F_DIAG_VAR) ? 1 : 0;
-    const int grid = std::max(1, std::min(cdiv(d.L, H > 64 ? 16 : 32), 148));
-    if (H <= 64 && getenv("VBMF_B200_BEPI_SIMT") == nullptr) {
+    if (H <= 64) {
         const int HP8 = (H + 7) & ~7;
         const size_t smem = (size_t)((HP8 + 96) * pitch4(HP8)) * sizeof(double);
         const int grid2 = std::max(1, std::min(cdiv(d.L, 32), 296));      // two CTAs per SM: the tile chain is latency bound
@@ -1918,28 +1635,15 @@ int k_B_epilogue(cudaStream_t st, const Dev& d, int flags) {
         VB_LAUNCH_OK();
         return 0;
     }
-    if (getenv("VBMF_B200_BEPI_SIMT") == nullptr) {
-        // H > 64: product-only DMMA epilogue (the Gram accumulators would not fit in registers), Grams by gram_dmma
-        const int HP8 = (H + 7) & ~7;
-        const size_t smem = (size_t)((HP8 + 32) * pitch4(HP8)) * sizeof(double);
-        const int grid3 = std::max(1, std::min(cdiv(d.L, 32), 148));
-        B_epilogue_dmma_kernel<1, false, false><<<grid3, 256, smem, st>>>(d, dv, PxDev(), 0, 0);
-        VB_LAUNCH_OK();
-        trbq_kernel<<<1, 256, 0, st>>>(d, grid3);
-        VB_LAUNCH_OK();
-        if (gram_dmma(st, d, d.B, false, d.L, d.BtB) || gram_dmma(st, d, d.D, false, d.L, d.DtD)) return -1;
-        return 0;
-    }
-#define BEPI(RR, TDD, TRR)                                                                                                   \
-    {                                                                                                                        \
-        const size_t smem = (size_t)((H + 3 * TRR) * (H + 1)) * sizeof(double);                                              \
-        B_epilogue_kernel<RR, TDD, TRR><<<grid, TDD * TDD, smem, st>>>(d, dv);                                               \
-    }
-    if (H <= 16) BEPI(1, 16, 32) else if (H <= 32) BEPI(2, 16, 32) else if (H <= 64) BEPI(4, 16, 32) else BEPI(4, 32, 16)
-#undef BEPI
+    // H > 64: product-only DMMA epilogue (the Gram accumulators would not fit in registers), Grams by gram_dmma
+    const int HP8 = (H + 7) & ~7;
+    const size_t smem = (size_t)((HP8 + 32) * pitch4(HP8)) * sizeof(double);
+    const int grid3 = std::max(1, std::min(cdiv(d.L, 32), 148));
+    B_epilogue_dmma_kernel<1, false, false><<<grid3, 256, smem, st>>>(d, dv, PxDev(), 0, 0);
     VB_LAUNCH_OK();
-    B_reduce_kernel<false><<<std::max(1, cdiv(2 * H * H + 1, 32)), 256, 0, st>>>(d, grid, PxDev());
+    trbq_kernel<<<1, 256, 0, st>>>(d, grid3);
     VB_LAUNCH_OK();
+    if (gram_dmma(st, d, d.B, false, d.L, d.BtB) || gram_dmma(st, d, d.D, false, d.L, d.DtD)) return -1;
     return 0;
 }
 // updateB!'s epilogue on this rank's share of the rows (peer exchange, H <= 64, homoscedastic noise)
@@ -2461,24 +2165,13 @@ int kernels_init_device() {
     VB_SMEM_ATTR((sparse_A_full_dmma_kernel<1, 4, false>), k4_dmma_smem<1>());
     VB_SMEM_ATTR((sparse_A_full_dmma_kernel<2, 4, false>), k4_dmma_smem<2>());
     VB_SMEM_ATTR((sparse_A_full_dmma_kernel<3, 3, false>), k4_dmma_smem<3>());
-    VB_SMEM_ATTR((sparse_A_full_dmma_kernel<4, 3, false>), k4_dmma_smem<4>());
-    VB_SMEM_ATTR((sparse_A_full_dmma_kernel<4, 2, false>), k4_dmma_smem<4>());
     VB_SMEM_ATTR((sparse_A_full_dmma_kernel<4, 4, true>), k4_dmma_smem<4>());
-    VB_SMEM_ATTR((sparse_A_full_dmma_kernel<4, 3, true>), k4_dmma_smem<4>());
-    VB_SMEM_ATTR(sparse_A_full_warp_kernel<8>, (8 * 32 + 8 * 64 + 8 * 32 + 8 * 8 * 32) * 8);
-    VB_SMEM_ATTR(sparse_A_full_warp_kernel<16>, (16 * 32 + 8 * 64 + 8 * 32 + 8 * 16 * 32) * 8);
-    VB_SMEM_ATTR(sparse_A_full_warp_kernel<24>, (24 * 32 + 8 * 64 + 8 * 32 + 8 * 24 * 32) * 8);
-    VB_SMEM_ATTR(sparse_A_full_warp_kernel<32>, (32 * 32 + 8 * 64 + 8 * 32 + 8 * 32 * 32) * 8);
     const int mxB = (int)((64 + 96) * pitch4(64) * 8);
     VB_SMEM_ATTR((B_epilogue_dmma_kernel<2, true, false>), mxB);
     VB_SMEM_ATTR((B_epilogue_dmma_kernel<8, true, false>), mxB);
     VB_SMEM_ATTR((B_epilogue_dmma_kernel<2, true, true>), mxB);
     VB_SMEM_ATTR((B_epilogue_dmma_kernel<8, true, true>), mxB);
     VB_SMEM_ATTR((B_epilogue_dmma_kernel<1, false, false>), (128 + 32) * pitch4(128) * 8);
-    VB_SMEM_ATTR((B_epilogue_kernel<1, 16, 32>), (16 + 96) * 17 * 8);
-    VB_SMEM_ATTR((B_epilogue_kernel<2, 16, 32>), (32 + 96) * 33 * 8);
-    VB_SMEM_ATTR((B_epilogue_kernel<4, 16, 32>), (64 + 96) * 65 * 8);
-    VB_SMEM_ATTR((B_epilogue_kernel<4, 32, 16>), (128 + 48) * 129 * 8);
     VB_SMEM_ATTR(sigma_rows_kernel, 128 * 128 * 8);
     VB_SMEM_ATTR(post_kernel, post_smem(128));
     VB_SMEM_ATTR(norms_kernel, post_smem(128));

@@ -94,8 +94,6 @@ int k_y_stats_chunk(cudaStream_t st, const Dev& d, int m0, int n, int first);   
 int k_copy_trYTY(cudaStream_t st, const Dev& d, const double* d_tr);      // sc->trYTY = *d_tr (device side, stream ordered)
 int k_sparse_A_diag(cudaStream_t st, const Dev& d, int flags);   // diagonal path incl. Q2 map; partial column sums of s
 int k_sparse_A_full(cudaStream_t st, const Dev& d, int flags);   // batched H x H SPD inverse per column
-int k_sparse_A_full_ex(cudaStream_t st, const Dev& d, int flags, const double* slabs, int S, size_t slab_stride, int fuse_ca);
-bool k_sparse_A_full_can_fuse(const Dev& d);                     // tensor-core path in use (H <= 32): slab sum / updateCA! can be fused
 // whole-loop diagonal path in one pass: slab sum, A, diag, mask, beta/CA (+ group sums), A'A, diag SigmaA -> packed
 int k_sparse_A_diag_fused(cudaStream_t st, const Dev& d, const double* slabs, int S, size_t slab_stride, int flags, int* defer_parts = nullptr);
 int k_sparse_diag_reduce(cudaStream_t st, const Dev& d, int nparts);   // the deferred reduction of the fused diagonal pass
