@@ -275,8 +275,13 @@ int vbmf_b200_solver_yhat(vbmf_b200_solver* s, double* YHat, int64_t ld);
  * kind = VBMF_B200_DENSE, _SPARSE, _DUAL or _TRIAL (the four branches of vbls!, :182-197); states[p] points to the matching
  * state struct of problem p, Y[p] to its L x states[p]->M matrix.  All problems share L, H (and H0); M (and M0) may differ.
  * flags: VBMF_B200_FULL_COV, VBMF_B200_DIAG_VAR (both ignored for dense).  Needs no attached Y.  Limits: H <= 64 for sparse / dual /
- * trial (H > 32 with full_cov inverts one column at a time with the whole CTA) and H <= 32 for dense, no labels; dense
- * problems need a diagonal invCA (what vbmf_init creates and updateCA! maintains).  A problem whose whole state fits one
+ * trial (H > 32 with full_cov inverts one column at a time with the whole CTA) and H <= 32 for dense.  Dense and sparse
+ * problems with H1 > 0 and labels get AHat[labels, H-H1+1:H] = 0 after every A update, as updateA! does (H1 in 0..H and
+ * labels 1-based within 1..M of their own problem, as solver creation requires, else an error naming the problem; H1 may
+ * differ per problem); dual and trial states have no labels.  A dense problem's first SigmaA uses its whole invCA;
+ * updateCA! then leaves invCA = inv(diagonal CA), so after niter >= 1 it comes back diagonal with zeros off the diagonal.
+ * Dense problems need a diagonal CA (what vbmf_init creates and updateCA! maintains).
+ * A problem whose whole state fits one
  * CTA's shared memory runs in a one-CTA-per-problem kernel (one launch for all of them); a larger one runs in the wide
  * kernel, one thread-block cluster of 1, 2, 4 or 8 CTAs per problem (one launch per cluster size), see
  * vbmf_b200_batched_plan. */

@@ -332,6 +332,7 @@ vbmf_trial(Y::Array{Float64,2}, p_in::vbmf_trial_parameters, niter::Int; kw...) 
 # Ys[k] is the L x M_k matrix of problem k, ps[k] its parameters (all of one type, with the same L, H, H0); one method per
 # branch of vbls! (:182-197).  kind: 0 dense, 1 sparse, 2 dual, 3 trial (include/vbmf_b200.h).  Bags of any size: those
 # too large for one CTA's shared memory run in the wide kernel (one thread-block cluster per bag) within the same call.
+# Dense and sparse states pass pointer(p.labels): with H1 > 0 every A update zeroes AHat[labels, H-H1+1:H].
 function batched_call(ctx::B200Context, kind::Int, Ys::Vector{Array{Float64,2}}, sts::Vector, niter::Int, flags::Int)
     yptr = Ptr{Float64}[pointer(Y) for Y in Ys]
     sptr = Ptr{Void}[convert(Ptr{Void}, Base.unsafe_convert(Ptr{eltype(r)}, r)) for r in sts]

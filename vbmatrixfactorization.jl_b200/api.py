@@ -961,7 +961,8 @@ def vbls_batched_(Ys, params_list, niter, full_cov=False, diag_var=False, ctx=No
     for one CTA's shared memory get a thread-block cluster each): the MIL classification pattern, classify(...; class_alg =
     "dual") runs it for every test bag and class model.  All params must be of one type (vbmf_parameters,
     vbmf_sparse_parameters, vbmf_dual_parameters or vbmf_trial_parameters - the four branches of vbls!) with the same L, H
-    (and H0); M (and M0) may differ per problem."""
+    (and H0); M (and M0) may differ per problem.  Dense and sparse parameters with H1 > 0 and labels get AHat[labels,
+    H-H1+1:H] = 0 after every A update, as updateA! does; a dense problem's first iteration uses its whole invCA."""
     batch = BatchedVbls(Ys, params_list, ctx=ctx, yhat=yhat, keep_blocks=keep_blocks)
     batch.run(niter, full_cov=full_cov, diag_var=diag_var)
     return batch.readback()

@@ -123,7 +123,7 @@ __global__ void __launch_bounds__(128, (HP == 0 ? 1 : 3)) batched_vbls_kernel(Ba
                         if (q == lane) dg = a[q];
                     }
                     if (live) {
-                        As[m * H + lane] = ok ? s : nan("");
+                        As[m * H + lane] = batch_masked(bd.mask, m0 + m, lane, H) ? 0.0 : ok ? s : nan("");
                         Ss[m * H + lane] = ok ? dg : nan("");
                         if (bd.blocks != nullptr && it == bd.niter - 1) {
 #pragma unroll
@@ -158,7 +158,7 @@ __global__ void __launch_bounds__(128, (HP == 0 ? 1 : 3)) batched_vbls_kernel(Ba
                     for (int h = t; h < H; h += nt) {
                         double s = 0.0;
                         for (int k = 0; k < H; ++k) s = fma(gs * Mx[h * ld + k], V[m * H + k], s);
-                        As[m * H + h] = ok ? s : nan("");
+                        As[m * H + h] = batch_masked(bd.mask, m0 + m, h, H) ? 0.0 : ok ? s : nan("");
                         Ss[m * H + h] = ok ? Mx[h * ld + h] : nan("");
                     }
                     for (int e = t; e < H * H; e += nt) {
@@ -176,7 +176,7 @@ __global__ void __launch_bounds__(128, (HP == 0 ? 1 : 3)) batched_vbls_kernel(Ba
                 const double dsrc = dvar ? dB[src] + (double)L * s_msv * SBg[src * H + src] : sh * dB[src] + (double)L * SBg[src * H + src];
                 const double s = 1.0 / (dsrc + CAs[e]);
                 Ss[e] = s;
-                As[e] = (gs * s) * V[e];
+                As[e] = batch_masked(bd.mask, m0 + e / H, e % H, H) ? 0.0 : (gs * s) * V[e];
             }
             __syncthreads();
             for (int e = t; e < H * H; e += nt) {
@@ -399,7 +399,7 @@ __global__ void __launch_bounds__(128, (HP == 0 ? 1 : HP == 32 ? 2 : 3)) batched
                         if (q == lane) dg = a[q];
                     }
                     if (live) {
-                        As[m * H + lane] = ok ? s : nan("");
+                        As[m * H + lane] = batch_masked(bd.mask, cb + m, lane, H) ? 0.0 : ok ? s : nan("");
                         Ss[m * H + lane] = ok ? dg : nan("");
                         if (bd.blocks != nullptr && it == bd.niter - 1) {
 #pragma unroll
@@ -433,7 +433,7 @@ __global__ void __launch_bounds__(128, (HP == 0 ? 1 : HP == 32 ? 2 : 3)) batched
                     for (int h = t; h < H; h += nt) {
                         double s = 0.0;
                         for (int k = 0; k < H; ++k) s = fma(gs * Mx[h * ld + k], V[m * H + k], s);
-                        As[m * H + h] = ok ? s : nan("");
+                        As[m * H + h] = batch_masked(bd.mask, cb + m, h, H) ? 0.0 : ok ? s : nan("");
                         Ss[m * H + h] = ok ? Mx[h * ld + h] : nan("");
                     }
                     for (int e = t; e < H * H; e += nt) {
@@ -452,7 +452,7 @@ __global__ void __launch_bounds__(128, (HP == 0 ? 1 : HP == 32 ? 2 : 3)) batched
                 const double dsrc = dvar ? dB[src] + (double)L * s_msv * SBg[src * H + src] : sh * dB[src] + (double)L * SBg[src * H + src];
                 const double s = 1.0 / (dsrc + CAs[e]);
                 Ss[e] = s;
-                As[e] = (gs * s) * V[e];
+                As[e] = batch_masked(bd.mask, cb + e / H, e % H, H) ? 0.0 : (gs * s) * V[e];
             }
             __syncthreads();
             for (int e = t; e < H * H; e += nt) {
@@ -634,6 +634,15 @@ int k_batched_vbls(cudaStream_t st, const BatchDesc& bd, const int (&n)[5], int 
 //   updateCA!     CA[h,h] = ||A[:,h]||^2/M + SigmaA[h,h];  invCA = inv(CA)                               src/vbmf.jl:129-134
 //   updateSigma2! sigma2 = (sum(Y.^2) - 2*tr(Y'B A') + tr((A'A + M*SigmaA)(B'B + L*SigmaB)))/(L*M)       src/vbmf.jl:153-157
 // One H x H inverse per iteration (warp 0, register-resident Gauss-Jordan); B'B, V = B'Y and sum(Y.^2) are loop invariants.
+// With labels, A[labels, H-H1+1:H] = 0 right after A is formed (src/vbmf.jl:101).
+
+// First iteration of a problem whose invCA the call packed in full: one warp writes the precision G0 + sigma2*invCA
+// (src/vbmf.jl:96) into SA, which the inverse then overwrites; updateCA! leaves invCA diagonal for the later iterations.
+__device__ __forceinline__ void dense_full_precision(const double* G0, const double* icF, double s2, double* SA, int H, int lane) {
+    for (int e = lane; e < H * H; e += 32) SA[e] = G0[e] + s2 * icF[e];
+    __syncwarp();
+}
+
 template <int HP>
 __global__ void __launch_bounds__(128) batched_vbls_dense_kernel(BatchDenseDesc bd) {
     extern __shared__ __align__(16) double sm[];
@@ -653,6 +662,7 @@ __global__ void __launch_bounds__(128) batched_vbls_dense_kernel(BatchDenseDesc 
     double* ic = AtA + H * H;                // [H]     diag(invCA)
     double* cd = ic + H;                     // [H]     diag(CA)
     double* scal = bd.scal + (size_t)p * 16;
+    const bool full_ic = bd.invCA != nullptr && scal[1] != 0.0;   // this problem's invCA was packed in full
     const double* Y = bd.Y + (size_t)m0 * L;
     const double* Bg = bd.B + (size_t)p * L * H;
     const double* SBg = bd.SigmaB + (size_t)p * H * H;
@@ -686,11 +696,16 @@ __global__ void __launch_bounds__(128) batched_vbls_dense_kernel(BatchDenseDesc 
         // ---- updateA!: SigmaA
         if (warp == 0) {
             const bool live = lane < H;
+            const bool full = it == 0 && full_ic;
+            if (full) dense_full_precision(G0, bd.invCA + (size_t)p * H * H, s2, SA, H, lane);
+            const double* Gs = full ? SA : G0;
+            const double icd = live && !full ? ic[lane] : 0.0;
+            // a[q] = G + s2*ic unfused, dg = fma(s2, ic, G): the roundings the diagonal-invCA path has always had
             double a[HP];
 #pragma unroll
             for (int q = 0; q < HP; ++q)
-                a[q] = ((q < H && live) ? G0[q * H + lane] : 0.0) + ((q == lane) ? (live ? s2 * ic[lane] : 1.0) : 0.0);
-            const double dg = live ? G0[lane * H + lane] + s2 * ic[lane] : 1.0;
+                a[q] = ((q < H && live) ? Gs[q * H + lane] : 0.0) + ((q == lane) ? (live ? __dmul_rn(s2, icd) : 1.0) : 0.0);
+            const double dg = live ? fma(s2, icd, Gs[lane * H + lane]) : 1.0;
             const bool ok = warp_spd_inverse_reg<HP>(a, dg, lane, s_col);
             if (live) {
 #pragma unroll
@@ -704,7 +719,7 @@ __global__ void __launch_bounds__(128) batched_vbls_dense_kernel(BatchDenseDesc 
             const int m = e / H, h = e - m * H;
             double s = 0.0;
             for (int k = 0; k < H; ++k) s = fma(V[m * H + k], SA[k * H + h], s);
-            As[e] = s / s2;
+            As[e] = batch_masked(bd.mask, m0 + m, h, H) ? 0.0 : s / s2;
         }
         __syncthreads();
         // ---- updateCA! and the Gram of A
@@ -746,16 +761,17 @@ __global__ void __launch_bounds__(128) batched_vbls_dense_kernel(BatchDenseDesc 
 
 // Dense kind, wide problems: one cluster per problem as batched_vbls_wide_kernel.  A, V = B'Y in global memory; after the
 // A'A reduction every CTA computes the H x H SigmaA inverse of the next iteration redundantly from identical inputs.
-// SigmaA = sigma2*inv(G0 + sigma2*diag(ic)) by one warp; kept out of line so that the register-resident inverse does not
-// share its register budget with the rest of the wide kernel
+// SigmaA = sigma2*inv(G0 + sigma2*diag(ic)) by one warp (ic = nullptr: inv(G0)/..., G0 then holds the whole precision);
+// kept out of line so that the register-resident inverse does not share its register budget with the rest of the wide kernel
 template <int HP>
 __device__ __noinline__ bool dense_sigmaA_warp(const double* G0, const double* ic, double s2, double* SA, double* col, int H, int lane) {
     const bool live = lane < H;
+    const double icd = live && ic != nullptr ? ic[lane] : 0.0;
     double a[HP];
 #pragma unroll
     for (int q = 0; q < HP; ++q)
-        a[q] = ((q < H && live) ? G0[q * H + lane] : 0.0) + ((q == lane) ? (live ? s2 * ic[lane] : 1.0) : 0.0);
-    const double dg = live ? G0[lane * H + lane] + s2 * ic[lane] : 1.0;
+        a[q] = ((q < H && live) ? G0[q * H + lane] : 0.0) + ((q == lane) ? (live ? __dmul_rn(s2, icd) : 1.0) : 0.0);
+    const double dg = live ? fma(s2, icd, G0[lane * H + lane]) : 1.0;     // roundings as batched_vbls_dense_kernel
     const bool ok = warp_spd_inverse_reg<HP>(a, dg, lane, col);
     if (live) {
 #pragma unroll
@@ -785,6 +801,7 @@ __global__ void __maxnreg__(255) batched_vbls_dense_wide_kernel(BatchDenseDesc b
     double* cd = ic + H;                     // [H]     diag(CA)
     double* sp = cd + H;                     // [1]     partial sum(Y.^2), then partial trace(V'A)
     double* scal = bd.scal + (size_t)p * 16;
+    const bool full_ic = bd.invCA != nullptr && scal[1] != 0.0;
     const size_t cb = (size_t)m0 + c0;
     const double* Y = bd.Y + cb * L;
     const double* Bg = bd.B + (size_t)p * L * H;
@@ -817,14 +834,18 @@ __global__ void __maxnreg__(255) batched_vbls_dense_wide_kernel(BatchDenseDesc b
     for (int it = 0; it < bd.niter; ++it) {
         const double s2 = s_sig;
         // ---- updateA!: SigmaA (identical on every rank)
-        if (warp == 0 && !dense_sigmaA_warp<HP>(G0, ic, s2, SA, s_col, H, lane) && lane == 0) s_fail = 1.0;
+        if (warp == 0) {
+            const bool full = it == 0 && full_ic;
+            if (full) dense_full_precision(G0, bd.invCA + (size_t)p * H * H, s2, SA, H, lane);
+            if (!dense_sigmaA_warp<HP>(full ? SA : G0, full ? nullptr : ic, s2, SA, s_col, H, lane) && lane == 0) s_fail = 1.0;
+        }
         __syncthreads();
         // ---- A = ((Y'B) * SigmaA) / sigma2 on this CTA's columns
         for (int e = t; e < nc * H; e += nt) {
             const int m = e / H, h = e - m * H;
             double s = 0.0;
             for (int k = 0; k < H; ++k) s = fma(V[m * H + k], SA[k * H + h], s);
-            As[e] = s / s2;
+            As[e] = batch_masked(bd.mask, cb + m, h, H) ? 0.0 : s / s2;
         }
         __syncthreads();
         for (int e = t; e < H * H; e += nt) {

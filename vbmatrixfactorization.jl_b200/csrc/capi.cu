@@ -1956,6 +1956,27 @@ extern "C" int vbmf_b200_batched_plan(int kind, int64_t L, int64_t H, int full_c
     return 0;
 }
 
+// Labels of one dense / sparse problem of a batched call: they take part when H1 > 0 (AHat[labels, H-H1+1:H] = 0.0 after
+// every A update, src/vbmf.jl:101, src/vbmf_sparse.jl:245).  Checked as solver creation checks them: H1 in 0..H, and any
+// labels 1-based within 1..M, whatever H1 is.
+template <class ST> static int batch_check_labels(const ST* s, int64_t p, bool& masked) {
+    if (s->H1 < 0 || s->H1 > s->H) { set_error("batched vbls: H1 of problem %lld must be in 0..H", (long long)p); return -1; }
+    if (s->n_labels <= 0) return 0;
+    if (s->labels == nullptr) { set_error("batched vbls: labels of problem %lld are NULL", (long long)p); return -1; }
+    for (int64_t i = 0; i < s->n_labels; ++i)
+        if (s->labels[i] < 1 || s->labels[i] > s->M) {
+            set_error("batched vbls: label %lld of problem %lld out of range 1..%lld", (long long)s->labels[i], (long long)p, (long long)s->M);
+            return -1;
+        }
+    masked = masked || s->H1 > 0;
+    return 0;
+}
+// the problem's M bytes of the column mask (BatchDesc::mask): H1 on labelled columns, else 0
+template <class ST> static void batch_pack_mask(const ST* s, unsigned char* mk) {
+    memset(mk, 0, (size_t)s->M);
+    if (s->n_labels > 0 && s->H1 > 0) for (int64_t i = 0; i < s->n_labels; ++i) mk[s->labels[i] - 1] = (unsigned char)s->H1;
+}
+
 template <class ST> struct BatchView {
     static const ST* get(void* const* states, int64_t p) { return (const ST*)states[p]; }
 };
@@ -1973,13 +1994,13 @@ static int batched_vbls_impl(vbmf_b200_ctx* c, int kind, int64_t nprob, const do
     if (L < 1 || H < 1 || H > 64) { set_error("batched vbls supports 1 <= H <= 64 (got H = %lld)", (long long)H); return -1; }
     if (H0 < 0 || H0 > H) { set_error("H must be at least H0!"); return -1; }
     std::vector<int> moff(nprob + 1, 0);
-    bool want_yhat = false, want_blocks = false;
+    bool want_yhat = false, want_blocks = false, want_mask = false;
     for (int64_t p = 0; p < nprob; ++p) {
         const ST* s = (const ST*)states[p];
         if (s == nullptr || Y[p] == nullptr) { set_error("batched vbls: NULL problem %lld", (long long)p); return -1; }
         if (s->L != L || s->H != H || s->M < 1) { set_error("batched vbls: problem %lld has different L/H or M < 1", (long long)p); return -1; }
         if constexpr (IS_DUAL || IS_TRIAL) { if (s->H0 != H0) { set_error("batched vbls: H0 differs"); return -1; } }
-        else { if (s->n_labels > 0 && s->H1 > 0) { set_error("batched vbls: labels are not supported"); return -1; } }
+        else { if (batch_check_labels(s, p, want_mask)) return -1; }
         if (dvar && (s->sigmaVecHat == nullptr || s->etaVec == nullptr)) { set_error("batched vbls: diag_var needs sigmaVecHat / etaVec of problem %lld", (long long)p); return -1; }
         moff[p + 1] = moff[p] + (int)s->M;
         want_yhat = want_yhat || s->YHat != nullptr;
@@ -1997,6 +2018,7 @@ static int batched_vbls_impl(vbmf_b200_ctx* c, int kind, int64_t nprob, const do
     const bool wide = ngrp[0] < nprob;
     const size_t o_moff = take((size_t)(nprob + 1) * 4), o_pl = take((size_t)nprob * 4), o_Y = take(L * Mtot * 8), o_B = take(nprob * LH * 8),
                  o_SB = take(nprob * HH * 8);
+    const size_t o_mk = want_mask ? take(Mtot) : 0;
     const size_t down_begin = off;
     const size_t o_CA = take(MH * 8), o_sc = take((size_t)nprob * 16 * 8);
     const size_t o_sv = dvar ? take((size_t)nprob * L * 8) : 0, o_ev = dvar ? take((size_t)nprob * L * 8) : 0;
@@ -2021,6 +2043,7 @@ static int batched_vbls_impl(vbmf_b200_ctx* c, int kind, int64_t nprob, const do
         memcpy(&hB[p * LH], s->BHat, LH * 8);
         memcpy(&hSB[p * HH], s->SigmaB, HH * 8);
         memcpy(&hCA[(size_t)moff[p] * H], s->CA, (size_t)s->M * H * 8);
+        if constexpr (!IS_DUAL && !IS_TRIAL) { if (want_mask) batch_pack_mask(s, (unsigned char*)(hb + o_mk) + moff[p]); }
         if (dvar) {
             memcpy((double*)(hb + o_sv) + (size_t)p * L, s->sigmaVecHat, (size_t)L * 8);
             memcpy((double*)(hb + o_ev) + (size_t)p * L, s->etaVec, (size_t)L * 8);
@@ -2049,6 +2072,7 @@ static int batched_vbls_impl(vbmf_b200_ctx* c, int kind, int64_t nprob, const do
     bd.plist = (const int*)(db + o_pl);
     bd.V = wide ? (double*)(db + o_V) : nullptr;
     bd.rowv = wide && dvar ? (double*)(db + o_rv) : nullptr;
+    bd.mask = want_mask ? (const unsigned char*)(db + o_mk) : nullptr;
     prof_mark(c, c->ev_k1);       // profiling: the kernels alone (read back through vbmf_b200_ctx_profile_read, K1 slot)
     if (bd.niter > 0) rc = k_batched_vbls(st, bd, ngrp, Mmax0);
     prof_mark(c, c->ev_k1);
@@ -2130,14 +2154,19 @@ static int batched_vbls_dense_impl(vbmf_b200_ctx* c, int64_t nprob, const double
     const int64_t L = s0->L, H = s0->H;
     if (L < 1 || H < 1 || H > 32) { set_error("batched vbls supports 1 <= H <= 32 (got H = %lld)", (long long)H); return -1; }
     std::vector<int> moff(nprob + 1, 0);
-    bool want_yhat = false;
+    std::vector<char> full_ic(nprob, 0);    // invCA of the problem has a non-zero off-diagonal entry
+    bool want_yhat = false, want_mask = false, want_icF = false;
     for (int64_t p = 0; p < nprob; ++p) {
         const ST* s = (const ST*)states[p];
         if (s == nullptr || Y[p] == nullptr) { set_error("batched vbls: NULL problem %lld", (long long)p); return -1; }
         if (s->L != L || s->H != H || s->M < 1) { set_error("batched vbls: problem %lld has different L/H or M < 1", (long long)p); return -1; }
-        if (s->n_labels > 0 && s->H1 > 0) { set_error("batched vbls: labels are not supported"); return -1; }
-        for (int64_t a = 0; a < H; ++a) for (int64_t b = 0; b < H; ++b)
-            if (a != b && s->invCA[a + b * H] != 0.0) { set_error("batched vbls: invCA of problem %lld is not diagonal", (long long)p); return -1; }
+        if (batch_check_labels(s, p, want_mask)) return -1;
+        // updateCA! sets the diagonal of CA and inverts the whole matrix (src/vbmf.jl:129-134); the kernels keep CA diagonal
+        if (s->CA) for (int64_t a = 0; a < H; ++a) for (int64_t b = 0; b < H; ++b)
+            if (a != b && s->CA[a + b * H] != 0.0) { set_error("batched vbls: CA of problem %lld is not diagonal", (long long)p); return -1; }
+        for (int64_t a = 0; a < H && !full_ic[p]; ++a) for (int64_t b = 0; b < H; ++b)
+            if (a != b && s->invCA[a + b * H] != 0.0) { full_ic[p] = 1; break; }
+        want_icF = want_icF || full_ic[p];
         moff[p + 1] = moff[p] + (int)s->M;
         want_yhat = want_yhat || s->YHat != nullptr;
     }
@@ -2151,6 +2180,8 @@ static int batched_vbls_dense_impl(vbmf_b200_ctx* c, int64_t nprob, const double
     const bool wide = ngrp[0] < nprob;
     const size_t o_moff = take((size_t)(nprob + 1) * 4), o_pl = take((size_t)nprob * 4), o_Y = take(L * Mtot * 8), o_B = take(nprob * LH * 8),
                  o_SB = take(nprob * HH * 8);
+    // the full invCA of every problem only when one of them is not diagonal, so that a call on diagonal ones copies no more
+    const size_t o_mk = want_mask ? take(Mtot) : 0, o_icF = want_icF ? take(nprob * HH * 8) : 0;
     const size_t down_begin = off;
     const size_t o_ic = take(nprob * H * 8), o_sc = take((size_t)nprob * 16 * 8);
     const size_t up_end = off;
@@ -2171,7 +2202,10 @@ static int batched_vbls_dense_impl(vbmf_b200_ctx* c, int64_t nprob, const double
         memcpy(&hB[p * LH], s->BHat, LH * 8);
         memcpy(&hSB[p * HH], s->SigmaB, HH * 8);
         for (int64_t h = 0; h < H; ++h) hic[p * H + h] = s->invCA[h + h * H];
+        if (want_icF) memcpy((double*)(hb + o_icF) + p * HH, s->invCA, HH * 8);
+        if (want_mask) batch_pack_mask(s, (unsigned char*)(hb + o_mk) + moff[p]);
         hsc[(size_t)p * 16] = s->sigma2;
+        hsc[(size_t)p * 16 + 1] = full_ic[p] ? 1.0 : 0.0;
     }
     cudaStream_t st = c->st;
     if (cudaMemcpyAsync(db, hb, up_end, cudaMemcpyHostToDevice, st) != cudaSuccess) { cudaGetLastError(); set_error("batched vbls: upload failed"); return -1; }
@@ -2181,6 +2215,8 @@ static int batched_vbls_dense_impl(vbmf_b200_ctx* c, int64_t nprob, const double
     bd.A = (double*)(db + o_A); bd.SigmaA = (double*)(db + o_SA); bd.icA = (double*)(db + o_ic); bd.cA = (double*)(db + o_c);
     bd.YHat = want_yhat ? (double*)(db + o_YH) : nullptr; bd.scal = (double*)(db + o_sc);
     bd.plist = (const int*)(db + o_pl); bd.V = wide ? (double*)(db + o_V) : nullptr;
+    bd.mask = want_mask ? (const unsigned char*)(db + o_mk) : nullptr;
+    bd.invCA = want_icF ? (const double*)(db + o_icF) : nullptr;
     int rc = 0;
     prof_mark(c, c->ev_k1);
     if (bd.niter > 0) rc = k_batched_vbls_dense(st, bd, ngrp, Mmax0);
@@ -2202,6 +2238,8 @@ static int batched_vbls_dense_impl(vbmf_b200_ctx* c, int64_t nprob, const double
             if (s->CA) s->CA[h + h * H] = hc[p * H + h];
             if (s->invCA) s->invCA[h + h * H] = hic[p * H + h];
         }
+        // updateCA! made invCA the inverse of the diagonal CA
+        if (full_ic[p] && s->invCA) for (int64_t a = 0; a < H; ++a) for (int64_t b = 0; b < H; ++b) if (a != b) s->invCA[a + b * H] = 0.0;
         if (s->YHat) memcpy(s->YHat, &hYH[(size_t)moff[p] * L], M * L * 8);
         s->sigma2 = hsc[(size_t)p * 16];
     }

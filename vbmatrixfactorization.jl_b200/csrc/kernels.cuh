@@ -162,7 +162,13 @@ struct BatchDesc {
     const int* plist;       // problem of each launched CTA (one-CTA kernel) or cluster (wide kernel)
     double* V;              // wide kernel: [Mtot][H] V = B'Y (diag_var: B'diag(sv)Y)
     double* rowv;           // wide kernel, diag_var: [nprob][1 + 8][L] = ||Y[l,:]||^2 | per-rank partials of Y[l,:]*(A*b_l)
+    const unsigned char* mask;   // [Mtot] or nullptr: H1 of the column's problem if the column is labelled, else 0;
+                                 // A[col, H-mask[col]:H] = 0 after every A update (src/vbmf_sparse.jl:245)
 };
+// true when element h of packed column col of A is zeroed by the labels (AHat[labels, H-H1+1:H] = 0.0)
+__device__ __forceinline__ bool batch_masked(const unsigned char* mask, size_t col, int h, int H) {
+    return mask != nullptr && h >= H - (int)mask[col];
+}
 struct BatchDenseDesc {
     int nprob, L, H, niter, Mmax;
     const int* moff;
@@ -174,9 +180,12 @@ struct BatchDenseDesc {
     double* icA;            // [nprob][H] in: diag(invCA), out: diag(invCA)
     double* cA;             // [nprob][H] out: diag(CA)
     double* YHat;           // [L][Mtot] out or nullptr
-    double* scal;           // [nprob][16]
+    double* scal;           // [nprob][16]: 0 sigma2 (in/out), 1 = 1 when the problem's invCA is in `invCA` (in), 13 fail (out)
     const int* plist;       // as BatchDesc::plist
     double* V;              // wide kernel: [Mtot][H] V = B'Y
+    const unsigned char* mask;   // as BatchDesc::mask (src/vbmf.jl:101)
+    const double* invCA;    // [nprob][H*H] or nullptr: the full invCA of the first iteration's SigmaA (src/vbmf.jl:96), read
+                            // for the problems flagged in scal[1]; the others keep the diagonal path's arithmetic
 };
 constexpr int BATCH_MAX_CLUSTER = 8;   // portable thread-block cluster size
 // CTAs of the wide kernel per problem: 0 = the problem fits the one-CTA kernel, else 1, 2, 4 or 8; -1 = H out of range
