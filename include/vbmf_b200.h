@@ -255,6 +255,19 @@ int vbmf_b200_solver_step(vbmf_b200_solver* s, int step, int flags);
 /* the while-loop of vbmf! (src/vbmf.jl:193-214), vbmf_sparse! (src/vbmf_sparse.jl:368-393), vbmf_dual!
  * (src/vbmf_dual.jl:480-513) with the convergence test on the device.  iters = iterations done, d = last delta. */
 int vbmf_b200_solver_run(vbmf_b200_solver* s, int64_t niter, double eps, int flags, int norm_mode, int64_t* iters, double* d);
+/* Run the loops of n solvers of ONE single-GPU context in lockstep, with one K1 and one K2 per iteration serving all of them
+ * (the sum of their H at most 64).  Each member behaves as vbmf_b200_solver_run would with its own flags[i]:
+ *   - the same updates, in the same order;
+ *   - its own convergence test: iters[i] and d[i] come back per member;
+ *   - a member that has stopped keeps its state while the others go on;
+ *   - failed[i] = 1 when its posterior precision was not positive definite: NaN in its state, its loop ended.
+ * A member's result depends only on its own uploaded state, the resident Y and the sum of the members' H (which fixes the
+ * split-K plans): reordering the members or changing another member's data leaves it bit for bit the same, and a group of
+ * one equals vbmf_b200_solver_run.  Refused: n < 1, a solver twice, solvers of different contexts, a context with world > 1
+ * or the peer exchange, a context without Y, a sum of H above 64.
+ * Returns -2 when any member failed and 0 otherwise; other errors as usual, with every member's state unchanged. */
+int vbmf_b200_solver_run_group(int n, vbmf_b200_solver* const* solvers, const int* flags, int64_t niter, double eps,
+                               int norm_mode, int64_t* iters, double* d, int* failed);
 /* The same loop with the reference's per-iteration logging hook (`update_log!(log, params)` after every iteration when
  * logdir != "", src/vbmf.jl:206-208, src/vbmf_sparse.jl:385-387, src/vbmf_dual.jl:505-507; log format src/data_manip.jl:6-66):
  * after each iteration the device is synchronised and cb(user, s, iterations_done, d) runs on the calling thread; it may call

@@ -20,7 +20,7 @@ import VBMatrixFactorization: vbmf!, vbmf, vbmf_sparse!, vbmf_sparse, vbmf_dual!
                               lowerBound, lowerBoundTrimmed
 
 export b200_context, b200_close, b200_peer_exchange, b200_default_context!, vbmf!, vbmf, vbmf_sparse!, vbmf_sparse, vbmf_dual!, vbmf_dual, vbmf_trial!, vbmf_trial,
-       lowerBound, lowerBoundTrimmed, vbls_batched!, lowerBound_batched, lowerBoundTrimmed_batched, preprocess
+       lowerBound, lowerBoundTrimmed, vbls_batched!, lowerBound_batched, lowerBoundTrimmed_batched, preprocess, vbmf_group!
 
 const LIB = get(ENV, "VBMF_B200_LIB", "libvbmf_b200.so")
 
@@ -327,6 +327,96 @@ function vbmf_trial(ctx::B200Context, Y, p_in::vbmf_trial_parameters, niter::Int
 end
 vbmf_trial!(Y::Array{Float64,2}, p::vbmf_trial_parameters, niter::Int; kw...) = vbmf_trial!(default_context(), Y, p, niter; kw...)
 vbmf_trial(Y::Array{Float64,2}, p_in::vbmf_trial_parameters, niter::Int; kw...) = vbmf_trial(default_context(), Y, p_in, niter; kw...)
+
+# ---- several models fitted to one Y in lockstep (vbmf_b200_solver_run_group) ---------------------------------------------------
+# ps may mix the four parameter types; opts[i] holds member i's keyword options of its solo driver (est_covs, est_var /
+# diag_var, full_cov, est_cb, est_priors) with the same defaults.  One pass of each contraction over Y per iteration serves
+# every member; their H must add up to at most 64.  Single-device contexts only.  Returns the (iterations, d) of each member.
+group_flags(p::vbmf_parameters, o) = (get(o, :est_covs, false) ? 16 : 0) | (get(o, :est_var, false) ? 32 : 0)
+group_flags(p::vbmf_sparse_parameters, o) = (get(o, :diag_var, false) ? 1 : 0) | (get(o, :full_cov, false) ? 2 : 0) |
+                                            (get(o, :est_cb, true) ? 4 : 0)
+group_flags(p::Union{vbmf_dual_parameters,vbmf_trial_parameters}, o) = (get(o, :diag_var, false) ? 1 : 0) | (get(o, :full_cov, false) ? 2 : 0) |
+                                                                       (get(o, :est_cb, true) ? 4 : 0) | (get(o, :est_priors, true) ? 8 : 0)
+function group_solver(ctx::B200Context, kind::Int, H::Int, split::Int, labels::Vector{Int64})
+    h = Ref{Ptr{Void}}(C_NULL)
+    check(ccall((:vbmf_b200_solver_create, LIB), Cint, (Ptr{Void}, Cint, Int64, Int64, Int64, Ptr{Int64}, Cint, Ptr{Ptr{Void}}),
+                ctx.handle, kind, H, split, length(labels), labels, 0, h))
+    return h[]
+end
+function group_member(ctx::B200Context, p::vbmf_parameters)
+    st = Ref(DenseState(p.L, p.M, p.H, p.H1, length(p.labels), pointer(p.labels), pointer(p.AHat), pointer(p.BHat),
+                        pointer(p.SigmaA), pointer(p.SigmaB), pointer(p.CA), pointer(p.CB), pointer(p.invCA), pointer(p.invCB),
+                        p.sigma2, convert(Ptr{Float64}, C_NULL)))
+    s = group_solver(ctx, 0, p.H, p.H1, p.labels)
+    check(ccall((:vbmf_b200_dense_upload, LIB), Cint, (Ptr{Void}, Ref{DenseState}), s, st))
+    return s, st
+end
+function group_member(ctx::B200Context, p::vbmf_sparse_parameters)
+    st = Ref(sparse_state(p, convert(Ptr{Float64}, C_NULL), false))
+    s = group_solver(ctx, 1, p.H, p.H1, p.labels)
+    check(ccall((:vbmf_b200_sparse_upload, LIB), Cint, (Ptr{Void}, Ref{SparseState}), s, st))
+    return s, st
+end
+function group_member(ctx::B200Context, p::vbmf_dual_parameters)
+    st = Ref(dual_state(p, false))
+    s = group_solver(ctx, 2, p.H, p.H0, Int64[])
+    check(ccall((:vbmf_b200_dual_upload, LIB), Cint, (Ptr{Void}, Ref{DualState}), s, st))
+    return s, st
+end
+function group_member(ctx::B200Context, p::vbmf_trial_parameters)
+    st = Ref(trial_state(p, false))
+    h = Ref{Ptr{Void}}(C_NULL)
+    check(ccall((:vbmf_b200_solver_create_trial, LIB), Cint, (Ptr{Void}, Int64, Int64, Int64, Cint, Ptr{Ptr{Void}}),
+                ctx.handle, p.H, p.H0, p.M0, 0, h))
+    check(ccall((:vbmf_b200_trial_upload, LIB), Cint, (Ptr{Void}, Ref{TrialState}), h[], st))
+    return h[], st
+end
+function group_readback!(p::vbmf_parameters, s, st)
+    check(ccall((:vbmf_b200_dense_download, LIB), Cint, (Ptr{Void}, Ref{DenseState}), s, st))
+    p.sigma2 = st[].sigma2
+end
+function group_readback!(p::vbmf_sparse_parameters, s, st)
+    check(ccall((:vbmf_b200_sparse_download, LIB), Cint, (Ptr{Void}, Ref{SparseState}), s, st))
+    p.sigmaHat = st[].sigmaHat; p.zeta = st[].zeta
+end
+function group_readback!(p::vbmf_dual_parameters, s, st)
+    check(ccall((:vbmf_b200_dual_download, LIB), Cint, (Ptr{Void}, Ref{DualState}), s, st))
+    r = st[]
+    p.sigmaHat = r.sigmaHat; p.zeta = r.zeta
+    p.alpha00 = r.alpha00; p.beta00 = r.beta00; p.alpha01 = r.alpha01; p.beta01 = r.beta01; p.alpha0 = r.alpha0; p.alpha1 = r.alpha1
+end
+function group_readback!(p::vbmf_trial_parameters, s, st)
+    check(ccall((:vbmf_b200_trial_download, LIB), Cint, (Ptr{Void}, Ref{TrialState}), s, st))
+    r = st[]
+    p.sigmaHat = r.sigmaHat; p.zeta = r.zeta
+    p.alpha01 = r.alpha01; p.beta01 = r.beta01; p.alpha02 = r.alpha02; p.beta02 = r.beta02; p.alpha03 = r.alpha03; p.beta03 = r.beta03
+    p.alpha1 = r.alpha1; p.alpha2 = r.alpha2; p.alpha3 = r.alpha3
+end
+function vbmf_group!(ctx::B200Context, Y, ps::Vector, niter::Int; eps::Float64 = 1e-6, opts::Vector = [Dict{Symbol,Any}() for p in ps],
+                     norm = :spectral)
+    ctx.multi && error("vbmf_group! runs on a single-device context")
+    length(opts) == length(ps) || error("vbmf_group!: one options entry per model")
+    attach!(ctx, Y)
+    for p in ps; p.YHat = Array{Float64}(0, 0); end
+    members = Any[]
+    try
+        for p in ps; push!(members, group_member(ctx, p)); end
+        n = length(ps)
+        hs = Ptr{Void}[m[1] for m in members]
+        flags = Cint[group_flags(p, o) for (p, o) in zip(ps, opts)]
+        iters = zeros(Int64, n); d = zeros(Float64, n); failed = zeros(Cint, n)
+        rc = ccall((:vbmf_b200_solver_run_group, LIB), Cint,
+                   (Cint, Ptr{Ptr{Void}}, Ptr{Cint}, Int64, Float64, Cint, Ptr{Int64}, Ptr{Float64}, Ptr{Cint}),
+                   n, hs, flags, niter, eps, NORM[norm], iters, d, failed)
+        rc == -2 || check(rc)
+        for (p, m) in zip(ps, members); group_readback!(p, m[1], m[2]); end
+        rc == -2 && warn("vbmf_group!: a posterior precision matrix was not positive definite (NaN written, loop ended) for members ",
+                         find(failed .!= 0))
+        return [(iters[i], d[i]) for i in 1:n]
+    finally
+        for m in members; ccall((:vbmf_b200_solver_destroy, LIB), Cint, (Ptr{Void},), m[1]); end
+    end
+end
 
 # ---- vbls! for many bags in one call (examples/mil_util.jl:179-203, 504-511) ----------------------------------------------------
 # Ys[k] is the L x M_k matrix of problem k, ps[k] its parameters (all of one type, with the same L, H, H0); one method per

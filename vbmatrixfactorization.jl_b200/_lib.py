@@ -100,6 +100,7 @@ SYMBOLS = {
     "vbmf_b200_trial_download": (C.c_int, [C.c_void_p, C.POINTER(TrialState)]),
     "vbmf_b200_solver_step": (C.c_int, [C.c_void_p, C.c_int, C.c_int]),
     "vbmf_b200_solver_run": (C.c_int, [C.c_void_p, c_i64, c_f64, C.c_int, C.c_int, p_i64, p_f64]),
+    "vbmf_b200_solver_run_group": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, c_i64, c_f64, C.c_int, p_i64, p_f64, C.c_void_p]),
     "vbmf_b200_solver_run_logged": (C.c_int, [C.c_void_p, c_i64, c_f64, C.c_int, C.c_int, ITER_CALLBACK, C.c_void_p, p_i64, p_f64]),
     "vbmf_b200_solver_lower_bound": (C.c_int, [C.c_void_p, c_f64, C.c_int, p_f64]),
     "vbmf_b200_solver_yhat": (C.c_int, [C.c_void_p, p_f64, c_i64]),

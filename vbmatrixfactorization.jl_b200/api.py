@@ -28,7 +28,7 @@ __all__ = [
     "vbmf_init", "vbmf_", "vbmf", "vbmf_sparse_init", "vbmf_sparse_", "vbmf_sparse", "vbmf_dual_init", "vbmf_dual_",
     "vbmf_dual", "updateA_", "updateB_", "updateCA_", "updateCB_", "updateSigma2_", "updateSigma_", "updateYHat_",
     "updateAlpha00_", "updateAlpha01_", "updateBeta00_", "updateBeta01_", "lowerBound", "lowerBoundTrimmed", "copy",
-    "vbls_", "vbls_batched_", "BatchedVbls", "lowerBound_batched", "lowerBoundTrimmed_batched", "preprocess", "VBMFWarning", "create_log", "update_log_", "save_log", "load_log", "extract_params_", "VBMFError",
+    "run_group", "vbmf_group_", "vbls_", "vbls_batched_", "BatchedVbls", "lowerBound_batched", "lowerBoundTrimmed_batched", "preprocess", "VBMFWarning", "create_log", "update_log_", "save_log", "load_log", "extract_params_", "VBMFError",
 ]
 
 VBMFError = L_.VBMFError
@@ -740,6 +740,78 @@ def vbmf_trial(Y, params_in, niter, **kw):
     p = copy(params_in)
     d = vbmf_trial_(Y, p, niter, **kw)
     return p, d
+
+
+# ----------------------------------------------------------------------------------------------------------- lockstep group
+def run_group(solvers, niter, eps=1e-6, flags=None, norm="spectral"):
+    """Run the loops of several Solvers of one single-GPU Context together (vbmf_b200_solver_run_group): one pass of each
+    contraction over the resident Y per iteration serves every member, whose H must add up to at most 64.  flags[i] are
+    member i's run flags (default 0).  Returns [(iters, d), ...] and sets each Solver.failed; a VBMFWarning names a member
+    whose posterior precision was not positive definite."""
+    solvers = list(solvers)
+    if any(isinstance(getattr(s, "ctx", None), MultiContext) for s in solvers):
+        raise VBMFError("run_group runs solvers of ONE single-device Context; a MultiContext is not supported")
+    n = len(solvers)
+    flags = [0] * n if flags is None else [int(f) for f in flags]
+    if len(flags) != n:
+        raise VBMFError("run_group: %d solvers but %d flags" % (n, len(flags)))
+    lib = L_.load()
+    hs = (C.c_void_p * max(n, 1))(*[s.h for s in solvers])
+    fl = (C.c_int * max(n, 1))(*flags)
+    it, d, failed = (C.c_int64 * max(n, 1))(), (C.c_double * max(n, 1))(), (C.c_int * max(n, 1))()
+    rc = L_.check(lib.vbmf_b200_solver_run_group(n, C.cast(hs, C.c_void_p), C.cast(fl, C.c_void_p), int(niter), float(eps),
+                                                 _NORMS[norm], C.cast(it, C.c_void_p), C.cast(d, C.c_void_p),
+                                                 C.cast(failed, C.c_void_p)), allow=(-2,))
+    for i, s in enumerate(solvers):
+        s.failed = bool(failed[i])
+    if rc == -2:
+        _not_pd(rc)
+    return [(it[i], d[i]) for i in range(n)]
+
+
+_GROUP_OPTIONS = {
+    L_.DENSE: {"est_covs": False, "est_var": False},
+    L_.SPARSE: {"diag_var": False, "full_cov": False, "est_cb": True, "keep_blocks": False},
+    L_.DUAL: {"diag_var": False, "full_cov": False, "est_priors": True, "est_cb": True, "keep_blocks": False},
+    L_.TRIAL: {"diag_var": False, "full_cov": False, "est_priors": True, "est_cb": True, "keep_blocks": False},
+}
+
+
+def vbmf_group_(Y, params_list, niter, eps=1e-6, options=None, norm="spectral", ctx=None, yhat=False):
+    """Fit several models to the same Y in lockstep (run_group): uploads every params object, runs, downloads, and sets
+    params.iterations, params.d and params.failed on each.  options[i] holds the keyword arguments of member i's solo driver
+    (vbmf_ / vbmf_sparse_ / vbmf_dual_ / vbmf_trial_: est_covs, est_var, diag_var, full_cov, est_cb, est_priors, keep_blocks)
+    with the same defaults.  yhat=True also downloads each member's YHat = BHat * AHat'.  Returns params_list."""
+    if isinstance(ctx, MultiContext):
+        raise VBMFError("vbmf_group_ runs on ONE single-device Context; a MultiContext is not supported")
+    params_list = list(params_list)
+    options = [{}] * len(params_list) if options is None else list(options)
+    if len(options) != len(params_list):
+        raise VBMFError("vbmf_group_: %d params but %d option sets" % (len(params_list), len(options)))
+    ctx = _ctx_for(Y, ctx)
+    solvers, flags = [], []
+    try:
+        for p, o in zip(params_list, options):
+            known = _GROUP_OPTIONS[p.kind]
+            unknown = set(o) - set(known)
+            if unknown:
+                raise TypeError("vbmf_group_: options %s do not apply to this member's kind" % sorted(unknown))
+            opt = dict(known, **o)
+            keep = bool(opt.pop("keep_blocks", False))
+            s = Solver(ctx, p, keep_blocks=keep)
+            solvers.append(s)
+            s.upload(p)
+            flags.append(_flags(**opt))
+        res = run_group(solvers, niter, eps, flags, norm)
+        for p, s, (it, d) in zip(params_list, solvers, res):
+            s.download(p, want_yhat=yhat)
+            if p.kind == L_.SPARSE:
+                p.AHat = _f(p.AHat)
+            p.iterations, p.d, p.failed = it, d, s.failed
+    finally:
+        for s in solvers:
+            s.close()
+    return params_list
 
 
 # ----------------------------------------------------------------------------------------------------------- step functions

@@ -830,6 +830,11 @@ struct vbmf_b200_solver {
     size_t px_packed = 0, px_B = 0, px_gpart = 0, px_small = 0;
     cudaEvent_t ev_a = nullptr, ev_sb = nullptr;   // A side of the iteration done (main) -> small exchange + SigmaB (side) -> epilogue (main)
     Scalars h_sc;
+    // vbmf_b200_solver_run_group: while set, the group's INT8 K1 / K2 have already written this solver's slabs, and enq_k1 /
+    // enq_k2 only reduce them.  gslab: slab buffers for the group's split-K plans when Ppart / Qpart are too small (grow-only).
+    bool grouped = false;
+    double* gslab = nullptr;
+    size_t gslab_elems = 0;
 };
 
 
@@ -984,6 +989,7 @@ extern "C" int vbmf_b200_solver_destroy(vbmf_b200_solver* s) {
     if (s->ev_sb) cudaEventDestroy(s->ev_sb);
     if (s->arena) cudaFree(s->arena);
     if (s->Qc) cudaFree(s->Qc);
+    if (s->gslab) cudaFree(s->gslab);
     if (s->h_flag) cudaFreeHost(s->h_flag);
     for (int i = 0; i < 2; ++i) if (s->ev[i]) cudaEventDestroy(s->ev[i]);
     if (s->px) s->c->px.claimed = false;
@@ -1243,6 +1249,11 @@ static int enq_k1(vbmf_b200_solver* s, bool scaledB, bool reduce_slabs = true) {
     const Dev& d = s->d;
     if (c->Y == nullptr) { set_error("this step contracts with Y: attach Y first (the context only holds its shape)"); return -1; }
     if (settle_upload(s)) return -1;
+    if (s->grouped) {
+        const int rc = (s->S1 > 1 && reduce_slabs) ? k_sum_slabs(c->st, s->Ppart, s->S1, (size_t)d.Mloc * d.H, d.P, d.sc) : 0;
+        prof_seg(c, SEG_K1);
+        return rc;
+    }
     bool i8 = false;
     if (s->i8 && ctx_slices(c, &i8)) return -1;
     prof_mark(c, c->ev_k1);
@@ -1267,10 +1278,16 @@ static int enq_k2(vbmf_b200_solver* s) {
     const Dev& d = s->d;
     if (c->Y == nullptr) { set_error("this step contracts with Y: attach Y first (the context only holds its shape)"); return -1; }
     if (settle_upload(s)) return -1;
+    int rc = 0;
+    if (s->grouped) {
+        prof_seg(c, SEG_K2);
+        rc = k_reduce_q(c->st, d, s->Qpart, s->S);
+        prof_seg(c, SEG_REDUCE_Q);
+        return rc;
+    }
     bool i8 = false;
     if (s->i8 && ctx_slices(c, &i8)) return -1;
     prof_mark(c, c->ev_k2);
-    int rc;
     if (i8) rc = i8_k2(c, &s->i8o, d.A, d.H, s->Qpart, d.ldB, s->S, s->kchunk, d.sc);
     else if (s->k2_simt) rc = launch_gemm_ya_simt(c->st, d.Y, d.ldY, d.A, s->Qpart, d.L, d.Mloc, d.H, d.ldB, s->kchunk, s->S, d.sc);
     else rc = launch_gemm_ya(c->st, &c->tmY2, &s->tmA, s->Qpart, d.L, d.Mloc, d.H, d.ldB, s->kchunk, s->S, d.sc, c->num_sms);
@@ -1390,49 +1407,61 @@ static PxDev px_view(vbmf_b200_solver* s, int nbar, int site) {
     }
     return p;
 }
+// whole-loop updateB! up to K2 (px: the peer exchange; otherwise one GPU): the Gram sums and SigmaB on the side stream
+static int enq_updateB_front(vbmf_b200_solver* s, int flags, bool px) {
+    const Dev& d = s->d;
+    cudaStream_t st = s->c->st;
+    // px: updateB! with the exchange done by our own kernels over NVLink: the small sums are gathered from the peers, SigmaB
+    // is inverted redundantly, every rank reduces its share of the rows of Y*AHat over the peers, runs the epilogue on
+    // them and writes the new BHat rows to every peer; the Grams of BHat / BHat - Bold are exchanged as rank partials.
+    // (The heteroscedastic row update needs all rows of the reduced Y*AHat on every rank: that case keeps the all-reduce.)
+    // One GPU: nothing to exchange.  Either way SigmaB needs the A side of the iteration only, so the Gram partial sum,
+    // the small exchange and the inverse run on the side stream beside K2 (their few CTAs share the SMs with K2's).
+    if (d.kind != KIND_DENSE && (flags & F_DIAG_VAR) && !s->mean_valid) { if (k_mean_sigma(st, d)) return -1; s->mean_valid = true; }
+    VB_CUDA_OK(cudaEventRecord(s->ev_a, st));
+    VB_CUDA_OK(cudaStreamWaitEvent(s->side, s->ev_a, 0));
+    // AHat'AHat (full covariance path: a Gram pass over AHat; otherwise the deferred sums of the A-side partials)
+    if (!s->ata_local && k_gram(s->side, d, d.A, true, d.Mloc, nullptr, d.packed + packed_ata(d))) return -1;
+    s->ata_local = false;
+    if (s->ata_parts > 0 && k_sum_gram_partials(s->side, d, s->ata_parts)) return -1;
+    s->ata_parts = 0;
+    if (s->diag_parts > 0 && k_sparse_diag_reduce(s->side, d, s->diag_parts)) return -1;
+    s->diag_parts = 0;
+    if (px && k_px_small(s->side, d, px_view(s, 1, 0))) return -1;
+    if (k_sigmaB(s->side, d, flags)) return -1;
+    VB_CUDA_OK(cudaEventRecord(s->ev_sb, s->side));
+    return 0;
+}
+// ... and after K2: the BHat epilogue
+static int enq_updateB_back(vbmf_b200_solver* s, int flags, bool px) {
+    const Dev& d = s->d;
+    cudaStream_t st = s->c->st;
+    if (px) prof_mark(s->c, s->c->ev_ar);
+    VB_CUDA_OK(cudaStreamWaitEvent(st, s->ev_sb, 0));
+    prof_seg(s->c, SEG_SIGMA_B);
+    if (px) {
+        int nparts = 1;
+        if (k_B_epilogue_px(st, d, flags, px_view(s, 1, 1), &nparts)) return -1;
+        prof_seg(s->c, SEG_B_EPI);
+        if (k_B_reduce_px(st, d, px_view(s, 1, 2), nparts)) return -1;
+        prof_seg(s->c, SEG_B_REDUCE);
+        prof_mark(s->c, s->c->ev_ar);
+    } else {
+        if (k_B_epilogue(st, d, flags)) return -1;
+        prof_seg(s->c, SEG_B_EPI);
+    }
+    s->ata_valid = true; s->extras_valid = true;
+    s->q_valid = !px;                           // px: packed.Q is reduced on this rank's rows only
+    s->btb_valid = !(d.kind != KIND_DENSE && (flags & F_DIAG_VAR));           // weighted Grams / Bs still stale with diag_var
+    return 0;
+}
 static int enq_updateB(vbmf_b200_solver* s, int flags, bool fused) {
     const Dev& d = s->d;
     cudaStream_t st = s->c->st;
     const bool px = fused && s->px && !(d.kind != KIND_DENSE && (flags & F_DIAG_VAR));
     if (px || (fused && s->c->world == 1)) {
-        // px: updateB! with the exchange done by our own kernels over NVLink: the small sums are gathered from the peers, SigmaB
-        // is inverted redundantly, every rank reduces its share of the rows of Y*AHat over the peers, runs the epilogue on
-        // them and writes the new BHat rows to every peer; the Grams of BHat / BHat - Bold are exchanged as rank partials.
-        // (The heteroscedastic row update needs all rows of the reduced Y*AHat on every rank: that case keeps the all-reduce.)
-        // One GPU: nothing to exchange.  Either way SigmaB needs the A side of the iteration only, so the Gram partial sum,
-        // the small exchange and the inverse run on the side stream beside K2 (their few CTAs share the SMs with K2's).
-        if (d.kind != KIND_DENSE && (flags & F_DIAG_VAR) && !s->mean_valid) { if (k_mean_sigma(st, d)) return -1; s->mean_valid = true; }
-        VB_CUDA_OK(cudaEventRecord(s->ev_a, st));
-        VB_CUDA_OK(cudaStreamWaitEvent(s->side, s->ev_a, 0));
-        // AHat'AHat (full covariance path: a Gram pass over AHat; otherwise the deferred sums of the A-side partials)
-        if (!s->ata_local && k_gram(s->side, d, d.A, true, d.Mloc, nullptr, d.packed + packed_ata(d))) return -1;
-        s->ata_local = false;
-        if (s->ata_parts > 0 && k_sum_gram_partials(s->side, d, s->ata_parts)) return -1;
-        s->ata_parts = 0;
-        if (s->diag_parts > 0 && k_sparse_diag_reduce(s->side, d, s->diag_parts)) return -1;
-        s->diag_parts = 0;
-        if (px && k_px_small(s->side, d, px_view(s, 1, 0))) return -1;
-        if (k_sigmaB(s->side, d, flags)) return -1;
-        VB_CUDA_OK(cudaEventRecord(s->ev_sb, s->side));
-        if (enq_k2(s)) return -1;
-        if (px) prof_mark(s->c, s->c->ev_ar);
-        VB_CUDA_OK(cudaStreamWaitEvent(st, s->ev_sb, 0));
-        prof_seg(s->c, SEG_SIGMA_B);
-        if (px) {
-            int nparts = 1;
-            if (k_B_epilogue_px(st, d, flags, px_view(s, 1, 1), &nparts)) return -1;
-            prof_seg(s->c, SEG_B_EPI);
-            if (k_B_reduce_px(st, d, px_view(s, 1, 2), nparts)) return -1;
-            prof_seg(s->c, SEG_B_REDUCE);
-            prof_mark(s->c, s->c->ev_ar);
-        } else {
-            if (k_B_epilogue(st, d, flags)) return -1;
-            prof_seg(s->c, SEG_B_EPI);
-        }
-        s->ata_valid = true; s->extras_valid = true;
-        s->q_valid = !px;                           // px: packed.Q is reduced on this rank's rows only
-        s->btb_valid = !(d.kind != KIND_DENSE && (flags & F_DIAG_VAR));           // weighted Grams / Bs still stale with diag_var
-        return 0;
+        if (enq_updateB_front(s, flags, px) || enq_k2(s)) return -1;
+        return enq_updateB_back(s, flags, px);
     }
     if (!fused && d.kind != KIND_DENSE) {
         // step-level: packed.SA must hold the (global) SigmaA the state carries
@@ -1514,15 +1543,20 @@ extern "C" int vbmf_b200_solver_step(vbmf_b200_solver* s, int step, int flags) {
     return 0;
 }
 
-static int enq_iteration(vbmf_b200_solver* s, int flags) {
+// One whole-loop iteration in three phases: iter_front (K1 and the A side), updateB! (K2 in its middle), iter_back (the
+// heteroscedastic row update and the tail).  vbmf_b200_solver_run_group interleaves the phases of several solvers.
+static int iter_front(vbmf_b200_solver* s, int flags) {
     const Dev& d = s->d;
-    cudaStream_t st = s->c->st;
     prof_seg(s->c, SEG_START);
     if (enq_updateA(s, flags, true)) return -1;                       // updateA!
     if (d.kind != KIND_DENSE && !s->ca_done && enq_updateCA(s, flags, true)) return -1;   // updateCA! (local; hoisted before the all-reduce)
     s->ca_done = false;
     prof_seg(s->c, SEG_A_EPI);
-    if (enq_updateB(s, flags, true)) return -1;                       // updateB! (+ Grams of BHat and of BHat - Bold)
+    return 0;
+}
+static int iter_back(vbmf_b200_solver* s, int flags) {
+    const Dev& d = s->d;
+    cudaStream_t st = s->c->st;
     if (d.kind != KIND_DENSE && (flags & F_DIAG_VAR)) {
         if (k_sigma_rows(st, d)) return -1;                           // updateSigma! (per-row)
         if (flags & F_FULL_COV) { if (k_gram(st, d, d.B, false, d.L, d.sigmaVec, d.BtBw)) return -1; }
@@ -1541,6 +1575,11 @@ static int enq_iteration(vbmf_b200_solver* s, int flags) {
     VB_CUDA_OK(cudaEventRecord(s->ev_p, s->side));
     s->post_pending = true;
     return 0;
+}
+static int enq_iteration(vbmf_b200_solver* s, int flags) {
+    if (iter_front(s, flags)) return -1;
+    if (enq_updateB(s, flags, true)) return -1;                       // updateB! (+ Grams of BHat and of BHat - Bold)
+    return iter_back(s, flags);
 }
 
 // First dense iteration while Y is still arriving (asynchronous chunked attach): row m of AHat needs only column m of Y, and
@@ -1682,6 +1721,206 @@ extern "C" int vbmf_b200_solver_run(vbmf_b200_solver* s, int64_t niter, double e
         return -1;
     }
     if (s->h_sc.chol_fail) { set_error("a posterior precision matrix was not positive definite (NaN written, loop ended)"); return -2; }
+    return 0;
+}
+
+// ---- several solvers of one context in lockstep ---------------------------------------------------------------------------
+// One pass over Y's INT8 digit planes per contraction serves every member: their operand digits are packed side by side
+// (member g at rows [off_g, off_g + H_g) of the group planes), the split-K plans are those of the total width, and the
+// flush writes each column to its member's own slabs.  Each member's other kernels are its solo ones, in the solo order.
+struct GroupRun {
+    vbmf_b200_ctx* c = nullptr;
+    std::vector<vbmf_b200_solver*> m;
+    std::vector<int> flags, off;
+    int Htot = 0;
+    bool i8 = false;
+    int S1 = 1, kbs1 = 1, S = 1, kchunk = 32;
+    I8Operands o;
+    I8GroupOut k1, k2;
+    struct Saved { double *Ppart, *Qpart; int S1, kbs1, S, kchunk; };
+    std::vector<Saved> saved;
+    ~GroupRun() {     // the members get their own plans and slab buffers back
+        for (size_t g = 0; g < saved.size(); ++g) {
+            vbmf_b200_solver* s = m[g];
+            s->Ppart = saved[g].Ppart; s->Qpart = saved[g].Qpart;
+            s->S1 = saved[g].S1; s->kbs1 = saved[g].kbs1; s->S = saved[g].S; s->kchunk = saved[g].kchunk;
+            s->grouped = false;
+        }
+    }
+};
+// The INT8 path of a group: digit planes for the total width and, per member, slabs for the group's plans (its own Ppart /
+// Qpart when they are large enough, else its grow-only gslab).  g->i8 stays false when the FP64 contractions are selected or
+// the planes cannot be allocated: the members then contract one after another with their own plans.
+static int group_setup_i8(GroupRun* g) {
+    vbmf_b200_ctx* c = g->c;
+    if (!ctx_int8_wanted(c, g->Htot)) return 0;
+    bool ok = false;
+    if (ctx_slices(c, &ok)) return -1;
+    if (!ok) return 0;
+    i8_plans(c->L, c->Mloc, g->Htot, c->num_sms, &g->S1, &g->kbs1, &g->S, &g->kchunk);
+    if (i8_operands_alloc(&g->o, c->L, c->Mloc, g->Htot, g->S, &ok)) return -1;
+    if (!ok) return 0;
+    const int Hp = i8_hpad(g->Htot), ldZ = i8_ld(c->L);
+    // the rows past the total width are never written: zero digits once
+    VB_CUDA_OK(cudaMemsetAsync(g->o.Wb, 0, (size_t)I8_NSL * Hp * ldZ, c->st));
+    VB_CUDA_OK(cudaMemsetAsync(g->o.Wa, 0, (size_t)I8_NSL * Hp * g->o.ldM, c->st));
+    memset(&g->k1, 0, sizeof(I8GroupOut));
+    memset(&g->k2, 0, sizeof(I8GroupOut));
+    g->k1.nmem = g->k2.nmem = (int)g->m.size();
+    for (size_t i = 0; i < g->m.size(); ++i) {
+        vbmf_b200_solver* s = g->m[i];
+        const Dev& d = s->d;
+        const size_t MH = (size_t)d.Mloc * d.H, LH = (size_t)d.H * d.ldB;
+        const bool own_p = g->S1 == 1 || (s->Ppart != nullptr && s->S1 >= g->S1);
+        const bool own_q = std::max(s->S, s->S_chunk) >= g->S;
+        const size_t need = (own_p ? 0 : (size_t)g->S1 * MH) + (own_q ? 0 : (size_t)g->S * LH);
+        if (need > s->gslab_elems) {
+            VB_CUDA_OK(cudaStreamSynchronize(c->st));
+            if (s->gslab) cudaFree(s->gslab);
+            s->gslab = nullptr; s->gslab_elems = 0;
+            if (cudaMalloc(&s->gslab, need * 8) != cudaSuccess) {
+                cudaGetLastError(); s->gslab = nullptr;
+                set_error("run_group: cudaMalloc of %zu bytes of split-K slabs failed", need * 8);
+                return -1;
+            }
+            s->gslab_elems = need;
+        }
+        g->saved.push_back({s->Ppart, s->Qpart, s->S1, s->kbs1, s->S, s->kchunk});
+        double* P = g->S1 == 1 ? d.P : (own_p ? s->Ppart : s->gslab);
+        double* Q = own_q ? s->Qpart : s->gslab + (own_p ? 0 : (size_t)g->S1 * MH);
+        s->Ppart = g->S1 == 1 ? s->Ppart : P; s->Qpart = Q;
+        s->S1 = g->S1; s->kbs1 = g->kbs1; s->S = g->S; s->kchunk = g->kchunk;
+        s->grouped = true;
+        for (int h = 0; h < d.H; ++h) {
+            const int j = g->off[i] + h;
+            g->k1.base[j] = P + h; g->k1.rs[j] = d.H; g->k1.slab[j] = (long long)MH;
+            g->k2.base[j] = Q + (size_t)h * d.ldB; g->k2.rs[j] = 1; g->k2.slab[j] = (long long)LH;
+        }
+        g->k1.sc[i] = g->k2.sc[i] = d.sc;
+    }
+    g->i8 = true;
+    return 0;
+}
+static int group_k1(GroupRun* g) {
+    vbmf_b200_ctx* c = g->c;
+    const int Hp = i8_hpad(g->Htot);
+    const int* F = c->Zexp;
+    const int* E = c->Zexp + c->L;
+    const int* Ebad = c->Zexp + 2 * c->L + c->Mloc;
+    prof_mark(c, c->ev_k1);
+    for (size_t i = 0; i < g->m.size(); ++i) {
+        const Dev& d = g->m[i]->d;
+        const double* B = (g->flags[i] & F_DIAG_VAR) ? d.Bs : d.B;       // enq_updateA: diag_var contracts diag(sigmaVecHat) * BHat
+        if (i8_slice_B_group(c->st, B, d.ldB, c->L, d.H, g->off[i], Hp, F, g->o.Wb, c->ldZ, g->o.Gb, d.sc)) return -1;
+    }
+    if (launch_gemm_i8_group(c->st, false, &c->tmZ1, &g->o.tmWb, g->k1, c->Mloc, c->L, g->S1, g->kbs1 * 16, g->Htot, E, Ebad, g->o.Gb, 0,
+                             c->num_sms)) return -1;
+    prof_mark(c, c->ev_k1);
+    return 0;
+}
+static int group_k2(GroupRun* g) {
+    vbmf_b200_ctx* c = g->c;
+    const int Hp = i8_hpad(g->Htot);
+    const int* F = c->Zexp;
+    const int* E = c->Zexp + c->L;
+    const int* Fbad = c->Zexp + c->L + c->Mloc;
+    prof_mark(c, c->ev_k2);
+    VB_CUDA_OK(cudaMemsetAsync(g->o.Ga, 0x80, (size_t)g->S * Hp * 4, c->st));
+    for (size_t i = 0; i < g->m.size(); ++i) {
+        const Dev& d = g->m[i]->d;
+        if (i8_slice_A_group(c->st, d.A, c->Mloc, d.H, g->off[i], Hp, E, g->kchunk, g->o.Wa, g->o.ldM, g->o.Ga, d.sc)) return -1;
+    }
+    if (launch_gemm_i8_group(c->st, true, &c->tmZ2, &g->o.tmWa, g->k2, c->L, c->Mloc, g->S, g->kchunk, g->Htot, F, Fbad, g->o.Ga, Hp,
+                             c->num_sms)) return -1;
+    prof_mark(c, c->ev_k2);
+    return 0;
+}
+// one iteration of every member: group K1, the A sides, group K2, the B sides and tails (without the INT8 path each member's
+// enq_k1 / enq_k2 contracts on its own)
+static int group_iteration(GroupRun* g) {
+    if (g->i8 && group_k1(g)) return -1;
+    for (size_t i = 0; i < g->m.size(); ++i)
+        if (iter_front(g->m[i], g->flags[i]) || enq_updateB_front(g->m[i], g->flags[i], false)) return -1;
+    if (g->i8 && group_k2(g)) return -1;
+    for (size_t i = 0; i < g->m.size(); ++i)
+        if (enq_k2(g->m[i]) || enq_updateB_back(g->m[i], g->flags[i], false) || iter_back(g->m[i], g->flags[i])) return -1;
+    return 0;
+}
+
+extern "C" int vbmf_b200_solver_run_group(int n, vbmf_b200_solver* const* solvers, const int* flags, int64_t niter, double eps,
+                                          int norm_mode, int64_t* iters, double* dout, int* failed) {
+    if (n < 1 || solvers == nullptr || flags == nullptr) { set_error("run_group: needs n >= 1 solvers and their flags"); return -1; }
+    GroupRun g;
+    for (int i = 0; i < n; ++i) {
+        vbmf_b200_solver* s = solvers[i];
+        if (s == nullptr) { set_error("run_group: solver %d is NULL", i); return -1; }
+        for (int j = 0; j < i; ++j)
+            if (solvers[j] == s) { set_error("run_group: solver %d appears twice (members %d and %d)", i, j, i); return -1; }
+        if (g.c == nullptr) g.c = s->c;
+        if (s->c != g.c) { set_error("run_group: every member must belong to one context (member %d does not)", i); return -1; }
+        g.m.push_back(s);
+        g.off.push_back(g.Htot);
+        g.flags.push_back(s->d.kind == KIND_DENSE ? flags[i] & (F_EST_COVS | F_EST_VAR) : flags[i]);
+        g.Htot += s->d.H;
+    }
+    vbmf_b200_ctx* c = g.c;
+    if (c->world > 1 || c->px.ok) { set_error("run_group: a context with world > 1 or the peer exchange is not supported (single-GPU contexts only)"); return -1; }
+    if (c->Y == nullptr) { set_error("run_group: the context has no Y attached (only its shape)"); return -1; }
+    if (g.Htot > I8_GROUP_MAX) {
+        set_error("run_group: the members' H add up to %d; a group shares one contraction of width at most %d", g.Htot, I8_GROUP_MAX);
+        return -1;
+    }
+    if (niter > 0x7fffffff) niter = 0x7fffffff;
+    if (niter < 0) niter = 0;
+    VB_CUDA_OK(cudaSetDevice(c->device));
+    cudaStream_t st = c->st;
+    // the loop set-up of vbmf_b200_solver_run, member by member; the group waits for an asynchronous upload as a whole
+    if (ctx_wait_upload(c)) return -1;
+    for (int i = 0; i < n; ++i) {
+        vbmf_b200_solver* s = g.m[i];
+        if (k_set_control(st, s->d, (int)niter, eps, norm_mode, 0)) return -1;
+        s->btb_valid = false; s->sigmaA_ahead = false; s->loop_ahead = true;
+        if (enq_gram_B(s, g.flags[i]) || k_norms_init(st, s->d) || settle_upload(s)) return -1;
+    }
+    int rc = group_setup_i8(&g);
+    int64_t enq = 0;
+    int slot = 0;
+    bool pending = false;
+    const int CHUNK = 4;
+    while (!rc && enq < niter) {
+        const int64_t k = std::min<int64_t>(CHUNK, niter - enq);
+        for (int64_t i = 0; i < k && !rc; ++i) rc = group_iteration(&g);
+        if (rc) break;
+        enq += k;
+        for (auto* s : g.m) {
+            if (cudaMemcpyAsync(&s->h_flag[slot], &s->d.sc->active, sizeof(int), cudaMemcpyDeviceToHost, s->side) != cudaSuccess ||
+                cudaEventRecord(s->ev[slot], s->side) != cudaSuccess) { set_error("run_group: flag copy failed"); rc = -1; break; }
+        }
+        if (rc) break;
+        if (pending) {
+            bool any = false;
+            for (auto* s : g.m) {
+                if (cudaEventSynchronize(s->ev[slot ^ 1]) != cudaSuccess) { set_error("run_group: synchronisation failed"); rc = -1; break; }
+                any |= s->h_flag[slot ^ 1] != 0;
+            }
+            if (rc || !any) break;
+        }
+        pending = true;
+        slot ^= 1;
+    }
+    bool any_failed = false;
+    for (int i = 0; i < n; ++i) {
+        vbmf_b200_solver* s = g.m[i];
+        s->loop_ahead = false; s->sigmaA_ahead = false;
+        if (wait_post(s) || pull_scalars(s)) return -1;
+        if (iters) iters[i] = s->h_sc.iter;
+        if (dout) dout[i] = s->h_sc.d;
+        const bool f = s->h_sc.chol_fail != 0;
+        if (failed) failed[i] = f ? 1 : 0;
+        any_failed |= f;
+    }
+    if (rc) return rc;
+    if (any_failed) { set_error("a posterior precision matrix was not positive definite (NaN written, loop ended)"); return -2; }
     return 0;
 }
 

@@ -67,6 +67,27 @@ int launch_gemm_i8(cudaStream_t st, bool mn, const CUtensorMap* tmA, const CUten
                    int S, int klen, int H, const int* rowexp, const int* rowbad, const int* colexp, int cstride, size_t slab,
                    size_t rs, size_t hs, const Scalars* sc, int num_sms);
 
+// ---- one INT8 contraction for several solvers of one context (vbmf_b200_solver_run_group), sum of their H <= 64 ----
+// Member g's columns are rows [off_g, off_g + H_g) of the operand planes [7][Hp][ld] (Hp = sum of H rounded up to 16); the
+// rows past the sum stay zero.  Output column j goes to its member's own buffer: element (row, j) of slab s is
+// base[j][s*slab[j] + row*rs[j]].  The launch does nothing once every member's sc->active is 0.
+constexpr int I8_GROUP_MAX = 64;
+struct I8GroupOut {
+    double* base[I8_GROUP_MAX];
+    long long rs[I8_GROUP_MAX], slab[I8_GROUP_MAX];
+    const Scalars* sc[I8_GROUP_MAX];
+    int nmem;
+};
+// the member's operand digits at row offset `off` of the group planes (plane stride Hp), gated by the member's sc
+int i8_slice_B_group(cudaStream_t st, const double* B, int ldB, int L, int H, int off, int Hp, const int* F, uint8_t* W, int ldZ,
+                     int* G, const Scalars* sc);
+// (the caller resets G[S][Hp] to 0x80808080 once per contraction before the members' calls)
+int i8_slice_A_group(cudaStream_t st, const double* A, int M, int H, int off, int Hp, const int* E, int kchunk, uint8_t* W, int ldM,
+                     int* G, const Scalars* sc);
+int launch_gemm_i8_group(cudaStream_t st, bool mn, const CUtensorMap* tmA, const CUtensorMap* tmB, const I8GroupOut& out, int nrows,
+                         int kdim, int S, int klen, int H, const int* rowexp, const int* rowbad, const int* colexp, int cstride,
+                         int num_sms);
+
 // Plain SIMT FP64 versions (debug / cross-check only; selected with VBMF_B200_GEMM=simt).
 int launch_gemm_ytb_simt(cudaStream_t st, const double* Y, int ldY, const double* B, int ldB, double* P,
                          int M, int L, int H, int ldP, const Scalars* sc);

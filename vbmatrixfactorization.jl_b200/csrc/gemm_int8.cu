@@ -258,8 +258,9 @@ __global__ void __launch_bounds__(256) a_exp_kernel(const double* __restrict__ A
     if (cur >= 0 && e > EXP_NONE) atomicMax(G + cur * Hp + h, e);
 }
 
-// 64 rows per CTA through shared memory; output K-major [7][Hp][ldM]
-__global__ void __launch_bounds__(256) a_slices_kernel(const double* __restrict__ A, int M, int H, int Hp, const int* __restrict__ E, int kchunk,
+// 64 rows per CTA through shared memory; output K-major [7][Hp][ldM], rows [0, Hw) written (solo: Hw = Hp, the padding rows get
+// zero digits; group member: Hw = H)
+__global__ void __launch_bounds__(256) a_slices_kernel(const double* __restrict__ A, int M, int H, int Hp, int Hw, const int* __restrict__ E, int kchunk,
                                                        const int* __restrict__ G, uint8_t* __restrict__ W, int ldM, const Scalars* __restrict__ sc) {
     if (sc != nullptr && !sc->active) return;
     __shared__ double tile[64 * 64];
@@ -268,7 +269,7 @@ __global__ void __launch_bounds__(256) a_slices_kernel(const double* __restrict_
     for (int t = threadIdx.x; t < nm * H; t += blockDim.x) tile[t] = A[(size_t)m0 * H + t];
     __syncthreads();
     const size_t plane = (size_t)Hp * ldM;
-    for (int t = threadIdx.x; t < Hp * 16; t += blockDim.x) {
+    for (int t = threadIdx.x; t < Hw * 16; t += blockDim.x) {
         const int h = t >> 4, g = t & 15;
         if (m0 + 4 * g >= ldM) continue;
         long long x[4];
@@ -290,12 +291,26 @@ __global__ void __launch_bounds__(256) a_slices_kernel(const double* __restrict_
 // multiple of 32).  Output element (row, h) of slab s: out[s*slab + row*rs + h*hs] = 2^(rowexp[row] + colexp[s*cstride + h])
 // * sum over the k range, or NaN when rowbad[row] is set or the column exponent is EXP_NAN (a non-finite input reaches the
 // element); rows >= nrows and h >= H are not written.
-template <bool MN>
-__global__ void __launch_bounds__(192, 1)
-gemm_i8_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, double* __restrict__ out,
-               int nrows, int kdim, int S, int klen, int H, int Hp, const int* __restrict__ rowexp,
-               const int* __restrict__ rowbad, const int* __restrict__ colexp, int cstride, size_t slab, size_t rs, size_t hs, const Scalars* __restrict__ sc) {
-    if (sc != nullptr && !sc->active) return;
+// Where the epilogue writes: `row(s, r)` once per work item and row, `col(that, h)` per element.
+struct SoloOut {            // one buffer with strides (slab, rs, hs)
+    double* out;
+    size_t slab, rs, hs;
+    __device__ __forceinline__ double* row(int sp, int r) const { return out + (size_t)sp * slab + (size_t)r * rs; }
+    __device__ __forceinline__ double* col(double* o, int h) const { return o + (size_t)h * hs; }
+};
+struct GroupOut {           // every column to its member's buffer (I8GroupOut, a kernel parameter)
+    const I8GroupOut* g;
+    struct Pos { int sp, r; };
+    __device__ __forceinline__ Pos row(int sp, int r) const { return {sp, r}; }
+    __device__ __forceinline__ double* col(Pos p, int h) const {
+        return g->base[h] + (size_t)p.sp * (size_t)g->slab[h] + (size_t)p.r * (size_t)g->rs[h];
+    }
+};
+
+template <bool MN, class Out>
+__device__ __forceinline__ void gemm_i8_body(const CUtensorMap* tmA, const CUtensorMap* tmB, const Out& out, int nrows, int kdim, int S,
+                                             int klen, int H, int Hp, const int* __restrict__ rowexp, const int* __restrict__ rowbad,
+                                             const int* __restrict__ colexp, int cstride) {
     extern __shared__ uint8_t smem_raw[];
     const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
     const uint32_t full0 = base + STAGES * SB, empty0 = full0 + STAGES * 8;
@@ -333,9 +348,9 @@ gemm_i8_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
                     const uint32_t s = it % STAGES, ph = (it / STAGES) & 1;
                     mbar_wait(empty0 + 8 * s, ph ^ 1);
                     mbar_expect_tx(full0 + 8 * s, tx_bytes);
-                    if (MN) tma_load_3d(base + s * SB, &tmA, full0 + 8 * s, r0, k, 0);
-                    else tma_load_3d(base + s * SB, &tmA, full0 + 8 * s, k, r0, 0);
-                    tma_load_3d(base + s * SB + A_BYTES, &tmB, full0 + 8 * s, k, 0, 0);
+                    if (MN) tma_load_3d(base + s * SB, tmA, full0 + 8 * s, r0, k, 0);
+                    else tma_load_3d(base + s * SB, tmA, full0 + 8 * s, k, r0, 0);
+                    tma_load_3d(base + s * SB + A_BYTES, tmB, full0 + 8 * s, k, 0, 0);
                 }
             }
         }
@@ -384,7 +399,7 @@ gemm_i8_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             const bool live = row < nrows;
             const int re = live ? rowexp[row] : 0;
             const bool bad = live && rowbad[row] != 0;
-            double* o = out + (size_t)sp * slab + (size_t)(live ? row : 0) * rs;
+            const auto o = out.row(sp, live ? row : 0);
             const int* ce = colexp + (size_t)sp * cstride;
             for (int kb0 = 0; kb0 < nkb; kb0 += SEG_KB, ++sg) {
                 mbar_wait(tfull, sg & 1);
@@ -404,7 +419,7 @@ gemm_i8_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
                         if (live && h < H) {
                             const double x = (bad || ce[h] == EXP_NAN) ? __longlong_as_double(0x7ff8000000000000ll)
                                                                        : ldexp(acc, re + ce[h] - 14);
-                            double* p = o + (size_t)h * hs;
+                            double* p = out.col(o, h);
                             *p = kb0 == 0 ? x : *p + x;
                         }
                     }
@@ -421,6 +436,27 @@ gemm_i8_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         tc_fence_after();
         asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(ncols) : "memory");
     }
+}
+
+template <bool MN>
+__global__ void __launch_bounds__(192, 1)
+gemm_i8_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, double* __restrict__ out,
+               int nrows, int kdim, int S, int klen, int H, int Hp, const int* __restrict__ rowexp,
+               const int* __restrict__ rowbad, const int* __restrict__ colexp, int cstride, size_t slab, size_t rs, size_t hs, const Scalars* __restrict__ sc) {
+    if (sc != nullptr && !sc->active) return;
+    gemm_i8_body<MN>(&tmA, &tmB, SoloOut{out, slab, rs, hs}, nrows, kdim, S, klen, H, Hp, rowexp, rowbad, colexp, cstride);
+}
+
+// Several solvers' columns in one pass over Y's digits; skipped as a whole once no member is active.
+template <bool MN>
+__global__ void __launch_bounds__(192, 1)
+gemm_i8_group_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const __grid_constant__ I8GroupOut g,
+                     int nrows, int kdim, int S, int klen, int H, int Hp, const int* __restrict__ rowexp,
+                     const int* __restrict__ rowbad, const int* __restrict__ colexp, int cstride) {
+    int live = 0;
+    for (int i = 0; i < g.nmem; ++i) live |= g.sc[i]->active;
+    if (!live) return;
+    gemm_i8_body<MN>(&tmA, &tmB, GroupOut{&g}, nrows, kdim, S, klen, H, Hp, rowexp, rowbad, colexp, cstride);
 }
 
 }  // namespace i8k
@@ -454,6 +490,8 @@ int make_tmap_3d_i8(CUtensorMap* out, const void* base, uint64_t d0, uint64_t d1
 int gemm_i8_init_device() {
     VB_CUDA_OK(cudaFuncSetAttribute(gemm_i8_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM));
     VB_CUDA_OK(cudaFuncSetAttribute(gemm_i8_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM));
+    VB_CUDA_OK(cudaFuncSetAttribute(gemm_i8_group_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM));
+    VB_CUDA_OK(cudaFuncSetAttribute(gemm_i8_group_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM));
     return 0;
 }
 
@@ -482,7 +520,24 @@ int i8_slice_A(cudaStream_t st, const double* A, int M, int H, const int* E, int
     VB_CUDA_OK(cudaMemsetAsync(G, 0x80, (size_t)S * Hp * 4, st));
     a_exp_kernel<<<(M + 255) / 256, 256, 0, st>>>(A, M, H, Hp, E, kchunk, G, sc);
     VB_LAUNCH_OK();
-    a_slices_kernel<<<(ldM + 63) / 64, 256, 0, st>>>(A, M, H, Hp, E, kchunk, G, W, ldM, sc);
+    a_slices_kernel<<<(ldM + 63) / 64, 256, 0, st>>>(A, M, H, Hp, Hp, E, kchunk, G, W, ldM, sc);
+    VB_LAUNCH_OK();
+    return 0;
+}
+
+int i8_slice_B_group(cudaStream_t st, const double* B, int ldB, int L, int H, int off, int Hp, const int* F, uint8_t* W, int ldZ,
+                     int* G, const Scalars* sc) {
+    b_slices_kernel<<<H, 512, 0, st>>>(B, ldB, L, H, Hp, F, W + (size_t)off * ldZ, ldZ, G + off, sc);
+    VB_LAUNCH_OK();
+    return 0;
+}
+
+int i8_slice_A_group(cudaStream_t st, const double* A, int M, int H, int off, int Hp, const int* E, int kchunk, uint8_t* W, int ldM,
+                     int* G, const Scalars* sc) {
+    if (M <= 0) return 0;
+    a_exp_kernel<<<(M + 255) / 256, 256, 0, st>>>(A, M, H, Hp, E, kchunk, G + off, sc);
+    VB_LAUNCH_OK();
+    a_slices_kernel<<<(ldM + 63) / 64, 256, 0, st>>>(A, M, H, Hp, H, E, kchunk, G + off, W + (size_t)off * ldM, ldM, sc);
     VB_LAUNCH_OK();
     return 0;
 }
@@ -497,6 +552,20 @@ int launch_gemm_i8(cudaStream_t st, bool mn, const CUtensorMap* tmA, const CUten
     const int grid = std::max(1, std::min(nwork, num_sms));
     if (mn) gemm_i8_kernel<true><<<grid, 192, SMEM, st>>>(*tmA, *tmB, out, nrows, kdim, S, klen, H, i8_hpad(H), rowexp, rowbad, colexp, cstride, slab, rs, hs, sc);
     else gemm_i8_kernel<false><<<grid, 192, SMEM, st>>>(*tmA, *tmB, out, nrows, kdim, S, klen, H, i8_hpad(H), rowexp, rowbad, colexp, cstride, slab, rs, hs, sc);
+    VB_LAUNCH_OK();
+    return 0;
+}
+
+int launch_gemm_i8_group(cudaStream_t st, bool mn, const CUtensorMap* tmA, const CUtensorMap* tmB, const I8GroupOut& out, int nrows,
+                         int kdim, int S, int klen, int H, const int* rowexp, const int* rowbad, const int* colexp, int cstride,
+                         int num_sms) {
+    if (H > I8_GROUP_MAX) { set_error("group width %d > %d is not supported by the INT8 contraction", H, I8_GROUP_MAX); return -1; }
+    if (klen % KB != 0) { set_error("INT8 split-K chunk %d is not a multiple of %d", klen, KB); return -1; }
+    if (nrows <= 0 || kdim <= 0 || H <= 0) return 0;
+    const int nwork = ((nrows + TM - 1) / TM) * S;
+    const int grid = std::max(1, std::min(nwork, num_sms));
+    if (mn) gemm_i8_group_kernel<true><<<grid, 192, SMEM, st>>>(*tmA, *tmB, out, nrows, kdim, S, klen, H, i8_hpad(H), rowexp, rowbad, colexp, cstride);
+    else gemm_i8_group_kernel<false><<<grid, 192, SMEM, st>>>(*tmA, *tmB, out, nrows, kdim, S, klen, H, i8_hpad(H), rowexp, rowbad, colexp, cstride);
     VB_LAUNCH_OK();
     return 0;
 }
