@@ -317,6 +317,16 @@ int vbmf_b200_batched_plan(int kind, int64_t L, int64_t H, int full_cov, int dia
  * bound is the same bit for bit whatever batch it is in. */
 int vbmf_b200_batched_lower_bound(vbmf_b200_ctx* ctx, int kind, int64_t nprob, const double* const* Y,
                                   void* const* states, double trim, int trimmed, double* out);
+/* norm(Y[p] - BHat*AHat') of nprob independent problems in one call, out[p] per problem.  norm_mode =
+ * VBMF_B200_NORM_SPECTRAL (Julia 0.5 norm(::Matrix), largest singular value) or VBMF_B200_NORM_FROBENIUS (vecnorm): the
+ * residual norms of classify(...; class_alg = "vbls") (examples/mil_util.jl:470-492) and, divided by L*M, of class_alg =
+ * "dual" (:519-533), without YHat.  kind = any of the four kinds; states[p] and Y[p] as for vbmf_b200_batched_vbls.  Reads
+ * only L, M, H, BHat and AHat of each state and writes nothing to it.  One L and H (H >= 1) for all problems, M >= 1 each,
+ * at most 2^31 columns in all, and min(L, M) <= 2048 per problem in spectral mode.  Needs no attached Y and leaves the
+ * context's resident Y and its solvers alone.  A NaN or Inf in a problem's residual gives NaN (spectral) or what the sum
+ * of squares gives (Frobenius) for that problem only; a problem's norm is the same bit for bit whatever batch it is in. */
+int vbmf_b200_batched_residual_norm(vbmf_b200_ctx* ctx, int kind, int64_t nprob, const double* const* Y,
+                                    void* const* states, int norm_mode, double* out);
 
 /* ---- one-call drop-ins: upload + loop + updateYHat! + download ---- */
 /* vbmf!(Y, params, niter; eps, est_covs, est_var)   src/vbmf.jl:175 */

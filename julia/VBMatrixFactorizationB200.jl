@@ -20,7 +20,7 @@ import VBMatrixFactorization: vbmf!, vbmf, vbmf_sparse!, vbmf_sparse, vbmf_dual!
                               lowerBound, lowerBoundTrimmed
 
 export b200_context, b200_close, b200_peer_exchange, b200_default_context!, vbmf!, vbmf, vbmf_sparse!, vbmf_sparse, vbmf_dual!, vbmf_dual, vbmf_trial!, vbmf_trial,
-       lowerBound, lowerBoundTrimmed, vbls_batched!, lowerBound_batched, lowerBoundTrimmed_batched, preprocess, vbmf_group!
+       lowerBound, lowerBoundTrimmed, vbls_batched!, lowerBound_batched, lowerBoundTrimmed_batched, residual_norm_batched, preprocess, vbmf_group!
 
 const LIB = get(ENV, "VBMF_B200_LIB", "libvbmf_b200.so")
 
@@ -422,45 +422,49 @@ end
 # Ys[k] is the L x M_k matrix of problem k, ps[k] its parameters (all of one type, with the same L, H, H0); one method per
 # branch of vbls! (:182-197).  kind: 0 dense, 1 sparse, 2 dual, 3 trial (include/vbmf_b200.h).  Bags of any size: those
 # too large for one CTA's shared memory run in the wide kernel (one thread-block cluster per bag) within the same call.
-# Dense and sparse states pass pointer(p.labels): with H1 > 0 every A update zeroes AHat[labels, H-H1+1:H].
+# Dense and sparse states pass pointer(p.labels): with H1 > 0 every A update zeroes AHat[labels, H-H1+1:H].  yhat = false
+# skips updateYHat! and leaves p.YHat empty, for a caller that only needs residual_norm_batched afterwards.
 function batched_call(ctx::B200Context, kind::Int, Ys::Vector{Array{Float64,2}}, sts::Vector, niter::Int, flags::Int)
     yptr = Ptr{Float64}[pointer(Y) for Y in Ys]
     sptr = Ptr{Void}[convert(Ptr{Void}, Base.unsafe_convert(Ptr{eltype(r)}, r)) for r in sts]
     check(ccall((:vbmf_b200_batched_vbls, LIB), Cint, (Ptr{Void}, Cint, Int64, Ptr{Ptr{Float64}}, Ptr{Ptr{Void}}, Int64, Cint),
                 ctx.handle, kind, length(sts), yptr, sptr, niter, flags))
 end
-function vbls_batched!(ctx::B200Context, Ys::Vector{Array{Float64,2}}, ps::Vector{vbmf_dual_parameters}, niter::Int; full_cov::Bool = false)
-    for p in ps; p.YHat = Array{Float64}(p.L, p.M); end
-    sts = [Ref(dual_state(p)) for p in ps]
+function vbls_batched!(ctx::B200Context, Ys::Vector{Array{Float64,2}}, ps::Vector{vbmf_dual_parameters}, niter::Int; full_cov::Bool = false,
+                       yhat::Bool = true)
+    for p in ps; p.YHat = yhat_buffer(p, yhat); end
+    sts = [Ref(dual_state(p, yhat)) for p in ps]
     batched_call(ctx, 2, Ys, sts, niter, full_cov ? 2 : 0)
     for (p, r) in zip(ps, sts)
         p.sigmaHat = r[].sigmaHat; p.zeta = r[].zeta; p.alpha0 = r[].alpha0; p.alpha1 = r[].alpha1
     end
     return [p.AHat for p in ps]
 end
-function vbls_batched!(ctx::B200Context, Ys::Vector{Array{Float64,2}}, ps::Vector{vbmf_sparse_parameters}, niter::Int; full_cov::Bool = false)
-    for p in ps; p.YHat = Array{Float64}(p.L, p.M); end
-    sts = [Ref(sparse_state(p, convert(Ptr{Float64}, C_NULL))) for p in ps]
+function vbls_batched!(ctx::B200Context, Ys::Vector{Array{Float64,2}}, ps::Vector{vbmf_sparse_parameters}, niter::Int; full_cov::Bool = false,
+                       yhat::Bool = true)
+    for p in ps; p.YHat = yhat_buffer(p, yhat); end
+    sts = [Ref(sparse_state(p, convert(Ptr{Float64}, C_NULL), yhat)) for p in ps]
     batched_call(ctx, 1, Ys, sts, niter, full_cov ? 2 : 0)
     for (p, r) in zip(ps, sts)
         p.sigmaHat = r[].sigmaHat; p.zeta = r[].zeta
     end
     return [p.AHat for p in ps]
 end
-function vbls_batched!(ctx::B200Context, Ys::Vector{Array{Float64,2}}, ps::Vector{vbmf_trial_parameters}, niter::Int; full_cov::Bool = false)
-    for p in ps; p.YHat = Array{Float64}(p.L, p.M); end
-    sts = [Ref(trial_state(p)) for p in ps]
+function vbls_batched!(ctx::B200Context, Ys::Vector{Array{Float64,2}}, ps::Vector{vbmf_trial_parameters}, niter::Int; full_cov::Bool = false,
+                       yhat::Bool = true)
+    for p in ps; p.YHat = yhat_buffer(p, yhat); end
+    sts = [Ref(trial_state(p, yhat)) for p in ps]
     batched_call(ctx, 3, Ys, sts, niter, full_cov ? 2 : 0)
     for (p, r) in zip(ps, sts)
         p.sigmaHat = r[].sigmaHat; p.zeta = r[].zeta; p.alpha1 = r[].alpha1; p.alpha2 = r[].alpha2; p.alpha3 = r[].alpha3
     end
     return [p.AHat for p in ps]
 end
-function vbls_batched!(ctx::B200Context, Ys::Vector{Array{Float64,2}}, ps::Vector{vbmf_parameters}, niter::Int)
-    for p in ps; p.YHat = Array{Float64}(p.L, p.M); end
+function vbls_batched!(ctx::B200Context, Ys::Vector{Array{Float64,2}}, ps::Vector{vbmf_parameters}, niter::Int; yhat::Bool = true)
+    for p in ps; p.YHat = yhat_buffer(p, yhat); end
     sts = [Ref(DenseState(p.L, p.M, p.H, p.H1, length(p.labels), pointer(p.labels), pointer(p.AHat), pointer(p.BHat),
                           pointer(p.SigmaA), pointer(p.SigmaB), pointer(p.CA), pointer(p.CB), pointer(p.invCA), pointer(p.invCB),
-                          p.sigma2, pointer(p.YHat))) for p in ps]
+                          p.sigma2, yhat_ptr(p, yhat))) for p in ps]
     batched_call(ctx, 0, Ys, sts, niter, 0)
     for (p, r) in zip(ps, sts); p.sigma2 = r[].sigma2; end
     return [p.AHat for p in ps]
@@ -496,6 +500,40 @@ batched_lower_bound(ctx::B200Context, Ys::Vector{Array{Float64,2}}, ps::Vector{v
 lowerBound_batched(ctx::B200Context, Ys::Vector{Array{Float64,2}}, ps::Vector) = batched_lower_bound(ctx, Ys, ps, 0.0, false)
 lowerBoundTrimmed_batched(ctx::B200Context, Ys::Vector{Array{Float64,2}}, ps::Vector, trim = 1e-1) =
     batched_lower_bound(ctx, Ys, ps, Float64(trim), true)
+
+# ---- norm(Y - BHat*AHat') for many bags in one call: the residual norms of classify (examples/mil_util.jl:470-492 with
+# class_alg = "vbls"; :519-533 with "dual", divided there by L*M), e.g. after vbls_batched! with yhat = false.
+# norm = :spectral (Julia 0.5 norm(::Matrix)) or :frobenius (vecnorm).  One type, one L and H; reads only L, M, H, BHat and
+# AHat; single-device contexts; needs no attached Y.  Returns a Vector{Float64}.
+function batched_rn_call(ctx::B200Context, kind::Int, Ys::Vector{Array{Float64,2}}, sts::Vector, norm::Symbol)
+    ctx.multi && error("the batched residual norm runs on one device: use a single-device context")
+    haskey(NORM, norm) || error("residual_norm_batched: norm must be :spectral or :frobenius")
+    yptr = Ptr{Float64}[pointer(Y) for Y in Ys]
+    sptr = Ptr{Void}[convert(Ptr{Void}, Base.unsafe_convert(Ptr{eltype(r)}, r)) for r in sts]
+    out = Array{Float64}(length(sts))
+    check(ccall((:vbmf_b200_batched_residual_norm, LIB), Cint,
+                (Ptr{Void}, Cint, Int64, Ptr{Ptr{Float64}}, Ptr{Ptr{Void}}, Cint, Ptr{Float64}),
+                ctx.handle, kind, length(sts), yptr, sptr, NORM[norm], out))
+    return out
+end
+function residual_norm_batched(ctx::B200Context, Ys::Vector{Array{Float64,2}}, ps::Vector{vbmf_parameters}; norm::Symbol = :spectral)
+    sts = [Ref(DenseState(p.L, p.M, p.H, p.H1, length(p.labels), pointer(p.labels), pointer(p.AHat), pointer(p.BHat),
+                          pointer(p.SigmaA), pointer(p.SigmaB), pointer(p.CA), pointer(p.CB), pointer(p.invCA), pointer(p.invCB),
+                          p.sigma2, convert(Ptr{Float64}, C_NULL))) for p in ps]
+    batched_rn_call(ctx, 0, Ys, sts, norm)
+end
+function residual_norm_batched(ctx::B200Context, Ys::Vector{Array{Float64,2}}, ps::Vector{vbmf_sparse_parameters}; norm::Symbol = :spectral)
+    for p in ps; isdefined(p, :YHat) || (p.YHat = Array{Float64}(0, 0)); end
+    batched_rn_call(ctx, 1, Ys, [Ref(sparse_state(p, convert(Ptr{Float64}, C_NULL), false)) for p in ps], norm)
+end
+function residual_norm_batched(ctx::B200Context, Ys::Vector{Array{Float64,2}}, ps::Vector{vbmf_dual_parameters}; norm::Symbol = :spectral)
+    for p in ps; isdefined(p, :YHat) || (p.YHat = Array{Float64}(0, 0)); end
+    batched_rn_call(ctx, 2, Ys, [Ref(dual_state(p, false)) for p in ps], norm)
+end
+function residual_norm_batched(ctx::B200Context, Ys::Vector{Array{Float64,2}}, ps::Vector{vbmf_trial_parameters}; norm::Symbol = :spectral)
+    for p in ps; isdefined(p, :YHat) || (p.YHat = Array{Float64}(0, 0)); end
+    batched_rn_call(ctx, 3, Ys, [Ref(trial_state(p, false)) for p in ps], norm)
+end
 
 # ---- preprocess(Y, lambda) (src/util.jl:73-87) on the device; the processed matrix stays resident (pass `nothing` for Y to
 # the solvers to run on it without another upload); single-device contexts

@@ -28,7 +28,7 @@ __all__ = [
     "vbmf_init", "vbmf_", "vbmf", "vbmf_sparse_init", "vbmf_sparse_", "vbmf_sparse", "vbmf_dual_init", "vbmf_dual_",
     "vbmf_dual", "updateA_", "updateB_", "updateCA_", "updateCB_", "updateSigma2_", "updateSigma_", "updateYHat_",
     "updateAlpha00_", "updateAlpha01_", "updateBeta00_", "updateBeta01_", "lowerBound", "lowerBoundTrimmed", "copy",
-    "run_group", "vbmf_group_", "vbls_", "vbls_batched_", "BatchedVbls", "lowerBound_batched", "lowerBoundTrimmed_batched", "preprocess", "VBMFWarning", "create_log", "update_log_", "save_log", "load_log", "extract_params_", "VBMFError",
+    "run_group", "vbmf_group_", "vbls_", "vbls_batched_", "BatchedVbls", "lowerBound_batched", "lowerBoundTrimmed_batched", "residual_norm_batched", "preprocess", "VBMFWarning", "create_log", "update_log_", "save_log", "load_log", "extract_params_", "VBMFError",
 ]
 
 VBMFError = L_.VBMFError
@@ -1027,6 +1027,22 @@ class BatchedVbls:
                                                             out.ctypes.data))
         return out
 
+    def residual_norm(self, norm="spectral"):
+        """norm(Y - BHat*AHat') of every problem in one C-ABI call (`vbmf_b200_batched_residual_norm`) on the structs this
+        object holds: after `run` they point at the vbls results, so nothing is marshalled again.  norm = "spectral" (Julia
+        0.5 norm(::Matrix), the largest singular value) or "frobenius".  Divided by L*M this is the error of
+        classify(...; class_alg="dual"); undivided, that of class_alg="vbls".  Returns a float64 array, one norm per problem."""
+        if norm not in _NORMS:
+            raise VBMFError('residual_norm: norm must be "spectral" or "frobenius" (got %r)' % (norm,))
+        out = np.zeros(self.n)
+        if self.n == 0:
+            return out
+        if isinstance(self.ctx, MultiContext):
+            raise VBMFError("the batched residual norm runs on one device: pass a single-device Context, not a MultiContext")
+        L_.check(self.ctx.lib.vbmf_b200_batched_residual_norm(self.ctx.h, self.kind, self.n, self.yp, self.sp, _NORMS[norm],
+                                                              out.ctypes.data))
+        return out
+
 
 def vbls_batched_(Ys, params_list, niter, full_cov=False, diag_var=False, ctx=None, yhat=True, keep_blocks=False):
     """`vbls!` (examples/mil_util.jl:179-203) for many problems in ONE C-ABI call (one CTA per problem; problems too large
@@ -1051,6 +1067,14 @@ def lowerBoundTrimmed_batched(Ys, params_list, trim=1e-1, ctx=None):
     """`lowerBoundTrimmed` (src/vbmf_sparse.jl:478, src/vbmf_dual.jl:606, src/vbmf_trial.jl:687) of many problems in one
     call, as `lowerBound_batched`."""
     return BatchedVbls(Ys, params_list, ctx=ctx, yhat=False).lower_bound(float(trim))
+
+
+def residual_norm_batched(Ys, params_list, norm="spectral", ctx=None):
+    """norm(Y - BHat*AHat') of many problems in ONE C-ABI call, the residual norms `classify` (examples/mil_util.jl:470-492,
+    :519-533) takes of every (bag, class model) pair.  params of one type (any of the four) with the same L and H; M may
+    differ.  norm = "spectral" (Julia 0.5 norm(::Matrix)) or "frobenius".  One device, no attached Y needed; reads only
+    L, M, H, BHat and AHat.  Returns a float64 array."""
+    return BatchedVbls(Ys, params_list, ctx=ctx, yhat=False).residual_norm(norm)
 
 
 def preprocess(Y, lam, verb=False, ctx=None):

@@ -1051,4 +1051,160 @@ int k_batched_lower_bound(cudaStream_t st, const BatchLbDesc& bd) {
     return 0;
 }
 
+
+// ---- batched residual norms norm(Y[p] - BHat*AHat') -------------------------------------------------------------------
+// examples/mil_util.jl:470-492 (class_alg = "vbls": norm(Y - B*A')) and :519-533 ("dual": norm(YHat - Y), YHat = B*A') for
+// every (bag, class model) pair.  Layout and phases: BatchRnDesc (kernels.cuh).
+
+// scaled residual entry R[l, m] * 2^-e of the problem whose Y, B, A start at Yp, Bp, Ap; 0 outside the L x M matrix
+__device__ __forceinline__ double rn_residual(const double* __restrict__ Yp, const double* __restrict__ Bp, const double* __restrict__ Ap,
+                                              int L, int M, int H, int l, int m, double sc) {
+    if (l >= L || m >= M) return 0.0;
+    double s = 0.0;
+    for (int h = 0; h < H; ++h) s = fma(__ldg(Bp + (size_t)h * L + l), __ldg(Ap + (size_t)h * M + m), s);
+    return (__ldg(Yp + (size_t)m * L + l) - s) * sc;
+}
+
+__device__ __forceinline__ int rn_exponent(double x) { int e; frexp(x, &e); return e; }
+
+// One CTA per problem: e with |Y| < 2^eY and H*|B|*|A| <= 2^(eB+eA+ceil(log2 H)), so |R| * 2^-e < 2.  The maxima are taken
+// over the finite entries (a non-finite one reaches the result through the arithmetic); an all-zero problem gets e = 0.
+// Scaling Y and B by 2^s moves e by exactly s, so the scaled residual and hence the norm's mantissa do not change.
+__global__ void __launch_bounds__(256) batched_rn_scale_kernel(BatchRnDesc bd) {
+    __shared__ unsigned long long s_max[3];
+    const int p = blockIdx.x, t = threadIdx.x, L = bd.L, H = bd.H;
+    const int m0 = bd.moff[p], M = bd.moff[p + 1] - m0;
+    if (t < 3) s_max[t] = 0ull;
+    __syncthreads();
+    const double* src[3] = {bd.Y + (size_t)m0 * L, bd.B + (size_t)p * L * H, bd.A + (size_t)m0 * H};
+    const size_t len[3] = {(size_t)L * M, (size_t)L * H, (size_t)M * H};
+    for (int k = 0; k < 3; ++k) {
+        double mx = 0.0;
+        for (size_t i = t; i < len[k]; i += blockDim.x) {
+            const double x = fabs(src[k][i]);
+            if (x <= 1.79e308) mx = fmax(mx, x);
+        }
+        atomicMax(&s_max[k], (unsigned long long)__double_as_longlong(mx));   // non-negative doubles order as their bits
+    }
+    __syncthreads();
+    if (t == 0) {
+        const double ya = __longlong_as_double((long long)s_max[0]), ba = __longlong_as_double((long long)s_max[1]),
+                     aa = __longlong_as_double((long long)s_max[2]);
+        int lh = 0;
+        while ((1 << lh) < H) ++lh;
+        const bool y = ya > 0.0, ba_ = ba > 0.0 && aa > 0.0;
+        const int ey = y ? rn_exponent(ya) : 0, eba = ba_ ? rn_exponent(ba) + rn_exponent(aa) + lh : 0;
+        bd.escale[p] = (y && ba_) ? max(ey, eba) : (y ? ey : eba);
+    }
+}
+
+// Spectral phase 1: one CTA per RN_TILE x RN_TILE tile (I, J), I <= J, of the problem's Gram.  Per chunk of RN_TILE summed
+// indices the two strips R(k, I-tile) and R(k, J-tile) are formed in shared memory, then every thread adds 4 products per
+// index to its 4 Gram entries, indices in increasing order.  Entry (i, j) and (j, i) of a diagonal tile see the same
+// operands in the same order, so the Gram is exactly symmetric; off-diagonal tiles are written to both triangles.
+__global__ void __launch_bounds__(256) batched_rn_gram_kernel(BatchRnDesc bd) {
+    __shared__ double RI[RN_TILE][RN_TILE + 1], RJ[RN_TILE][RN_TILE + 1];
+    const int c = blockIdx.x, p = bd.tprob[c], t = threadIdx.x;
+    const int L = bd.L, H = bd.H, m0 = bd.moff[p], M = bd.moff[p + 1] - m0;
+    const bool cols = M <= L;                    // R'R (n = M, summed over the L rows), else RR' (n = L, summed over M)
+    const int n = cols ? M : L, K = cols ? L : M, nt = (n + RN_TILE - 1) / RN_TILE;
+    int k = c - bd.toff[p], I = 0;
+    while (k >= nt - I) { k -= nt - I; ++I; }
+    const int J = I + k;
+    const double* Yp = bd.Y + (size_t)m0 * L;
+    const double* Bp = bd.B + (size_t)p * L * H;
+    const double* Ap = bd.A + (size_t)m0 * H;
+    const double sc = ldexp(1.0, -bd.escale[p]);
+    const int j = t & 31, i0 = t >> 5;          // this thread's Gram entries: (I*32 + i0 + 8q, J*32 + j), q < 4
+    double acc[4] = {0.0, 0.0, 0.0, 0.0};
+    for (int k0 = 0; k0 < K; k0 += RN_TILE) {
+        for (int e = t; e < RN_TILE * RN_TILE; e += blockDim.x) {
+            const int a = e & 31, b = e >> 5;
+            const int kk = cols ? a : b, ii = cols ? b : a;   // consecutive threads walk down a column of Y
+            const int kg = k0 + kk, gi = I * RN_TILE + ii, gj = J * RN_TILE + ii;
+            RI[kk][ii] = cols ? rn_residual(Yp, Bp, Ap, L, M, H, kg, gi, sc) : rn_residual(Yp, Bp, Ap, L, M, H, gi, kg, sc);
+            if (J != I) RJ[kk][ii] = cols ? rn_residual(Yp, Bp, Ap, L, M, H, kg, gj, sc) : rn_residual(Yp, Bp, Ap, L, M, H, gj, kg, sc);
+        }
+        __syncthreads();
+        const double(*R2)[RN_TILE + 1] = J == I ? RI : RJ;
+#pragma unroll 8
+        for (int kk = 0; kk < RN_TILE; ++kk) {
+            const double b = R2[kk][j];
+#pragma unroll
+            for (int q = 0; q < 4; ++q) acc[q] = fma(RI[kk][i0 + 8 * q], b, acc[q]);
+        }
+        __syncthreads();
+    }
+    double* G = bd.work + bd.goff[p];
+    const int gj = J * RN_TILE + j;
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+        const int gi = I * RN_TILE + i0 + 8 * q;
+        if (gi < n && gj < n) { G[(size_t)gi * n + gj] = acc[q]; G[(size_t)gj * n + gi] = acc[q]; }
+    }
+}
+
+// Frobenius phase 1: one CTA per batched_rn_cols(L) columns, the squares of the scaled residual summed per thread in
+// element order, then over the CTA by block_sum's fixed tree.
+__global__ void __launch_bounds__(256) batched_rn_sumsq_kernel(BatchRnDesc bd) {
+    __shared__ double red[32];
+    const int c = blockIdx.x, p = bd.tprob[c], t = threadIdx.x;
+    const int L = bd.L, H = bd.H, m0 = bd.moff[p], M = bd.moff[p + 1] - m0;
+    const int lo = (c - bd.toff[p]) * batched_rn_cols(L), hi = min(M, lo + batched_rn_cols(L));
+    const double* Yp = bd.Y + (size_t)m0 * L;
+    const double* Bp = bd.B + (size_t)p * L * H;
+    const double* Ap = bd.A + (size_t)m0 * H;
+    const double sc = ldexp(1.0, -bd.escale[p]);
+    double s = 0.0;
+    for (size_t e = (size_t)lo * L + t; e < (size_t)hi * L; e += blockDim.x) {
+        const int m = (int)(e / L), l = (int)(e - (size_t)m * L);
+        const double r = rn_residual(Yp, Bp, Ap, L, M, H, l, m, sc);
+        s = fma(r, r, s);
+    }
+    s = block_sum(s, red);
+    if (t == 0) bd.work[c] = s;
+}
+
+// Phase 2, one CTA per problem.  Spectral: sym_lambda_max on the Gram, copied to shared memory when n <= RN_SMEM_NMAX, else
+// in place in global memory with its scratch there too; norm = sqrt(max(lambda, 0)) * 2^e, NaN kept.  Frobenius: the
+// partials added in tile order.
+__global__ void __launch_bounds__(512) batched_rn_final_kernel(BatchRnDesc bd) {
+    extern __shared__ double sm[];
+    const int p = blockIdx.x, t = threadIdx.x;
+    const int e = bd.escale[p];
+    if (bd.mode == 1) {
+        if (t == 0) {
+            double s = 0.0;
+            for (int c = bd.toff[p]; c < bd.toff[p + 1]; ++c) s += bd.work[c];
+            bd.out[p] = ldexp(sqrt(s), e);
+        }
+        return;
+    }
+    const int M = bd.moff[p + 1] - bd.moff[p], n = min(bd.L, M);
+    double* G = bd.work + bd.goff[p];
+    double v;
+    if (n <= RN_SMEM_NMAX) {
+        for (int i = t; i < n * n; i += blockDim.x) sm[i] = G[i];
+        __syncthreads();
+        v = sym_lambda_max(sm, n, n, sm + n * n);
+    } else {
+        v = sym_lambda_max(G, n, n, G + (size_t)n * n);
+    }
+    if (t == 0) bd.out[p] = ldexp(sqrt(fmax(v, 0.0)), e) + (v != v ? v : 0.0);
+}
+
+int k_batched_residual_norm(cudaStream_t st, const BatchRnDesc& bd, int smem_n) {
+    if (bd.nprob <= 0) return 0;
+    batched_rn_scale_kernel<<<bd.nprob, 256, 0, st>>>(bd);
+    VB_LAUNCH_OK();
+    if (bd.mode == 1) batched_rn_sumsq_kernel<<<bd.ntile, 256, 0, st>>>(bd);
+    else batched_rn_gram_kernel<<<bd.ntile, 256, 0, st>>>(bd);
+    VB_LAUNCH_OK();
+    const size_t smem = bd.mode == 1 ? 0 : (size_t)(smem_n * smem_n + 4 * smem_n) * sizeof(double);
+    VB_CUDA_OK(cudaFuncSetAttribute(batched_rn_final_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    batched_rn_final_kernel<<<bd.nprob, 512, smem, st>>>(bd);
+    VB_LAUNCH_OK();
+    return 0;
+}
+
 }  // namespace vb

@@ -2609,6 +2609,103 @@ extern "C" int vbmf_b200_batched_lower_bound(vbmf_b200_ctx* c, int kind, int64_t
     return -1;
 }
 
+// ---- batched residual norms norm(Y[p] - BHat*AHat') ------------------------------------------------------------------------
+// Reads L, M, H, BHat and AHat of every state, the fields updateYHat! reads (src/vbmf.jl:120, src/vbmf_sparse.jl:275), and
+// packs them with Y into the staging arena; the kernels are in batched.cu (BatchRnDesc).
+template <class ST>
+static int batched_residual_norm_impl(vbmf_b200_ctx* c, int64_t nprob, const double* const* Y, void* const* states, int mode,
+                                      double* out) {
+    if (nprob <= 0) return 0;
+    const ST* s0 = (const ST*)states[0];
+    if (s0 == nullptr) { set_error("batched residual norm: NULL problem 0"); return -1; }
+    const int64_t L = s0->L, H = s0->H;
+    if (L < 1 || L > 0x7fffff00LL || H < 1 || H > 0x7fffff00LL) {
+        set_error("batched residual norm needs L >= 1 and H >= 1 (got L = %lld, H = %lld)", (long long)L, (long long)H); return -1;
+    }
+    std::vector<int> moff(nprob + 1, 0), toff(nprob + 1, 0);
+    std::vector<long long> goff(nprob, 0);
+    long long gtot = 0;
+    int smem_n = 0;
+    for (int64_t p = 0; p < nprob; ++p) {
+        const ST* s = (const ST*)states[p];
+        if (s == nullptr || Y[p] == nullptr) { set_error("batched residual norm: NULL problem %lld", (long long)p); return -1; }
+        if (s->L != L || s->H != H) { set_error("batched residual norm: problem %lld has a different L or H", (long long)p); return -1; }
+        if (s->M < 1) { set_error("batched residual norm: problem %lld has M < 1", (long long)p); return -1; }
+        if (s->BHat == nullptr || s->AHat == nullptr) { set_error("batched residual norm: BHat or AHat of problem %lld is NULL", (long long)p); return -1; }
+        if ((int64_t)moff[p] + s->M > 0x7fffff00LL) { set_error("batched residual norm: more than 2^31 columns in one call"); return -1; }
+        const int M = (int)s->M, n = (int)std::min<int64_t>(L, M);
+        if (mode == VBMF_B200_NORM_SPECTRAL) {
+            if (n > vb::RN_SPECTRAL_NMAX) {
+                set_error("batched residual norm: the spectral norm of problem %lld needs min(L, M) <= %d (got %d)", (long long)p,
+                          vb::RN_SPECTRAL_NMAX, n);
+                return -1;
+            }
+            goff[p] = gtot;
+            gtot += (long long)n * n + 4 * n;
+            if (n <= vb::RN_SMEM_NMAX) smem_n = std::max(smem_n, n);
+        }
+        moff[p + 1] = moff[p] + M;
+        toff[p + 1] = toff[p] + vb::batched_rn_tiles(mode, (int)L, M);
+    }
+    const int ntile = toff[nprob];
+    const size_t Mtot = (size_t)moff[nprob], LH = (size_t)L * H;
+    VB_CUDA_OK(cudaSetDevice(c->device));
+    // one arena: [inputs | scales, results | device-only Grams or partials]; one upload, one download of the results
+    size_t off = 0;
+    auto take = [&](size_t bytes) { const size_t o = off; off += align_up(bytes, 256); return o; };
+    const size_t o_moff = take((size_t)(nprob + 1) * 4), o_toff = take((size_t)(nprob + 1) * 4), o_tp = take((size_t)ntile * 4),
+                 o_goff = take((size_t)nprob * 8), o_Y = take(L * Mtot * 8), o_B = take(nprob * LH * 8), o_A = take(Mtot * H * 8);
+    const size_t up_end = off;
+    const size_t o_e = take((size_t)nprob * 4), o_out = take((size_t)nprob * 8);
+    const size_t o_w = take((mode == VBMF_B200_NORM_SPECTRAL ? (size_t)gtot : (size_t)ntile) * 8);
+    if (batch_reserve(c, off)) return -1;
+    char* hb = c->batch_host;
+    char* db = c->batch_dev;
+    memcpy(hb + o_moff, moff.data(), (size_t)(nprob + 1) * 4);
+    memcpy(hb + o_toff, toff.data(), (size_t)(nprob + 1) * 4);
+    memcpy(hb + o_goff, goff.data(), (size_t)nprob * 8);
+    int* htp = (int*)(hb + o_tp);
+    for (int64_t p = 0; p < nprob; ++p) for (int k = toff[p]; k < toff[p + 1]; ++k) htp[k] = (int)p;
+    double *hY = (double*)(hb + o_Y), *hB = (double*)(hb + o_B), *hA = (double*)(hb + o_A);
+    parallel_for(nprob, [&](int64_t p) {
+        const ST* s = (const ST*)states[p];
+        memcpy(&hY[(size_t)moff[p] * L], Y[p], (size_t)s->M * L * 8);
+        memcpy(&hB[p * LH], s->BHat, LH * 8);
+        memcpy(&hA[(size_t)moff[p] * H], s->AHat, (size_t)s->M * H * 8);
+    });
+    cudaStream_t st = c->st;
+    if (cudaMemcpyAsync(db, hb, up_end, cudaMemcpyHostToDevice, st) != cudaSuccess) { cudaGetLastError(); set_error("batched residual norm: upload failed"); return -1; }
+    BatchRnDesc bd;
+    bd.nprob = (int)nprob; bd.ntile = ntile; bd.L = (int)L; bd.H = (int)H; bd.mode = mode;
+    bd.moff = (const int*)(db + o_moff); bd.toff = (const int*)(db + o_toff); bd.tprob = (const int*)(db + o_tp);
+    bd.goff = (const long long*)(db + o_goff); bd.Y = (const double*)(db + o_Y); bd.B = (const double*)(db + o_B);
+    bd.A = (const double*)(db + o_A); bd.escale = (int*)(db + o_e); bd.work = (double*)(db + o_w); bd.out = (double*)(db + o_out);
+    prof_mark(c, c->ev_k1);       // profiling: the kernels alone (vbmf_b200_ctx_profile_read, K1 slot)
+    int rc = k_batched_residual_norm(st, bd, smem_n);
+    prof_mark(c, c->ev_k1);
+    if (!rc && cudaMemcpyAsync(hb + o_out, db + o_out, (size_t)nprob * 8, cudaMemcpyDeviceToHost, st) != cudaSuccess) {
+        cudaGetLastError(); set_error("batched residual norm: download failed"); rc = -1;
+    }
+    { cudaError_t e = cudaStreamSynchronize(st); if (e != cudaSuccess && !rc) { set_error("batched residual norm: %s", cudaGetErrorString(e)); rc = -1; } }
+    if (rc) return rc;
+    memcpy(out, hb + o_out, (size_t)nprob * 8);
+    return 0;
+}
+
+extern "C" int vbmf_b200_batched_residual_norm(vbmf_b200_ctx* c, int kind, int64_t nprob, const double* const* Y, void* const* states,
+                                               int norm_mode, double* out) {
+    if (!c || (nprob > 0 && (!Y || !states || !out))) { set_error("batched residual norm: NULL argument"); return -1; }
+    if (norm_mode != VBMF_B200_NORM_SPECTRAL && norm_mode != VBMF_B200_NORM_FROBENIUS) {
+        set_error("batched residual norm: unknown norm mode %d", norm_mode); return -1;
+    }
+    if (kind == VBMF_B200_DENSE) return batched_residual_norm_impl<vbmf_b200_dense_state>(c, nprob, Y, states, norm_mode, out);
+    if (kind == VBMF_B200_SPARSE) return batched_residual_norm_impl<vbmf_b200_sparse_state>(c, nprob, Y, states, norm_mode, out);
+    if (kind == VBMF_B200_DUAL) return batched_residual_norm_impl<vbmf_b200_dual_state>(c, nprob, Y, states, norm_mode, out);
+    if (kind == VBMF_B200_TRIAL) return batched_residual_norm_impl<vbmf_b200_trial_state>(c, nprob, Y, states, norm_mode, out);
+    set_error("batched residual norm: unknown parameter kind %d", kind);
+    return -1;
+}
+
 extern "C" int vbmf_b200_batched_vbls(vbmf_b200_ctx* c, int kind, int64_t nprob, const double* const* Y, void* const* states,
                                       int64_t niter, int flags) {
     if (!c || (nprob > 0 && (!Y || !states))) { set_error("batched vbls: NULL argument"); return -1; }

@@ -223,4 +223,40 @@ constexpr int LB_NPART = 12;
 __host__ __device__ inline int batched_lb_cols(int H) { return 16384 / H > 16 ? 16384 / H : 16; }
 int k_batched_lower_bound(cudaStream_t st, const BatchLbDesc& bd);
 
+// Batched residual norms norm(Y[p] - B[p]*A[p]') (csrc/batched.cu), spectral or Frobenius.  R = Y - B*A' is recomputed where
+// it is read and never stored.  Every problem gets a power-of-two scale 2^-e from its own max|Y| and max|B|*max|A|*H, so
+// that the scaled residual stays below 2 and its squares neither overflow nor underflow.  Spectral: phase 1 cuts the
+// problem's n x n Gram of the scaled residual (n = min(L, M): R'R when M <= L, else RR') into RN_TILE x RN_TILE tiles of
+// its upper triangle, one CTA each, and phase 2 runs sym_lambda_max on it, one CTA per problem.  Frobenius: phase 1 sums the
+// squares of batched_rn_cols(L) columns per CTA, phase 2 adds the partials in order.  The split depends on the problem's own
+// L, M alone, so its norm is the same bit for bit whatever batch it is in.
+struct BatchRnDesc {
+    int nprob, ntile, L, H, mode;   // mode: VBMF_B200_NORM_SPECTRAL (0) or VBMF_B200_NORM_FROBENIUS (1)
+    const int* moff;        // [nprob+1] column offsets into the packed Y / A
+    const int* toff;        // [nprob+1] first phase-1 tile of each problem
+    const int* tprob;       // [ntile]   problem of each tile
+    const long long* goff;  // [nprob]   spectral: offset in `work` of the problem's n*n Gram and 4n sym_lambda_max scratch
+    const double* Y;        // [L][Mtot] column-major, problems concatenated
+    const double* B;        // [nprob][L*H] BHat, column-major L x H
+    const double* A;        // AHat of problem p at moff[p]*H, column-major M x H
+    int* escale;            // [nprob] e of the scale 2^-e
+    double* work;           // spectral: the Grams; Frobenius: [ntile] partial sums of squares
+    double* out;            // [nprob]
+};
+constexpr int RN_TILE = 32;
+// Largest n whose Gram and sym_lambda_max scratch, n*n + 4n doubles, fit the 227 KB of shared memory an sm_100 CTA may opt
+// into (next to sym_lambda_max's 60 static bytes): 168*168 + 4*168 = 28896 doubles = 231168 B.  Larger Grams stay in
+// global memory and the same routine runs on them there.
+constexpr int RN_SMEM_NMAX = 168;
+// Spectral limit: one CTA tridiagonalises the n x n Gram, O(n^3) with n syncs; beyond this an iterative method is the tool.
+constexpr int RN_SPECTRAL_NMAX = 2048;
+__host__ __device__ inline int batched_rn_cols(int L) { return 8192 / L > 1 ? 8192 / L : 1; }
+__host__ __device__ inline int batched_rn_tiles(int mode, int L, int M) {
+    if (mode == 1) return (M + batched_rn_cols(L) - 1) / batched_rn_cols(L);
+    const int nt = ((M < L ? M : L) + RN_TILE - 1) / RN_TILE;
+    return nt * (nt + 1) / 2;
+}
+// smem_n = the largest n <= RN_SMEM_NMAX of a spectral batch (0 when there is none): the shared memory of phase 2
+int k_batched_residual_norm(cudaStream_t st, const BatchRnDesc& bd, int smem_n);
+
 }  // namespace vb

@@ -8,7 +8,10 @@ the wide kernel (one thread-block cluster per bag) for bags too large for one CT
 
 Only the VB-based classifiers are mirrored ("vbls", "dual"); "ols"/"rls" are two-line host least-squares formulas with no VB
 update in them and stay with the caller.  The matrix norms of the L x M residuals follow Julia 0.5 (`norm(::Matrix)` =
-spectral norm, SURVEY quirk Q1) and are evaluated on the host: they are outputs of the path, a few hundred flops per bag.
+spectral norm, SURVEY quirk Q1) and are evaluated here on the host, one LAPACK SVD per bag and class model.  That is not
+cheap: on the Musk2-shaped batch of tools/batched/large_bags.py it takes about 1 s per pair of class models, against
+15 ms for `residual_norm_batched` / `BatchedVbls.residual_norm`, which compute the same norms on the device without
+downloading YHat (DESIGN section 5).
 """
 import numpy as np
 
